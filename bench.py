@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: object-updates/s and p50/p99 frame latency of the collision hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -31,6 +31,8 @@ Extra keys at N > 1 (same run, after the headline): `strong_scaling` = configs[3
 objects in total over the N slabs); at N = 8 also `configs4_10m` (10M objects, heavy skew).
 `verify`: a sample of queries of the headline frame re-computed by the CPU oracle (outside every timed
 region) and compared with what the GPUs emitted -- pair set exact, values to 1e-4.
+--dump-outputs DIR: what the last device-timed frame computed, as DIR/<name>.npy (see dump_outputs), so that two builds
+can be compared output by output on the same seeded frames.
 """
 from __future__ import annotations
 
@@ -218,7 +220,7 @@ def run_reference(args):
     frames, desc, _bounds, _side = make_frames(args.workload, args.gpus, args.objects_per_gpu, 2)
     n = len(frames[0]["px"])
     pattern = np.full(n, 2, np.uint8)
-    steps = max(1, args.steps)
+    steps = args.steps
     budget = max(1.0, min(20.0, 90.0 / (steps + args.warmup)))  # the whole run stays within a few minutes
     times, measured, extrap = [], [], False
     info, plan = None, None
@@ -601,9 +603,55 @@ def verify_counts(job: SlabJob, k: int, n_queries: int):
             "risks_checked": int(want[q].sum()), "ok": bool(ok), "oracle_seconds": round(time.perf_counter() - t0, 2)}
 
 
+# --dump-outputs: the headline frame emits ~8 M pairs (~400 MB of records), so the pairs of a seeded sample of query
+# objects are written; the files stay under 64 MB at every workload
+DUMP_SEED = 2026
+DUMP_QUERIES = 1 << 15      # query objects whose pair records are written
+DUMP_PAIRS_MAX = 1 << 19    # records written at most (64 B each as written)
+DUMP_COUNTS_MAX = 1 << 21   # objects whose risk counts are written (all of them up to this many; 12 B each)
+
+
+def dump_outputs(job: SlabJob, k: int, out_dir: str) -> None:
+    """Write what frame k (the last timed frame, still on the device) hands a caller, as DIR/<name>.npy:
+      pairs_<field>  the rcd_pair records (rcd_download) whose querying object i is in a seeded sample, sorted by
+                     (i, j, predicted), one file per field: i, j in float64, the rest in float32
+      risk_counts    risks emitted per object (rcd_download_risk_counts), float32, for the objects in object_ids (float64)
+      total_pairs    float64 [pairs the frame emitted], summed over ranks (exact even when the pair buffer overflows)
+    Object ids are global and every pair is emitted once, by the owner of i, so the files do not depend on how the frame
+    was cut into slabs (as long as no rank's pair buffer overflows: then which records were stored is not fixed)."""
+    import torch.distributed as dist
+    n, world, rank = job.n_total, job.world, job.rank
+    rng = np.random.default_rng(DUMP_SEED)
+    queries = np.sort(rng.choice(n, min(n, DUMP_QUERIES), replace=False))
+    objects = np.arange(n) if n <= DUMP_COUNTS_MAX else np.sort(rng.choice(n, DUMP_COUNTS_MAX, replace=False))
+    pairs = job.eng.download()
+    ids = job.own_ids[k % len(job.own_ids)]
+    c = job.eng.counts()
+    mine = (pairs[np.isin(pairs["i"], queries)], ids, job.eng.risk_counts()[: len(ids)], c["n_pairs"])
+    parts = [mine]
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, mine)
+    if rank != 0:
+        return
+    pairs = np.sort(np.concatenate([p[0] for p in parts]), order=["i", "j", "predicted"])[:DUMP_PAIRS_MAX]
+    risk = np.zeros(n, np.float32)
+    for p in parts:
+        risk[p[1]] = p[2]
+    out = {f"pairs_{f}": pairs[f].astype(np.float64 if f in ("i", "j") else np.float32)
+           for f in pairs.dtype.names if f != "reserved"}
+    out["risk_counts"] = risk[objects]
+    out["object_ids"] = objects.astype(np.float64)
+    out["total_pairs"] = np.array([sum(p[3] for p in parts)], np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def measure(args, workload, per_gpu, world, rank, local_rank, flush, steps, warmup, rebalance_rounds, with_e2e=True,
-            with_verify=True, sampler=None, max_pairs=None, verify_kind="pairs", verify_queries=None):
-    """Everything for one workload: (re-balanced) slabs, device-timed frames, end-to-end frames, verification."""
+            with_verify=True, sampler=None, max_pairs=None, verify_kind="pairs", verify_queries=None, dump_dir=None):
+    """Everything for one workload: (re-balanced) slabs, device-timed frames, end-to-end frames, verification.
+    dump_dir: write the outputs of the last device-timed frame there (dump_outputs) before anything else runs a frame."""
     import torch
     from rcd_b200.host import _native as N
     cuts, rb_hist = (None, [])
@@ -611,6 +659,8 @@ def measure(args, workload, per_gpu, world, rank, local_rank, flush, steps, warm
         cuts, rb_hist = rebalance(args, workload, per_gpu, world, rank, local_rank, flush, rebalance_rounds, max_pairs)
     job = SlabJob(args, workload, per_gpu, world, rank, local_rank, cuts=cuts, profile=True, graph=args.graph, max_pairs=max_pairs)
     lat, halo_ms, stage_ms, launches, counts, t_wall = time_resident(job, steps, warmup, flush)
+    if dump_dir is not None:
+        dump_outputs(job, steps - 1, dump_dir)
     # a halo region that was too small would have dropped records: look at the device-side counts once, after the frames
     halo_overflow = reduce_max(world, [1.0 if (job.exch is not None and job.exch.overflowed()) else 0.0])[0] > 0
     n_own_mean = float(np.mean([len(o["px"]) for o in job.own]))
@@ -719,7 +769,7 @@ def run_b200(args):
         time.sleep(0.3)
     steps = args.steps
     m = measure(args, args.workload, args.objects_per_gpu, world, rank, local_rank, flush, steps, args.warmup,
-                args.rebalance if world > 1 else 0, verify_kind=args.verify_kind)
+                args.rebalance if world > 1 else 0, verify_kind=args.verify_kind, dump_dir=args.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
     job = m["job"]
 
@@ -906,7 +956,14 @@ def main():
                     help="at N = 8: leave out the two configs[4] lines (10 M heavy-skew objects, 256 M-pair buffers) of the extras")
     ap.add_argument("--no-extras", dest="extras", action="store_false",
                     help="skip the strong-scaling / 10M lines that follow the headline at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed frame computed to DIR/<name>.npy (seeded sample of the pairs, per-object "
+                         "risk counts, total pairs): for comparing two builds output by output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     if args.objects_per_gpu is None:
         args.objects_per_gpu = {"cfg1_1k_city": 1000, "cfg2_5k_city": 5000, "cfg3_100k_uniform2d": 100_000,
                                 "cfg4_1m_clustered3d": PER_GPU_DEFAULT, "cfg5_10m_skew3d": 1_250_000,

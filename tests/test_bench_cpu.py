@@ -24,6 +24,13 @@ def test_reference_arm_prints_one_contract_line():
     assert d["config"]["objects"] == 1000 and "gpu_arm" in d["config"] and d["gpu_launches"] == 0
 
 
+def test_refused_arguments():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], cwd=ROOT, capture_output=True, text=True,
+                           timeout=120)
+        assert r.returncode == 2 and "error:" in r.stderr, (extra, r.stderr[-2000:])
+
+
 def test_both_arms_build_the_same_config_object():
     sys.path.insert(0, ROOT)
     import bench
