@@ -5,8 +5,10 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "rcd_common.cuh"
@@ -25,9 +27,152 @@ thread_local std::string g_create_error;
 constexpr u32 CELLS_CAP_MAX = 1u << 24;
 constexpr u32 CELLS_CAP_MIN = 1u << 16;
 
+// ---- owning handles of CUDA resources: move-only, released by the destructor --------------------------------
+template <typename T, cudaError_t (*Release)(T)>
+class Owned {
+public:
+    Owned() = default;
+    Owned(Owned &&o) noexcept : v_(std::exchange(o.v_, nullptr)) {}
+    Owned &operator=(Owned &&o) noexcept {
+        if (this != &o) { reset(); v_ = std::exchange(o.v_, nullptr); }
+        return *this;
+    }
+    ~Owned() { reset(); }
+    void reset() {
+        if (v_) Release(v_);
+        v_ = nullptr;
+    }
+    T get() const { return v_; }
+    operator T() const { return v_; }
+
+protected:
+    T v_ = nullptr;
+};
+
+template <typename T> cudaError_t alloc_device(T **p, size_t bytes) { return cudaMalloc(reinterpret_cast<void **>(p), bytes); }
+template <typename T> cudaError_t free_device(T *p) { return cudaFree(p); }
+template <typename T> cudaError_t alloc_host(T **p, size_t bytes) { return cudaMallocHost(reinterpret_cast<void **>(p), bytes); }
+template <typename T> cudaError_t free_host(T *p) { return cudaFreeHost(p); }
+
+// An array of T (at least one element); kernels take it as a T *.
+template <typename T, cudaError_t (*Alloc)(T **, size_t), cudaError_t (*Free)(T *)>
+struct Buffer : Owned<T *, Free> {
+    cudaError_t alloc(size_t count = 1) {
+        this->reset();
+        return Alloc(&this->v_, std::max<size_t>(count, 1) * sizeof(T));
+    }
+    T *operator->() const { return this->v_; }
+};
+template <typename T> using DevBuf = Buffer<T, alloc_device<T>, free_device<T>>;
+template <typename T> using HostBuf = Buffer<T, alloc_host<T>, free_host<T>>;  // pinned
+
+struct Stream : Owned<cudaStream_t, cudaStreamDestroy> {
+    cudaError_t create(int priority = 0) {
+        reset();
+        return cudaStreamCreateWithPriority(&v_, cudaStreamNonBlocking, priority);
+    }
+};
+
+struct Event : Owned<cudaEvent_t, cudaEventDestroy> {
+    cudaError_t create(unsigned flags = cudaEventDisableTiming) {
+        reset();
+        return cudaEventCreateWithFlags(&v_, flags);
+    }
+};
+
+struct GraphExec : Owned<cudaGraphExec_t, cudaGraphExecDestroy> {
+    cudaError_t instantiate(cudaGraph_t g) {
+        reset();
+        return cudaGraphInstantiate(&v_, g, 0);
+    }
+};
+
 struct Stage {
-    cudaEvent_t begin = nullptr, end = nullptr;
+    Event begin, end;
     bool used = false;
+};
+
+// The cell-ordered index a step derives from the objects; a graph replay restores it.
+struct IndexState {
+    GridParams grid = {};
+    bool valid = false;
+    float cell_req = 0.0f;
+    int sorted_buf = 0;
+    int qorder_kind = 0;   // 0 none, 1 balls (radius queries), 2 capsules (predict queries)
+    int q_sorted_buf = 0;
+};
+
+// What a frame writes.  A pending delivery still reads the previous frame's set, so the handle keeps a twin.
+struct FrameBuffers {
+    DevBuf<rcd_pair> out;
+    DevBuf<Counters> counters;
+    DevBuf<u32> risk_count;
+};
+
+// Resources of the pipelined deliveries (rcd_download_begin / _finish, rcd_summary_begin / _finish), made at
+// their first use.  Built completely before the handle takes them, so a failed attempt leaves nothing behind.
+struct Delivery {
+    HostBuf<Counters> counters_host;             // snapshot of the pending frame's totals
+    HostBuf<AlertCounters> alert_counters_host;
+    Stream copy_stream;
+    Event pend_event;
+    // summary deliveries fold the frame into the alert table on a stream of their own, next to the kernels of the
+    // following frame (random 40-byte accesses beside ALU-bound pair kernels)
+    Stream alert_stream;
+    Event ev_frame_done, ev_alert_done;
+};
+
+// The kernels of one frame variant (index: the variant number of step_impl).
+struct FrameKernels {
+    void (*tile_plan)(PairParams);
+    void (*pairs)(PairParams);
+    void (*pairs_overflow)(PairParams);
+    void (*narrow)(PairParams);
+    void (*exact)(PairParams);
+    void (*exact_resolved)(PairParams);  // second k_exact launch (RESOLVED records); null: none
+};
+
+const FrameKernels FRAME_KERNELS[5] = {
+    // 0: detect
+    {k_tile_plan<RCD_MODE_DETECT>, k_pairs<RCD_MODE_DETECT, false, false>, k_pairs<RCD_MODE_DETECT, false, true>,
+     k_narrow<RCD_MODE_DETECT, false>, k_exact<RCD_MODE_DETECT, 0>, nullptr},
+    // 1: predict
+    {k_tile_plan<RCD_MODE_PREDICT>, k_pairs<RCD_MODE_PREDICT, false, false>, k_pairs<RCD_MODE_PREDICT, false, true>,
+     k_narrow<RCD_MODE_PREDICT, false>, k_exact<RCD_MODE_PREDICT, 1>, k_exact<RCD_MODE_PREDICT, 2>},
+    // 2: predict, counting candidates (RCD_FLAG_COUNT_PREDICT_CANDIDATES)
+    {k_tile_plan<RCD_MODE_PREDICT>, k_pairs<RCD_MODE_PREDICT, true, false>, k_pairs<RCD_MODE_PREDICT, true, true>,
+     k_narrow<RCD_MODE_PREDICT, true>, k_exact<RCD_MODE_PREDICT, 1>, k_exact<RCD_MODE_PREDICT, 2>},
+    // 3: compute node
+    {k_tile_plan<RCD_MODE_COMPUTE_NODE>, k_pairs<RCD_MODE_COMPUTE_NODE, false, false>,
+     k_pairs<RCD_MODE_COMPUTE_NODE, false, true>, k_narrow<RCD_MODE_COMPUTE_NODE, false>, k_exact<RCD_MODE_COMPUTE_NODE, 0>,
+     nullptr},
+    // 4: detect + predict in one sweep
+    {k_tile_plan<RCD_MODE_PREDICT>, k_pairs<MODE_PREDICT_WITH_DETECT, false, false>,
+     k_pairs<MODE_PREDICT_WITH_DETECT, false, true>, k_narrow<MODE_PREDICT_WITH_DETECT, false>,
+     k_exact<MODE_PREDICT_WITH_DETECT, 1>, k_exact<MODE_PREDICT_WITH_DETECT, 2>},
+};
+
+// RCD_FLAG_GRAPH: the launch sequence of a step is a pure function of this key (every other kernel argument is
+// a buffer that lives as long as the handle).
+struct StepKey {
+    int32_t mode = -1;
+    float R = 0, T = 0, pt = 0, thr = 0, index_cell_req = 0;
+    u64 n = 0, n_owned = 0;
+    int index_valid = 0, sorted_buf = 0, frame_done = 0, qorder_kind = 0, q_sorted_buf = 0;
+    const void *out = nullptr;
+    bool operator==(const StepKey &o) const {
+        return mode == o.mode && R == o.R && T == o.T && pt == o.pt && thr == o.thr && index_cell_req == o.index_cell_req &&
+               n == o.n && n_owned == o.n_owned && index_valid == o.index_valid && sorted_buf == o.sorted_buf &&
+               frame_done == o.frame_done && qorder_kind == o.qorder_kind && q_sorted_buf == o.q_sorted_buf && out == o.out;
+    }
+};
+
+struct StepGraph {
+    GraphExec exec;
+    StepKey key;
+    IndexState idx;
+    int last_mode = 0;
+    u64 launches = 0;
 };
 
 }  // namespace
@@ -35,61 +180,55 @@ struct Stage {
 struct rcd_handle_s {
     int device = 0;
     u32 flags = 0;
-    cudaStream_t stream = nullptr;
+    int sms = 1;  // multiprocessors of the device
+    Stream stream;
     u64 cap = 0, max_pairs = 0;
     u64 n = 0, n_owned = 0;
 
-    float *in_f[11] = {};
-    uint8_t *in_type = nullptr, *in_pattern = nullptr;
-    u32 *in_id = nullptr;
+    DevBuf<float> in_f[11];
+    DevBuf<uint8_t> in_type, in_pattern;
+    DevBuf<u32> in_id;
 
-    u32 *keys[2] = {}, *vals[2] = {};
-    u32 *hist = nullptr, *tile_status = nullptr, *tile_counter = nullptr;
+    DevBuf<u32> keys[2], vals[2];
+    DevBuf<u32> hist, tile_status, tile_counter;
     size_t tile_status_words = 0;
-    int sorted_buf = 0;
 
-    float4 *P0 = nullptr, *P1 = nullptr, *P2 = nullptr;
-    float4 *U = nullptr;  // packed 48-byte records in upload order
-    u32 *sorted_slot = nullptr;
-    u32 *sorted_id = nullptr;   // caller ids in cell order (the frame kernels never touch the upload buffers)
+    DevBuf<float4> P0, P1, P2;
+    DevBuf<float4> U;  // packed 48-byte records in upload order
+    DevBuf<u32> sorted_slot;
+    DevBuf<u32> sorted_id;   // caller ids in cell order (the frame kernels never touch the upload buffers)
     // uploads from host memory run on their own stream and overlap the previous frame: the upload buffers are
     // free again as soon as that frame's index is built (k_pack_keys + k_reorder have consumed them)
-    cudaStream_t up_stream = nullptr;
-    cudaEvent_t ev_upload_done = nullptr, ev_inputs_free = nullptr;
+    Stream up_stream;
+    Event ev_upload_done, ev_inputs_free;
     bool upload_pending = false, inputs_busy = false, capturing = false;
-    u32 *cell_begin = nullptr;  // [cells_cap + 1] dense cell table
+    DevBuf<u32> cell_begin;  // [cells_cap + 1] dense cell table
     u32 cells_cap = 0;
     float cell_scale = 0.5f;    // grid cell edge (x, y) as a fraction of the query radius
-    u32 *qkeys[2] = {}, *qvals[2] = {};  // query order: Morton keys of the query volumes + permutation
-    int q_sorted_buf = 0;
-    int qorder_kind = 0;        // 0 none, 1 balls (radius queries), 2 capsules (predict queries)
+    DevBuf<u32> qkeys[2], qvals[2];  // query order: Morton keys of the query volumes + permutation
 
     bool world_static = false;
     float wmin[3] = {}, wmax[3] = {};
-    int *bbox_dev = nullptr;
-    int *bbox_host = nullptr;  // pinned
-    GridParams grid = {};
-    bool index_valid = false;
-    float index_cell_req = 0.0f;
+    DevBuf<int> bbox_dev;
+    HostBuf<int> bbox_host;
+    IndexState idx;
 
-    rcd_pair *out = nullptr;
-    Counters *counters = nullptr;
-    Counters *counters_host = nullptr;  // pinned
-    u32 *cand_count = nullptr;
-    u32 *risk_count = nullptr, *risk_count_alt = nullptr;
-    u32 *pair_tile_counter = nullptr;
-    QEntry *q3 = nullptr;
+    FrameBuffers bufs[2];  // the current set and the twin of the pipelined deliveries
+    int cur = 0;
+    HostBuf<Counters> counters_host;
+    DevBuf<u32> cand_count;
+    DevBuf<u32> pair_tile_counter;
+    DevBuf<QEntry> q3;
     u32 qcap = 0;
-    uint2 *qa = nullptr;        // pair queue k_pairs -> k_narrow
-    u32 *qa_fill = nullptr;
+    DevBuf<uint2> qa;        // pair queue k_pairs -> k_narrow
+    DevBuf<u32> qa_fill;
     u32 qa_blocks_cap = 0;
-    uint4 *ovf = nullptr;       // work items (or rests of them) left to the overflow pass of k_pairs
+    DevBuf<uint4> ovf;       // work items (or rests of them) left to the overflow pass of k_pairs
     u32 ovf_cap = 0;
-    uint4 *items = nullptr;     // work items of k_pairs (k_tile_plan)
+    DevBuf<uint4> items;     // work items of k_pairs (k_tile_plan)
     u32 items_cap = 0;
-    int4 *tile_box = nullptr;   // [2 * tiles]
-    uint2 *tile_rowx = nullptr; // [TILE_ROWS * tiles]
-    int stage_blocks = 0, stage_blocks_sms = 148;
+    DevBuf<int4> tile_box;   // [2 * tiles]
+    DevBuf<uint2> tile_rowx; // [TILE_ROWS * tiles]
     int narrow_blocks[5] = {0, 0, 0, 0, 0};
     int pair_blocks[5] = {0, 0, 0, 0, 0};  // resident blocks per SM x SMs, per kernel variant
     bool frame_done = false;
@@ -98,47 +237,18 @@ struct rcd_handle_s {
     Stage stages[3][RCD_NUM_STAGES];  // per frame mode
     int stage_mode = 0;
     float cn_prediction_time = 5.0f, cn_risk_threshold = 0.5f;
-    Sample64 *traj = nullptr;  // trajectory rings, [max_history][cap]
-    u32 *traj_count = nullptr;
+    DevBuf<Sample64> traj;  // trajectory rings, [max_history][cap]
+    DevBuf<u32> traj_count;
     u32 traj_len = 0;
     u64 launches = 0;
     // CUDA-graph replay of rcd_step (RCD_FLAG_GRAPH)
-    struct StepKey {
-        int32_t mode = -1;
-        float R = 0, T = 0, pt = 0, thr = 0, index_cell_req = 0;
-        u64 n = 0, n_owned = 0;
-        int index_valid = 0, sorted_buf = 0, frame_done = 0, qorder_kind = 0, q_sorted_buf = 0;
-        const void *out = nullptr;
-        bool operator==(const StepKey &o) const {
-            return mode == o.mode && R == o.R && T == o.T && pt == o.pt && thr == o.thr && index_cell_req == o.index_cell_req &&
-                   n == o.n && n_owned == o.n_owned && index_valid == o.index_valid && sorted_buf == o.sorted_buf &&
-                   frame_done == o.frame_done && qorder_kind == o.qorder_kind && q_sorted_buf == o.q_sorted_buf && out == o.out;
-        }
-    };
-    struct StepGraph {
-        cudaGraphExec_t exec = nullptr;
-        StepKey key;
-        GridParams grid = {};
-        float index_cell_req = 0;
-        int sorted_buf = 0, last_mode = 0, qorder_kind = 0, q_sorted_buf = 0;
-        u64 launches = 0;
-    };
     StepGraph graphs[4];
     int graph_next = 0;
     StepKey graph_candidates[4];  // keys seen recently (twin pair buffers make consecutive frames alternate)
     int graph_cand_next = 0;
     bool graph_broken = false;
     u64 graph_replays = 0;
-    // pipelined delivery (rcd_download_begin / _finish): twin pair buffer + totals, copy stream
-    rcd_pair *out_alt = nullptr;
-    Counters *counters_alt = nullptr;
-    Counters *pend_counters_host = nullptr;  // pinned snapshot of the pending frame's totals
-    cudaStream_t copy_stream = nullptr;
-    cudaEvent_t pend_event = nullptr;
-    // summary deliveries fold the frame into the alert table on a stream of their own, next to the kernels of the
-    // following frame (random 40-byte accesses beside ALU-bound pair kernels)
-    cudaStream_t alert_stream = nullptr;
-    cudaEvent_t ev_frame_done = nullptr, ev_alert_done = nullptr;
+    Delivery dl;
     bool alert_async = false;  // work on alert_stream the handle's stream has not been ordered after yet
     u64 last_n_pairs = 0;      // emitted pairs of the last frame whose totals reached the host (sizes the alert fold's grid)
     u64 last_n_detect_end = 0; // ... and where its records with predicted = 0 ended (grid of the fold's detect pass)
@@ -146,19 +256,35 @@ struct rcd_handle_s {
     rcd_pair *pend_dev = nullptr, *pend_out = nullptr;
     u64 pend_cap = 0, pend_n = 0, pend_n_owned = 0;
     int pend_kind = 0;                       // 0 pairs, 1 compact pairs, 2 summary (alert events + risk counts)
-    rcd_pair_compact *compact_dev = nullptr; // scratch of rcd_download_begin_compact
+    DevBuf<rcd_pair_compact> compact_dev;    // scratch of rcd_download_begin_compact
     rcd_pair_compact *pend_out_compact = nullptr;
     u32 *pend_risk = nullptr;
     rcd_alert_event *pend_ev = nullptr;
-    AlertCounters *pend_alert_counters_host = nullptr;  // pinned
     // alert table (rcd_alerts.cuh)
-    AlertEntry *alert_tab[2] = {nullptr, nullptr};
+    DevBuf<AlertEntry> alert_tab[2];
     int alert_cur = 0;
     u64 alert_cap = 0, alert_ev_cap = 0;
-    rcd_alert_event *alert_ev = nullptr, *alert_ev_alt = nullptr;  // (twin: summary deliveries in flight)
-    AlertCounters *alert_counters = nullptr;
-    AlertCounters *alert_counters_host = nullptr;  // pinned
+    DevBuf<rcd_alert_event> alert_ev, alert_ev_alt;  // (twin: summary deliveries in flight)
+    DevBuf<AlertCounters> alert_counters;
+    HostBuf<AlertCounters> alert_counters_host;
     std::string err;
+
+    FrameBuffers &fb() { return bufs[cur]; }
+    // The previous frame is being delivered: the next one writes into the twin buffers.
+    void flip() {
+        cur ^= 1;
+        flip_pending = false;
+    }
+
+    // The streams finish their work before the members release themselves.
+    ~rcd_handle_s() {
+        cudaSetDevice(device);
+        if (up_stream) cudaStreamSynchronize(up_stream);
+        if (stream) cudaStreamSynchronize(stream);
+        if (dl.alert_stream) cudaStreamSynchronize(dl.alert_stream);
+        if (dl.copy_stream) cudaStreamSynchronize(dl.copy_stream);
+        (void)cudaGetLastError();
+    }
 };
 
 namespace {
@@ -177,6 +303,13 @@ int fail(rcd_handle h, int code, const std::string &msg) {
         }                                                                                          \
     } while (0)
 
+// Return a status other than RCD_OK to the caller.
+#define RC_TRY(call)                                                                               \
+    do {                                                                                           \
+        const int rc__ = (call);                                                                   \
+        if (rc__ != RCD_OK) return rc__;                                                           \
+    } while (0)
+
 #define KERNEL_CHECK(h)                                                                            \
     do {                                                                                           \
         cudaError_t e__ = cudaGetLastError();                                                      \
@@ -184,9 +317,12 @@ int fail(rcd_handle h, int code, const std::string &msg) {
         ++(h)->launches;                                                                           \
     } while (0)
 
-template <typename T>
-cudaError_t dev_alloc(T **p, size_t count) {
-    return cudaMalloc(reinterpret_cast<void **>(p), std::max<size_t>(count, 1) * sizeof(T));
+// Mark the profiling stages of one frame mode (mode < 0: of every mode, upload and download included) unused.
+void reset_stages(rcd_handle h, int mode) {
+    for (int m = 0; m < 3; ++m)
+        for (int s = 0; s < RCD_NUM_STAGES; ++s)
+            if (mode < 0 || (m == mode && s != RCD_STAGE_UPLOAD && s != RCD_STAGE_DOWNLOAD && s != RCD_STAGE_TOTAL))
+                h->stages[m][s].used = false;
 }
 
 void stage_begin(rcd_handle h, int s, cudaStream_t on = nullptr) {
@@ -224,6 +360,36 @@ InputState input_state(rcd_handle h) {
     in.size = h->in_f[9]; in.heading = h->in_f[10];
     in.type = h->in_type; in.pattern = h->in_pattern; in.id = h->in_id;
     return in;
+}
+
+MutableState mutable_state(rcd_handle h) {
+    MutableState st;
+    for (int k = 0; k < 11; ++k) st.f[k] = h->in_f[k];
+    st.type = h->in_type; st.pattern = h->in_pattern; st.id = h->in_id;
+    return st;
+}
+
+// A frame's totals reached the host: they size the next alert fold's grid, and fill `out` unless it is null.
+void fill_counts(rcd_handle h, const Counters &c, u64 n, u64 n_owned, rcd_counts_t *out) {
+    h->last_n_pairs = c.n_pairs;
+    h->last_n_detect_end = c.n_detect_end;
+    if (!out) return;
+    out->n_objects = n;
+    out->n_owned = n_owned;
+    out->n_candidates = c.n_candidates;
+    out->n_potential = c.n_potential;
+    out->n_pairs = c.n_pairs;
+    out->n_high_risk = c.n_high_risk;
+    out->n_written = std::min<u64>(c.n_pairs, h->max_pairs);
+    for (int k = 0; k < 4; ++k) out->n_alerts[k] = c.n_alerts[k];
+    out->n_exact = c.n_exact;
+    out->n_fallback = c.n_fallback;
+}
+
+void fill_alert_stats(const AlertCounters &c, rcd_alert_stats *st) {
+    if (!st) return;
+    st->n_events = c.n_events; st->n_created = c.n_created; st->n_changed = c.n_changed;
+    st->n_refreshed = c.n_refreshed; st->n_expired = c.n_expired; st->n_live = c.n_live; st->n_dropped = c.n_dropped;
 }
 
 // Grid for a query radius.  The pair kernel and the radius queries walk the cells under the bounding box of
@@ -268,18 +434,15 @@ int key_passes(u32 ncells) {
 // Build the cell-ordered index for the current objects (keys -> sort -> reorder + ranges).
 int build_index(rcd_handle h, float cell_req) {
     const u32 n = (u32)h->n;
-    if (h->index_valid && h->index_cell_req == cell_req) return RCD_OK;
-    h->index_valid = false;
-    h->qorder_kind = 0;
-    {
-        int rcw = wait_upload(h);
-        if (rcw) return rcw;
-    }
+    if (h->idx.valid && h->idx.cell_req == cell_req) return RCD_OK;
+    h->idx.valid = false;
+    h->idx.qorder_kind = 0;
+    RC_TRY(wait_upload(h));
     if (n == 0) {
         float z[3] = {0, 0, 0};
-        h->grid = make_grid(z, z, cell_req, h->cell_scale, h->cells_cap);
-        h->index_valid = true;
-        h->index_cell_req = cell_req;
+        h->idx.grid = make_grid(z, z, cell_req, h->cell_scale, h->cells_cap);
+        h->idx.valid = true;
+        h->idx.cell_req = cell_req;
         return RCD_OK;
     }
     if (!h->world_static) {
@@ -297,8 +460,8 @@ int build_index(rcd_handle h, float cell_req) {
             if (!(h->wmin[d] <= h->wmax[d])) h->wmin[d] = h->wmax[d] = 0.0f;  // no finite coordinate
         }
     }
-    h->grid = make_grid(h->wmin, h->wmax, cell_req, h->cell_scale, h->cells_cap);
-    const GridParams g = h->grid;
+    h->idx.grid = make_grid(h->wmin, h->wmax, cell_req, h->cell_scale, h->cells_cap);
+    const GridParams g = h->idx.grid;
     const int passes = key_passes(g.ncells + 1);  // + the cell of the objects without a position (rcd_index.cuh)
     const u32 tiles = (n + SORT_TILE - 1) / SORT_TILE;
 
@@ -317,24 +480,22 @@ int build_index(rcd_handle h, float cell_req) {
     stage_end(h, RCD_STAGE_KEYS);
 
     stage_begin(h, RCD_STAGE_SORT);
-    const int cur = launch_onesweep(h->keys, h->vals, n, passes, h->hist, h->tile_status, h->tile_counter, h->stream);
+    u32 *const keys[2] = {h->keys[0], h->keys[1]}, *const vals[2] = {h->vals[0], h->vals[1]};
+    const int cur = launch_onesweep(keys, vals, n, passes, h->hist, h->tile_status, h->tile_counter, h->stream);
     KERNEL_CHECK(h);
-    h->sorted_buf = cur;
+    h->idx.sorted_buf = cur;
     stage_end(h, RCD_STAGE_SORT);
 
     stage_begin(h, RCD_STAGE_REORDER);
     k_reorder<<<(n + REORDER_THREADS - 1) / REORDER_THREADS, REORDER_THREADS, 0, h->stream>>>(
         h->vals[cur], n, h->U, h->P0, h->P1, h->P2, h->sorted_slot, h->sorted_id);
     KERNEL_CHECK(h);
-    {
-        int rcr = release_inputs(h);
-        if (rcr) return rcr;
-    }
+    RC_TRY(release_inputs(h));
     k_cell_table<<<(g.ncells + 1 + CT_CELLS - 1) / CT_CELLS, CT_THREADS, 0, h->stream>>>(h->keys[cur], n, g.ncells + 1, h->cell_begin);
     KERNEL_CHECK(h);
     stage_end(h, RCD_STAGE_REORDER);
-    h->index_valid = true;
-    h->index_cell_req = cell_req;
+    h->idx.valid = true;
+    h->idx.cell_req = cell_req;
     return RCD_OK;
 }
 
@@ -342,8 +503,8 @@ int build_index(rcd_handle h, float cell_req) {
 // volumes overlap.  kind 1: balls about the objects; kind 2: capsules of the predict queries.
 int build_query_order(rcd_handle h, int kind) {
     const u32 n = (u32)h->n;
-    if (h->qorder_kind == kind || n == 0) return RCD_OK;
-    const GridParams g = h->grid;
+    if (h->idx.qorder_kind == kind || n == 0) return RCD_OK;
+    const GridParams g = h->idx.grid;
     const u32 tiles = (n + SORT_TILE - 1) / SORT_TILE;
     stage_begin(h, RCD_STAGE_QORDER);
     CUDA_TRY(h, cudaMemsetAsync(h->hist, 0, MAX_PASSES * RADIX * sizeof(u32), h->stream));
@@ -368,11 +529,12 @@ int build_query_order(rcd_handle h, int kind) {
     KERNEL_CHECK(h);
     k_scan_hist<<<1, RADIX, 0, h->stream>>>(h->hist, QKEY_PASSES);
     KERNEL_CHECK(h);
-    const int cur = launch_onesweep(h->qkeys, h->qvals, n, QKEY_PASSES, h->hist, h->tile_status, h->tile_counter, h->stream);
+    u32 *const keys[2] = {h->qkeys[0], h->qkeys[1]}, *const vals[2] = {h->qvals[0], h->qvals[1]};
+    const int cur = launch_onesweep(keys, vals, n, QKEY_PASSES, h->hist, h->tile_status, h->tile_counter, h->stream);
     KERNEL_CHECK(h);
     stage_end(h, RCD_STAGE_QORDER);
-    h->q_sorted_buf = cur;
-    h->qorder_kind = kind;
+    h->idx.q_sorted_buf = cur;
+    h->idx.qorder_kind = kind;
     return RCD_OK;
 }
 
@@ -385,8 +547,7 @@ int copy_in(rcd_handle h, void *dst, const void *src, size_t bytes, int32_t srck
 // released the upload buffers.  Device memory: the handle's stream (ordered after a pending host upload).
 int upload_stream(rcd_handle h, int32_t src, cudaStream_t *on) {
     if (src == RCD_SRC_DEVICE) {
-        int rc = wait_upload(h);
-        if (rc) return rc;
+        RC_TRY(wait_upload(h));
         *on = h->stream;
         return RCD_OK;
     }
@@ -424,7 +585,7 @@ int rcd_create(const rcd_config *cfg, rcd_handle *out) {
         (void)cudaGetLastError();
         return fail(nullptr, RCD_ENODEVICE, "rcd_create: no usable CUDA device (this library has no CPU fallback)");
     }
-    rcd_handle h = new (std::nothrow) rcd_handle_s();
+    std::unique_ptr<rcd_handle_s> h(new (std::nothrow) rcd_handle_s());  // (a failed create frees what it made)
     if (!h) return fail(nullptr, RCD_ENOMEM, "rcd_create: out of host memory");
     h->device = cfg->device;
     h->flags = cfg->flags;
@@ -434,137 +595,86 @@ int rcd_create(const rcd_config *cfg, rcd_handle *out) {
     for (int d = 0; d < 3; ++d) { h->wmin[d] = cfg->world_min[d]; h->wmax[d] = cfg->world_max[d]; }
     h->cells_cap = (u32)std::min<u64>(std::max<u64>(4 * h->cap, CELLS_CAP_MIN), CELLS_CAP_MAX);
 
-#define CREATE_TRY(call)                                                                   \
-    do {                                                                                   \
-        cudaError_t e__ = (call);                                                          \
-        if (e__ != cudaSuccess) {                                                          \
-            int rc__ = fail(nullptr, e__ == cudaErrorMemoryAllocation ? RCD_ENOMEM : RCD_ECUDA, \
-                            std::string(#call) + ": " + cudaGetErrorString(e__));         \
-            rcd_destroy(h);                                                                \
-            return rc__;                                                                   \
-        }                                                                                  \
-    } while (0)
-
-    CREATE_TRY(cudaSetDevice(h->device));
+    CUDA_TRY(nullptr, cudaSetDevice(h->device));
+    {
+        int sms = 0;
+        CUDA_TRY(nullptr, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
+        h->sms = std::max(1, sms);
+    }
     {   // the frame's stream outranks the alert stream: block slots go to the frame's kernels first
         int least = 0, greatest = 0;
-        CREATE_TRY(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-        CREATE_TRY(cudaStreamCreateWithPriority(&h->stream, cudaStreamNonBlocking, greatest));
+        CUDA_TRY(nullptr, cudaDeviceGetStreamPriorityRange(&least, &greatest));
+        CUDA_TRY(nullptr, h->stream.create(greatest));
     }
-    CREATE_TRY(cudaStreamCreateWithFlags(&h->up_stream, cudaStreamNonBlocking));
-    CREATE_TRY(cudaEventCreateWithFlags(&h->ev_upload_done, cudaEventDisableTiming));
-    CREATE_TRY(cudaEventCreateWithFlags(&h->ev_inputs_free, cudaEventDisableTiming));
+    CUDA_TRY(nullptr, h->up_stream.create());
+    CUDA_TRY(nullptr, h->ev_upload_done.create());
+    CUDA_TRY(nullptr, h->ev_inputs_free.create());
     const size_t cap = (size_t)h->cap;
     for (int k = 0; k < 11; ++k) {
-        CREATE_TRY(dev_alloc(&h->in_f[k], cap));
-        CREATE_TRY(cudaMemsetAsync(h->in_f[k], 0, cap * sizeof(float), h->stream));
+        CUDA_TRY(nullptr, h->in_f[k].alloc(cap));
+        CUDA_TRY(nullptr, cudaMemsetAsync(h->in_f[k], 0, cap * sizeof(float), h->stream));
     }
-    CREATE_TRY(dev_alloc(&h->in_type, cap));
-    CREATE_TRY(dev_alloc(&h->in_pattern, cap));
-    CREATE_TRY(dev_alloc(&h->in_id, cap));
+    CUDA_TRY(nullptr, h->in_type.alloc(cap));
+    CUDA_TRY(nullptr, h->in_pattern.alloc(cap));
+    CUDA_TRY(nullptr, h->in_id.alloc(cap));
     for (int k = 0; k < 2; ++k) {
-        CREATE_TRY(dev_alloc(&h->keys[k], cap + 4));
-        CREATE_TRY(dev_alloc(&h->vals[k], cap + 4));
+        CUDA_TRY(nullptr, h->keys[k].alloc(cap + 4));
+        CUDA_TRY(nullptr, h->vals[k].alloc(cap + 4));
     }
-    CREATE_TRY(dev_alloc(&h->hist, MAX_PASSES * RADIX));
+    CUDA_TRY(nullptr, h->hist.alloc(MAX_PASSES * RADIX));
     h->tile_status_words = (size_t)MAX_PASSES * ((cap + SORT_TILE - 1) / SORT_TILE) * RADIX;
-    CREATE_TRY(dev_alloc(&h->tile_status, h->tile_status_words));
-    CREATE_TRY(dev_alloc(&h->tile_counter, MAX_PASSES));
-    CREATE_TRY(dev_alloc(&h->P0, cap));
-    CREATE_TRY(dev_alloc(&h->P1, cap));
-    CREATE_TRY(dev_alloc(&h->P2, cap));
-    CREATE_TRY(dev_alloc(&h->U, 4 * (cap + 4)));
-    CREATE_TRY(dev_alloc(&h->sorted_slot, cap));
-    CREATE_TRY(dev_alloc(&h->sorted_id, cap));
-    CREATE_TRY(dev_alloc(&h->cell_begin, (size_t)h->cells_cap + 2));
+    CUDA_TRY(nullptr, h->tile_status.alloc(h->tile_status_words));
+    CUDA_TRY(nullptr, h->tile_counter.alloc(MAX_PASSES));
+    CUDA_TRY(nullptr, h->P0.alloc(cap));
+    CUDA_TRY(nullptr, h->P1.alloc(cap));
+    CUDA_TRY(nullptr, h->P2.alloc(cap));
+    CUDA_TRY(nullptr, h->U.alloc(4 * (cap + 4)));
+    CUDA_TRY(nullptr, h->sorted_slot.alloc(cap));
+    CUDA_TRY(nullptr, h->sorted_id.alloc(cap));
+    CUDA_TRY(nullptr, h->cell_begin.alloc((size_t)h->cells_cap + 2));
     for (int k = 0; k < 2; ++k) {
-        CREATE_TRY(dev_alloc(&h->qkeys[k], cap + 4));
-        CREATE_TRY(dev_alloc(&h->qvals[k], cap + 4));
+        CUDA_TRY(nullptr, h->qkeys[k].alloc(cap + 4));
+        CUDA_TRY(nullptr, h->qvals[k].alloc(cap + 4));
     }
     if (const char *e = getenv("RCD_CELL_SCALE")) {  // kernel-tuning experiments only
         const double v = atof(e);
         if (v >= 0.05 && v <= 4.0) h->cell_scale = (float)v;
     }
-    CREATE_TRY(dev_alloc(&h->bbox_dev, 6));
-    CREATE_TRY(cudaMallocHost(reinterpret_cast<void **>(&h->bbox_host), 6 * sizeof(int)));
-    CREATE_TRY(dev_alloc(&h->out, (size_t)h->max_pairs));
-    CREATE_TRY(dev_alloc(&h->counters, 1));
-    CREATE_TRY(cudaMallocHost(reinterpret_cast<void **>(&h->counters_host), sizeof(Counters)));
-    CREATE_TRY(dev_alloc(&h->cand_count, cap));
-    CREATE_TRY(dev_alloc(&h->risk_count, cap));
-    CREATE_TRY(dev_alloc(&h->pair_tile_counter, 2));
+    CUDA_TRY(nullptr, h->bbox_dev.alloc(6));
+    CUDA_TRY(nullptr, h->bbox_host.alloc(6));
+    CUDA_TRY(nullptr, h->bufs[0].out.alloc(h->max_pairs));
+    CUDA_TRY(nullptr, h->bufs[0].counters.alloc());
+    CUDA_TRY(nullptr, h->counters_host.alloc());
+    CUDA_TRY(nullptr, h->cand_count.alloc(cap));
+    CUDA_TRY(nullptr, h->bufs[0].risk_count.alloc(cap));
+    CUDA_TRY(nullptr, h->pair_tile_counter.alloc(2));
     // the fp32 stages forward about 5 candidate entries per emitted pair on clustered frames; a full
     // queue is not an error (the pair is then finished in place) but it is slower
     h->qcap = (u32)std::min<u64>(6 * h->max_pairs + 65536, (1ull << 31) - (1ull << 24));  // (32-bit entry indices)
-    CREATE_TRY(dev_alloc(&h->q3, (size_t)h->qcap));
+    CUDA_TRY(nullptr, h->q3.alloc(h->qcap));
     // the S1 filter forwards ~60 (predict) / ~20 (detect) pairs per object at the density of the bench frame;
     // the pair queue is handed out in blocks of QA_BLOCK entries, one per warp at a time
     // (+ one partly filled block per resident warp of k_pairs)
     h->qa_blocks_cap = (u32)(h->qcap / QA_BLOCK + 148 * 8 * PAIR_WARPS);
-    CREATE_TRY(dev_alloc(&h->qa, (size_t)h->qa_blocks_cap * QA_BLOCK));
-    CREATE_TRY(dev_alloc(&h->qa_fill, (size_t)h->qa_blocks_cap));
+    CUDA_TRY(nullptr, h->qa.alloc((size_t)h->qa_blocks_cap * QA_BLOCK));
+    CUDA_TRY(nullptr, h->qa_fill.alloc(h->qa_blocks_cap));
     h->items_cap = (u32)((cap / TQ + 1) * ITEMS_PER_TILE_CAP);  // k_tile_plan never makes more
-    CREATE_TRY(dev_alloc(&h->items, (size_t)h->items_cap));
-    CREATE_TRY(dev_alloc(&h->tile_box, 2 * (cap / TQ + 1)));
-    CREATE_TRY(dev_alloc(&h->tile_rowx, (size_t)TILE_ROWS * (cap / TQ + 1)));
+    CUDA_TRY(nullptr, h->items.alloc(h->items_cap));
+    CUDA_TRY(nullptr, h->tile_box.alloc(2 * (cap / TQ + 1)));
+    CUDA_TRY(nullptr, h->tile_rowx.alloc((size_t)TILE_ROWS * (cap / TQ + 1)));
     h->ovf_cap = h->items_cap;  // every work item is handed over at most once
-    CREATE_TRY(dev_alloc(&h->ovf, (size_t)h->ovf_cap));
-    for (int m = 0; m < 3; ++m)
-        for (int s = 0; s < RCD_NUM_STAGES; ++s) {
-            CREATE_TRY(cudaEventCreate(&h->stages[m][s].begin));
-            CREATE_TRY(cudaEventCreate(&h->stages[m][s].end));
+    CUDA_TRY(nullptr, h->ovf.alloc(h->ovf_cap));
+    for (auto &mode : h->stages)
+        for (Stage &st : mode) {
+            CUDA_TRY(nullptr, st.begin.create(cudaEventDefault));
+            CUDA_TRY(nullptr, st.end.create(cudaEventDefault));
         }
-    CREATE_TRY(cudaStreamSynchronize(h->stream));
-#undef CREATE_TRY
-    *out = h;
+    CUDA_TRY(nullptr, cudaStreamSynchronize(h->stream));
+    *out = h.release();
     return RCD_OK;
 }
 
 int rcd_destroy(rcd_handle h) {
-    if (!h) return RCD_OK;
-    cudaSetDevice(h->device);
-    if (h->up_stream) cudaStreamSynchronize(h->up_stream);
-    if (h->stream) cudaStreamSynchronize(h->stream);
-    if (h->alert_stream) cudaStreamSynchronize(h->alert_stream);
-    if (h->copy_stream) cudaStreamSynchronize(h->copy_stream);
-    for (int k = 0; k < 11; ++k) cudaFree(h->in_f[k]);
-    cudaFree(h->sorted_id);
-    if (h->ev_upload_done) cudaEventDestroy(h->ev_upload_done);
-    if (h->ev_inputs_free) cudaEventDestroy(h->ev_inputs_free);
-    if (h->up_stream) cudaStreamDestroy(h->up_stream);
-    cudaFree(h->in_type); cudaFree(h->in_pattern); cudaFree(h->in_id);
-    for (int k = 0; k < 2; ++k) { cudaFree(h->keys[k]); cudaFree(h->vals[k]); }
-    cudaFree(h->hist); cudaFree(h->tile_status); cudaFree(h->tile_counter);
-    cudaFree(h->P0); cudaFree(h->P1); cudaFree(h->P2); cudaFree(h->sorted_slot);
-    cudaFree(h->U);
-    cudaFree(h->cell_begin); cudaFree(h->bbox_dev);
-    for (int k = 0; k < 2; ++k) { cudaFree(h->qkeys[k]); cudaFree(h->qvals[k]); }
-    cudaFree(h->qa); cudaFree(h->qa_fill); cudaFree(h->ovf); cudaFree(h->items); cudaFree(h->tile_box); cudaFree(h->tile_rowx);
-    if (h->bbox_host) cudaFreeHost(h->bbox_host);
-    cudaFree(h->out); cudaFree(h->counters); cudaFree(h->cand_count); cudaFree(h->pair_tile_counter);
-    cudaFree(h->q3);
-    cudaFree(h->traj); cudaFree(h->traj_count);
-    for (auto &g : h->graphs)
-        if (g.exec) cudaGraphExecDestroy(g.exec);
-    cudaFree(h->out_alt); cudaFree(h->counters_alt); cudaFree(h->risk_count); cudaFree(h->risk_count_alt);
-    cudaFree(h->compact_dev); cudaFree(h->alert_ev_alt);
-    if (h->pend_alert_counters_host) cudaFreeHost(h->pend_alert_counters_host);
-    if (h->pend_counters_host) cudaFreeHost(h->pend_counters_host);
-    if (h->pend_event) cudaEventDestroy(h->pend_event);
-    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    if (h->alert_stream) { cudaStreamSynchronize(h->alert_stream); cudaStreamDestroy(h->alert_stream); }
-    if (h->ev_frame_done) cudaEventDestroy(h->ev_frame_done);
-    if (h->ev_alert_done) cudaEventDestroy(h->ev_alert_done);
-    cudaFree(h->alert_tab[0]); cudaFree(h->alert_tab[1]); cudaFree(h->alert_ev); cudaFree(h->alert_counters);
-    if (h->alert_counters_host) cudaFreeHost(h->alert_counters_host);
-    if (h->counters_host) cudaFreeHost(h->counters_host);
-    for (int m = 0; m < 3; ++m)
-        for (int s = 0; s < RCD_NUM_STAGES; ++s) {
-            if (h->stages[m][s].begin) cudaEventDestroy(h->stages[m][s].begin);
-            if (h->stages[m][s].end) cudaEventDestroy(h->stages[m][s].end);
-        }
-    if (h->stream) cudaStreamDestroy(h->stream);
-    (void)cudaGetLastError();
     delete h;
     return RCD_OK;
 }
@@ -576,43 +686,35 @@ int rcd_upload(rcd_handle h, uint64_t n, const float *px, const float *py, const
     if (n > h->cap) return fail(h, RCD_ECAPACITY, "rcd_upload: n exceeds max_objects");
     if (n && (!px || !py || !pz || !vx || !vy || !vz)) return fail(h, RCD_EINVAL, "rcd_upload: position/velocity arrays are required");
     CUDA_TRY(h, cudaSetDevice(h->device));
-    for (int m = 0; m < 3; ++m)
-        for (int s = 0; s < RCD_NUM_STAGES; ++s) h->stages[m][s].used = false;
+    reset_stages(h, -1);
     h->stage_mode = 0;
     cudaStream_t on = nullptr;
-    {
-        int rc = upload_stream(h, src, &on);
-        if (rc) return rc;
-    }
+    RC_TRY(upload_stream(h, src, &on));
     stage_begin(h, RCD_STAGE_UPLOAD, on);
     const float *f[11] = {px, py, pz, vx, vy, vz, ax, ay, az, size, heading};
     const size_t bytes = (size_t)n * sizeof(float);
     for (int k = 0; k < 11 && n; ++k) {
         if (f[k]) {
-            int rc = copy_in(h, h->in_f[k], f[k], bytes, src, on);
-            if (rc) return rc;
+            RC_TRY(copy_in(h, h->in_f[k], f[k], bytes, src, on));
         } else {
             CUDA_TRY(h, cudaMemsetAsync(h->in_f[k], 0, bytes, on));
         }
     }
     if (n) {
-        if (type) { int rc = copy_in(h, h->in_type, type, (size_t)n, src, on); if (rc) return rc; }
+        if (type) RC_TRY(copy_in(h, h->in_type, type, (size_t)n, src, on));
         else CUDA_TRY(h, cudaMemsetAsync(h->in_type, 0, (size_t)n, on));
         CUDA_TRY(h, cudaMemsetAsync(h->in_pattern, RCD_PAT_ACCELERATING, (size_t)n, on));
-        if (id) { int rc = copy_in(h, h->in_id, id, (size_t)n * sizeof(u32), src, on); if (rc) return rc; }
+        if (id) RC_TRY(copy_in(h, h->in_id, id, (size_t)n * sizeof(u32), src, on));
         else {
             k_iota<<<(unsigned)((n + 255) / 256), 256, 0, on>>>(h->in_id, (u32)n);
             KERNEL_CHECK(h);
         }
     }
     stage_end(h, RCD_STAGE_UPLOAD, on);
-    {
-        int rc = upload_issued(h, on);
-        if (rc) return rc;
-    }
+    RC_TRY(upload_issued(h, on));
     h->n = n;
     h->n_owned = n;
-    h->index_valid = false;
+    h->idx.valid = false;
     h->frame_done = false;
     return RCD_OK;
 }
@@ -623,14 +725,12 @@ int rcd_set_patterns(rcd_handle h, uint64_t n, const uint8_t *pattern, int32_t s
     CUDA_TRY(h, cudaSetDevice(h->device));
     if (n) {
         cudaStream_t on = nullptr;
-        int rc = upload_stream(h, pattern ? src : RCD_SRC_HOST, &on);
-        if (rc) return rc;
-        if (pattern) { rc = copy_in(h, h->in_pattern, pattern, (size_t)n, src, on); if (rc) return rc; }
+        RC_TRY(upload_stream(h, pattern ? src : RCD_SRC_HOST, &on));
+        if (pattern) RC_TRY(copy_in(h, h->in_pattern, pattern, (size_t)n, src, on));
         else CUDA_TRY(h, cudaMemsetAsync(h->in_pattern, RCD_PAT_ACCELERATING, (size_t)n, on));
-        rc = upload_issued(h, on);
-        if (rc) return rc;
+        RC_TRY(upload_issued(h, on));
     }
-    h->index_valid = false;  // the pattern is packed into the cell-ordered state
+    h->idx.valid = false;  // the pattern is packed into the cell-ordered state
     h->frame_done = false;
     return RCD_OK;
 }
@@ -639,7 +739,7 @@ int rcd_set_owned(rcd_handle h, uint64_t n_owned) {
     if (!h) return RCD_EINVAL;
     if (n_owned > h->n) return fail(h, RCD_EINVAL, "rcd_set_owned: n_owned exceeds the object count");
     h->n_owned = n_owned;
-    h->index_valid = false;
+    h->idx.valid = false;
     h->frame_done = false;
     return RCD_OK;
 }
@@ -655,8 +755,7 @@ static int step_impl(rcd_handle h, int32_t mode, float search_radius, float time
     if (with_detect) {
         fused = search_radius == PREDICT_RADIUS && time_window == 10.0f && !(h->flags & RCD_FLAG_COUNT_PREDICT_CANDIDATES);
         if (!fused) {  // other parameters: the two passes back to back
-            int rc2 = step_impl(h, RCD_MODE_DETECT | (append ? RCD_STEP_APPEND : 0), search_radius, time_window);
-            if (rc2) return rc2;
+            RC_TRY(step_impl(h, RCD_MODE_DETECT | (append ? RCD_STEP_APPEND : 0), search_radius, time_window));
             return step_impl(h, RCD_MODE_PREDICT | RCD_STEP_APPEND, search_radius, time_window);
         }
     }
@@ -665,36 +764,28 @@ static int step_impl(rcd_handle h, int32_t mode, float search_radius, float time
     if (mode == RCD_MODE_DETECT && !(time_window >= 0.0f)) return fail(h, RCD_EINVAL, "rcd_step: time_window must be >= 0");
     CUDA_TRY(h, cudaSetDevice(h->device));
     if (!append) h->launches = 0;
-    if (!append && h->flip_pending) {  // the previous frame is being delivered: write into the twin buffers
-        std::swap(h->out, h->out_alt);
-        std::swap(h->counters, h->counters_alt);
-        std::swap(h->risk_count, h->risk_count_alt);
-        h->flip_pending = false;
-    }
+    if (!append && h->flip_pending) h->flip();
     h->frame_done = false;
     h->stage_mode = mode;
-    for (int s = RCD_STAGE_KEYS; s <= RCD_STAGE_EXACT; ++s) h->stages[mode][s].used = false;
-    h->stages[mode][RCD_STAGE_QORDER].used = false;
+    reset_stages(h, mode);
     stage_begin(h, RCD_STAGE_TOTAL);
     const float cell_req = (mode == RCD_MODE_PREDICT) ? PREDICT_RADIUS : search_radius;
-    int rc = build_index(h, cell_req);
-    if (rc) return rc;
+    RC_TRY(build_index(h, cell_req));
 
     if (h->n && h->n_owned) {
-        rc = build_query_order(h, mode == RCD_MODE_PREDICT ? 2 : 1);
-        if (rc) return rc;
+        RC_TRY(build_query_order(h, mode == RCD_MODE_PREDICT ? 2 : 1));
     }
     stage_begin(h, RCD_STAGE_PAIRS);
-    if (!append) CUDA_TRY(h, cudaMemsetAsync(h->counters, 0, sizeof(Counters), h->stream));
+    if (!append) CUDA_TRY(h, cudaMemsetAsync(h->fb().counters, 0, sizeof(Counters), h->stream));
     if (h->n) CUDA_TRY(h, cudaMemsetAsync(h->cand_count, 0, (size_t)h->n * sizeof(u32), h->stream));
-    if (h->n && !append) CUDA_TRY(h, cudaMemsetAsync(h->risk_count, 0, (size_t)h->n * sizeof(u32), h->stream));
+    if (h->n && !append) CUDA_TRY(h, cudaMemsetAsync(h->fb().risk_count, 0, (size_t)h->n * sizeof(u32), h->stream));
     if (h->n && h->n_owned) {
         PairParams P;
         P.n = (u32)h->n;
         P.n_owned = (u32)h->n_owned;
-        P.g = h->grid;
+        P.g = h->idx.grid;
         P.P0 = h->P0; P.P1 = h->P1; P.P2 = h->P2;
-        P.qorder = h->qvals[h->q_sorted_buf];
+        P.qorder = h->qvals[h->idx.q_sorted_buf];
         P.sorted_slot = h->sorted_slot;
         P.sorted_id = h->sorted_id;
         P.cell_begin = h->cell_begin;
@@ -713,11 +804,11 @@ static int step_impl(rcd_handle h, int32_t mode, float search_radius, float time
             P.use_t1 = mode == RCD_MODE_PREDICT ? 1 : 0;
         }
         P.D *= 1.0f + 1.0e-6f;
-        P.out = h->out;
+        P.out = h->fb().out;
         P.out_cap = h->max_pairs;
-        P.counters = h->counters;
+        P.counters = h->fb().counters;
         P.cand_count = h->cand_count;
-        P.risk_count = h->risk_count;
+        P.risk_count = h->fb().risk_count;
         P.ntiles = (u32)((h->n_owned + TQ - 1) / TQ);
         P.tile_counter = h->pair_tile_counter;
         P.qa = h->qa; P.qa_fill = h->qa_fill; P.qa_blocks_cap = h->qa_blocks_cap;
@@ -729,91 +820,47 @@ static int step_impl(rcd_handle h, int32_t mode, float search_radius, float time
         P.q3 = h->q3; P.qcap = h->qcap;
         P.q3_split = mode == RCD_MODE_PREDICT ? h->qcap / 4 : h->qcap;
         CUDA_TRY(h, cudaMemsetAsync(h->pair_tile_counter, 0, 2 * sizeof(u32), h->stream));
-        CUDA_TRY(h, cudaMemsetAsync(&h->counters->n_qa_blocks, 0, 6 * sizeof(unsigned long long), h->stream));
+        CUDA_TRY(h, cudaMemsetAsync(&h->fb().counters->n_qa_blocks, 0, 6 * sizeof(unsigned long long), h->stream));
         const bool count = (h->flags & RCD_FLAG_COUNT_PREDICT_CANDIDATES) != 0;
         // persistent launch: as many blocks as can be resident, warps pull tiles from a counter
         const int variant = fused ? 4 : mode == RCD_MODE_DETECT ? 0 : (mode == RCD_MODE_COMPUTE_NODE ? 3 : (count ? 2 : 1));
+        const FrameKernels &K = FRAME_KERNELS[variant];
         if (h->pair_blocks[variant] == 0) {
-            int per_sm = 0, sms = 0;
-            const void *fn = variant == 0 ? (const void *)k_pairs<RCD_MODE_DETECT, false, false>
-                           : variant == 1 ? (const void *)k_pairs<RCD_MODE_PREDICT, false, false>
-                           : variant == 2 ? (const void *)k_pairs<RCD_MODE_PREDICT, true, false>
-                           : variant == 4 ? (const void *)k_pairs<MODE_PREDICT_WITH_DETECT, false, false>
-                                          : (const void *)k_pairs<RCD_MODE_COMPUTE_NODE, false, false>;
-            const void *fn2 = variant == 0 ? (const void *)k_narrow<RCD_MODE_DETECT, false>
-                            : variant == 1 ? (const void *)k_narrow<RCD_MODE_PREDICT, false>
-                            : variant == 2 ? (const void *)k_narrow<RCD_MODE_PREDICT, true>
-                            : variant == 4 ? (const void *)k_narrow<MODE_PREDICT_WITH_DETECT, false>
-                                           : (const void *)k_narrow<RCD_MODE_COMPUTE_NODE, false>;
-            CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
-            h->stage_blocks_sms = std::max(1, sms);
-            CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, PAIR_THREADS, 0));
-            h->pair_blocks[variant] = std::max(1, per_sm) * std::max(1, sms);
-            CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn2, STAGE_THREADS, 0));
-            h->narrow_blocks[variant] = std::max(1, per_sm) * std::max(1, sms);
+            int per_sm = 0;
+            CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, K.pairs, PAIR_THREADS, 0));
+            h->pair_blocks[variant] = std::max(1, per_sm) * h->sms;
+            CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, K.narrow, STAGE_THREADS, 0));
+            h->narrow_blocks[variant] = std::max(1, per_sm) * h->sms;
         }
         // plan: the tiles' cell boxes and work items of even size; then the persistent pair kernel
-        {
-            const unsigned pb = (unsigned)std::min<u64>((P.ntiles + 3) / 4, (u64)h->stage_blocks_sms * 8);
-            if (variant == 0) k_tile_plan<RCD_MODE_DETECT><<<pb, 128, 0, h->stream>>>(P);
-            else if (variant == 3) k_tile_plan<RCD_MODE_COMPUTE_NODE><<<pb, 128, 0, h->stream>>>(P);
-            else k_tile_plan<RCD_MODE_PREDICT><<<pb, 128, 0, h->stream>>>(P);
-            KERNEL_CHECK(h);
-        }
+        const unsigned pb = (unsigned)std::min<u64>((P.ntiles + 3) / 4, (u64)h->sms * 8);
+        K.tile_plan<<<pb, 128, 0, h->stream>>>(P);
+        KERNEL_CHECK(h);
         const u64 items = (u64)P.ntiles * PLAN_ITEMS_PER_TILE;  // (upper estimate: the grid is capped by residency)
         const unsigned blocks = (unsigned)std::min<u64>((items + PAIR_WARPS - 1) / PAIR_WARPS, (u64)h->pair_blocks[variant]);
         // the regular pass, then the overflow pass (returns at once unless the pair queue ran out)
-        const unsigned oblocks = std::min(blocks, (unsigned)h->stage_blocks_sms * 4u);
-        if (variant == 0) {
-            k_pairs<RCD_MODE_DETECT, false, false><<<blocks, PAIR_THREADS, 0, h->stream>>>(P);
-            k_pairs<RCD_MODE_DETECT, false, true><<<oblocks, PAIR_THREADS, 0, h->stream>>>(P);
-        } else if (variant == 1) {
-            k_pairs<RCD_MODE_PREDICT, false, false><<<blocks, PAIR_THREADS, 0, h->stream>>>(P);
-            k_pairs<RCD_MODE_PREDICT, false, true><<<oblocks, PAIR_THREADS, 0, h->stream>>>(P);
-        } else if (variant == 2) {
-            k_pairs<RCD_MODE_PREDICT, true, false><<<blocks, PAIR_THREADS, 0, h->stream>>>(P);
-            k_pairs<RCD_MODE_PREDICT, true, true><<<oblocks, PAIR_THREADS, 0, h->stream>>>(P);
-        } else if (variant == 4) {
-            k_pairs<MODE_PREDICT_WITH_DETECT, false, false><<<blocks, PAIR_THREADS, 0, h->stream>>>(P);
-            k_pairs<MODE_PREDICT_WITH_DETECT, false, true><<<oblocks, PAIR_THREADS, 0, h->stream>>>(P);
-        } else {
-            k_pairs<RCD_MODE_COMPUTE_NODE, false, false><<<blocks, PAIR_THREADS, 0, h->stream>>>(P);
-            k_pairs<RCD_MODE_COMPUTE_NODE, false, true><<<oblocks, PAIR_THREADS, 0, h->stream>>>(P);
-        }
+        const unsigned oblocks = std::min(blocks, (unsigned)h->sms * 4u);
+        K.pairs<<<blocks, PAIR_THREADS, 0, h->stream>>>(P);
+        K.pairs_overflow<<<oblocks, PAIR_THREADS, 0, h->stream>>>(P);
         ++h->launches;
         KERNEL_CHECK(h);
         stage_end(h, RCD_STAGE_PAIRS);
         // the later stages read their queue lengths on the device: fixed grids, no host round trip
-        if (h->stage_blocks == 0) {
-            int sms = 0;
-            CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
-            h->stage_blocks = std::max(1, sms) * 8;
-        }
         stage_begin(h, RCD_STAGE_NARROW);
-        {
-            const unsigned nb = (unsigned)std::min<u64>((u64)h->narrow_blocks[variant], (u64)P.ntiles * 8 / STAGE_WARPS + 1);
-            if (variant == 0) k_narrow<RCD_MODE_DETECT, false><<<nb, STAGE_THREADS, 0, h->stream>>>(P);
-            else if (variant == 1) k_narrow<RCD_MODE_PREDICT, false><<<nb, STAGE_THREADS, 0, h->stream>>>(P);
-            else if (variant == 2) k_narrow<RCD_MODE_PREDICT, true><<<nb, STAGE_THREADS, 0, h->stream>>>(P);
-            else if (variant == 4) k_narrow<MODE_PREDICT_WITH_DETECT, false><<<nb, STAGE_THREADS, 0, h->stream>>>(P);
-            else k_narrow<RCD_MODE_COMPUTE_NODE, false><<<nb, STAGE_THREADS, 0, h->stream>>>(P);
-            KERNEL_CHECK(h);
-        }
+        const unsigned nb = (unsigned)std::min<u64>((u64)h->narrow_blocks[variant], (u64)P.ntiles * 8 / STAGE_WARPS + 1);
+        K.narrow<<<nb, STAGE_THREADS, 0, h->stream>>>(P);
+        KERNEL_CHECK(h);
         stage_end(h, RCD_STAGE_NARROW);
-        const unsigned sb = (unsigned)std::min<u64>((u64)h->stage_blocks, (h->n + STAGE_THREADS - 1) / STAGE_THREADS + 1);
+        const unsigned sb = (unsigned)std::min<u64>((u64)h->sms * 8, (h->n + STAGE_THREADS - 1) / STAGE_THREADS + 1);
         stage_begin(h, RCD_STAGE_EXACT);
-        if (variant == 0) k_exact<RCD_MODE_DETECT, 0><<<sb, STAGE_THREADS, 0, h->stream>>>(P);
-        else if (variant == 3) k_exact<RCD_MODE_COMPUTE_NODE, 0><<<sb, STAGE_THREADS, 0, h->stream>>>(P);
-        else if (variant == 4) k_exact<MODE_PREDICT_WITH_DETECT, 1><<<sb, STAGE_THREADS, 0, h->stream>>>(P);
-        else k_exact<RCD_MODE_PREDICT, 1><<<sb, STAGE_THREADS, 0, h->stream>>>(P);
+        K.exact<<<sb, STAGE_THREADS, 0, h->stream>>>(P);
         KERNEL_CHECK(h);
         // every record with predicted = 0 has been emitted by now (overflow passes, in-place fall-backs, detect entries):
         // the alert fold's detect pass stops here instead of walking the whole buffer
-        CUDA_TRY(h, cudaMemcpyAsync(&h->counters->n_detect_end, &h->counters->n_pairs, sizeof(unsigned long long),
+        CUDA_TRY(h, cudaMemcpyAsync(&h->fb().counters->n_detect_end, &h->fb().counters->n_pairs, sizeof(unsigned long long),
                                     cudaMemcpyDeviceToDevice, h->stream));
-        if (variant == 4) k_exact<MODE_PREDICT_WITH_DETECT, 2><<<sb, STAGE_THREADS, 0, h->stream>>>(P);
-        else if (variant == 1 || variant == 2) k_exact<RCD_MODE_PREDICT, 2><<<sb, STAGE_THREADS, 0, h->stream>>>(P);
-        KERNEL_CHECK(h);
+        if (K.exact_resolved) K.exact_resolved<<<sb, STAGE_THREADS, 0, h->stream>>>(P);
+        KERNEL_CHECK(h);  // (counted with or without the RESOLVED pass)
         stage_end(h, RCD_STAGE_EXACT);
     } else {
         stage_end(h, RCD_STAGE_PAIRS);
@@ -824,10 +871,27 @@ static int step_impl(rcd_handle h, int32_t mode, float search_radius, float time
     return RCD_OK;
 }
 
-// RCD_FLAG_GRAPH: the launch sequence of a step is a pure function of the key below (every other kernel
-// argument is a buffer that lives as long as the handle).  First sighting of a key: run normally and
-// remember it; second sighting in a row: capture, instantiate, launch; from then on: one graph launch plus the
-// host-side state changes step_impl would have made.
+// The graph key of a step: the index fields count only while the index is valid (q_sorted_buf only with a query
+// order), and `out` is the pair buffer the step will write, after a pending flip.
+static StepKey step_key(rcd_handle h, int32_t mode, float search_radius, float time_window, bool append, bool flip) {
+    const IndexState &ix = h->idx;
+    StepKey key;
+    key.mode = mode; key.R = search_radius; key.T = time_window;
+    key.pt = h->cn_prediction_time; key.thr = h->cn_risk_threshold;
+    key.n = h->n; key.n_owned = h->n_owned;
+    key.index_valid = ix.valid ? 1 : 0;
+    key.index_cell_req = ix.valid ? ix.cell_req : 0.0f;
+    key.sorted_buf = ix.valid ? ix.sorted_buf : 0;
+    key.qorder_kind = ix.valid ? ix.qorder_kind : 0;
+    key.q_sorted_buf = (ix.valid && ix.qorder_kind) ? ix.q_sorted_buf : 0;
+    key.frame_done = append ? (h->frame_done ? 1 : 0) : 0;
+    key.out = h->bufs[flip ? h->cur ^ 1 : h->cur].out.get();
+    return key;
+}
+
+// RCD_FLAG_GRAPH: the launch sequence of a step is a pure function of its StepKey.  First sighting of a key: run
+// normally and remember it; second sighting in a row: capture, instantiate, launch; from then on: one graph
+// launch plus the host-side state changes step_impl would have made.
 int rcd_step(rcd_handle h, int32_t mode, float search_radius, float time_window) {
     if (!h) return RCD_EINVAL;
     const bool want = (h->flags & RCD_FLAG_GRAPH) && !(h->flags & RCD_FLAG_PROFILE) && h->world_static && !h->graph_broken &&
@@ -837,43 +901,19 @@ int rcd_step(rcd_handle h, int32_t mode, float search_radius, float time_window)
     const bool flip = !append && h->flip_pending;
     {   // (events of other streams stay outside the graph: order the stream before the launch / the capture)
         CUDA_TRY(h, cudaSetDevice(h->device));
-        int rcw = wait_upload(h);
-        if (rcw) return rcw;
+        RC_TRY(wait_upload(h));
     }
-    rcd_handle_s::StepKey key;
-    key.mode = mode; key.R = search_radius; key.T = time_window;
-    key.pt = h->cn_prediction_time; key.thr = h->cn_risk_threshold;
-    key.n = h->n; key.n_owned = h->n_owned;
-    key.index_valid = h->index_valid ? 1 : 0;
-    key.index_cell_req = h->index_valid ? h->index_cell_req : 0.0f;
-    key.sorted_buf = h->index_valid ? h->sorted_buf : 0;
-    key.qorder_kind = h->index_valid ? h->qorder_kind : 0;
-    key.q_sorted_buf = (h->index_valid && h->qorder_kind) ? h->q_sorted_buf : 0;
-    key.frame_done = append ? (h->frame_done ? 1 : 0) : 0;
-    key.out = flip ? (const void *)h->out_alt : (const void *)h->out;
+    const StepKey key = step_key(h, mode, search_radius, time_window, append, flip);
     for (auto &g : h->graphs) {
         if (!g.exec || !(g.key == key)) continue;
         // ---- replay ----
         CUDA_TRY(h, cudaSetDevice(h->device));
-        if (flip) {
-            std::swap(h->out, h->out_alt);
-            std::swap(h->counters, h->counters_alt);
-            std::swap(h->risk_count, h->risk_count_alt);
-            h->flip_pending = false;
-        }
+        if (flip) h->flip();
         h->frame_done = false;
         CUDA_TRY(h, cudaGraphLaunch(g.exec, h->stream));
-        {
-            int rcr = release_inputs(h);  // (at the end of the step: a graph has no events inside)
-            if (rcr) return rcr;
-        }
+        RC_TRY(release_inputs(h));  // (at the end of the step: a graph has no events inside)
         h->launches = (append ? h->launches : 0) + g.launches;
-        h->grid = g.grid;
-        h->index_valid = true;
-        h->index_cell_req = g.index_cell_req;
-        h->sorted_buf = g.sorted_buf;
-        h->qorder_kind = g.qorder_kind;
-        h->q_sorted_buf = g.q_sorted_buf;
+        h->idx = g.idx;
         h->stage_mode = g.last_mode;
         h->last_mode = g.last_mode;
         h->frame_done = true;
@@ -890,20 +930,18 @@ int rcd_step(rcd_handle h, int32_t mode, float search_radius, float time_window)
     // ---- second sighting: capture ----
     CUDA_TRY(h, cudaSetDevice(h->device));
     struct Saved {
-        rcd_pair *out, *out_alt; Counters *counters, *counters_alt; u32 *risk_count, *risk_count_alt; bool flip_pending, frame_done, index_valid;
-        float index_cell_req; int sorted_buf, last_mode, stage_mode; GridParams grid; u64 launches; int qorder_kind, q_sorted_buf;
-    } pre = {h->out, h->out_alt, h->counters, h->counters_alt, h->risk_count, h->risk_count_alt, h->flip_pending, h->frame_done, h->index_valid,
-             h->index_cell_req, h->sorted_buf, h->last_mode, h->stage_mode, h->grid, h->launches, h->qorder_kind, h->q_sorted_buf};
+        IndexState idx;
+        int cur, last_mode, stage_mode;
+        bool flip_pending, frame_done;
+        u64 launches;
+    };
+    const Saved pre = {h->idx, h->cur, h->last_mode, h->stage_mode, h->flip_pending, h->frame_done, h->launches};
     auto restore = [&]() {
-        h->out = pre.out; h->out_alt = pre.out_alt; h->counters = pre.counters; h->counters_alt = pre.counters_alt;
-        h->risk_count = pre.risk_count; h->risk_count_alt = pre.risk_count_alt;
-        h->flip_pending = pre.flip_pending; h->frame_done = pre.frame_done; h->index_valid = pre.index_valid;
-        h->index_cell_req = pre.index_cell_req; h->sorted_buf = pre.sorted_buf; h->last_mode = pre.last_mode;
-        h->stage_mode = pre.stage_mode; h->grid = pre.grid; h->launches = pre.launches;
-        h->qorder_kind = pre.qorder_kind; h->q_sorted_buf = pre.q_sorted_buf;
+        h->idx = pre.idx; h->cur = pre.cur; h->last_mode = pre.last_mode; h->stage_mode = pre.stage_mode;
+        h->flip_pending = pre.flip_pending; h->frame_done = pre.frame_done; h->launches = pre.launches;
     };
     cudaGraph_t graph = nullptr;
-    cudaGraphExec_t exec = nullptr;
+    GraphExec exec;
     cudaError_t e = cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal);
     int rc = RCD_OK;
     if (e == cudaSuccess) {
@@ -913,36 +951,28 @@ int rcd_step(rcd_handle h, int32_t mode, float search_radius, float time_window)
         cudaError_t e2 = cudaStreamEndCapture(h->stream, &graph);
         if (e2 != cudaSuccess) e = e2;
     }
-    if (e == cudaSuccess && rc == RCD_OK && graph) e = cudaGraphInstantiate(&exec, graph, 0);
+    if (e == cudaSuccess && rc == RCD_OK && graph) e = exec.instantiate(graph);
     if (graph) cudaGraphDestroy(graph);
     if (e != cudaSuccess || rc != RCD_OK || !exec) {  // not capturable here: never try again, run the step for real
         (void)cudaGetLastError();
-        if (exec) cudaGraphExecDestroy(exec);
+        exec.reset();
         restore();
         h->graph_broken = true;
         return step_impl(h, mode, search_radius, time_window);
     }
     e = cudaGraphLaunch(exec, h->stream);
     if (e != cudaSuccess) {
-        cudaGraphExecDestroy(exec);
+        exec.reset();
         restore();
         h->graph_broken = true;
         return step_impl(h, mode, search_radius, time_window);
     }
-    {
-        int rcr = release_inputs(h);
-        if (rcr) return rcr;
-    }
-    rcd_handle_s::StepGraph &slot = h->graphs[h->graph_next];
+    RC_TRY(release_inputs(h));
+    StepGraph &slot = h->graphs[h->graph_next];
     h->graph_next = (h->graph_next + 1) % 4;
-    if (slot.exec) cudaGraphExecDestroy(slot.exec);
-    slot.exec = exec;
+    slot.exec = std::move(exec);  // (releases the graph the slot held)
     slot.key = key;
-    slot.grid = h->grid;
-    slot.index_cell_req = h->index_cell_req;
-    slot.sorted_buf = h->sorted_buf;
-    slot.qorder_kind = h->qorder_kind;
-    slot.q_sorted_buf = h->q_sorted_buf;
+    slot.idx = h->idx;
     slot.last_mode = h->last_mode;
     slot.launches = h->launches - (append ? pre.launches : 0);
     return RCD_OK;
@@ -969,14 +999,14 @@ int rcd_truncate(rcd_handle h, uint64_t n) {
     if (n > h->n) return fail(h, RCD_EINVAL, "rcd_truncate: n exceeds the object count");
     h->n = n;
     h->n_owned = n;
-    h->index_valid = false;
+    h->idx.valid = false;
     h->frame_done = false;
     return RCD_OK;
 }
 
 int rcd_invalidate(rcd_handle h) {
     if (!h) return RCD_EINVAL;
-    h->index_valid = false;
+    h->idx.valid = false;
     h->frame_done = false;
     return RCD_OK;
 }
@@ -987,7 +1017,7 @@ int rcd_build_index(rcd_handle h, float cell_radius) {
     CUDA_TRY(h, cudaSetDevice(h->device));
     h->launches = 0;
     h->stage_mode = RCD_MODE_DETECT;
-    for (int s = RCD_STAGE_KEYS; s <= RCD_STAGE_EXACT; ++s) h->stages[RCD_MODE_DETECT][s].used = false;
+    reset_stages(h, RCD_MODE_DETECT);
     stage_begin(h, RCD_STAGE_TOTAL);
     int rc = build_index(h, cell_radius);
     stage_end(h, RCD_STAGE_TOTAL);
@@ -998,34 +1028,21 @@ int rcd_counts(rcd_handle h, rcd_counts_t *out) {
     if (!h || !out) return RCD_EINVAL;
     if (!h->frame_done) return fail(h, RCD_ESTATE, "rcd_counts: no frame has been stepped");
     CUDA_TRY(h, cudaSetDevice(h->device));
-    CUDA_TRY(h, cudaMemcpyAsync(h->counters_host, h->counters, sizeof(Counters), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(h->counters_host, h->fb().counters, sizeof(Counters), cudaMemcpyDeviceToHost, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    const Counters &c = *h->counters_host;
-    h->last_n_pairs = c.n_pairs;
-    h->last_n_detect_end = c.n_detect_end;
-    out->n_objects = h->n;
-    out->n_owned = h->n_owned;
-    out->n_candidates = c.n_candidates;
-    out->n_potential = c.n_potential;
-    out->n_pairs = c.n_pairs;
-    out->n_high_risk = c.n_high_risk;
-    out->n_written = std::min<u64>(c.n_pairs, h->max_pairs);
-    for (int k = 0; k < 4; ++k) out->n_alerts[k] = c.n_alerts[k];
-    out->n_exact = c.n_exact;
-    out->n_fallback = c.n_fallback;
+    fill_counts(h, *h->counters_host, h->n, h->n_owned, out);
     return RCD_OK;
 }
 
 static int download_impl(rcd_handle h, rcd_pair *out, uint64_t cap, uint64_t *n_out, bool sorted) {
     if (!h || !n_out || (cap && !out)) return RCD_EINVAL;
     rcd_counts_t c;
-    int rc = rcd_counts(h, &c);
-    if (rc) return rc;
+    RC_TRY(rcd_counts(h, &c));
     h->stage_mode = 0;
     stage_begin(h, RCD_STAGE_DOWNLOAD);
     u64 m = std::min<u64>(c.n_written, cap);
     if (m) {
-        CUDA_TRY(h, cudaMemcpyAsync(out, h->out, (size_t)m * sizeof(rcd_pair), cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(h, cudaMemcpyAsync(out, h->fb().out, (size_t)m * sizeof(rcd_pair), cudaMemcpyDeviceToHost, h->stream));
         CUDA_TRY(h, cudaStreamSynchronize(h->stream));
         if (sorted) {
             // sort 16-byte (key, index) records instead of the 48-byte pairs, then permute once
@@ -1052,48 +1069,36 @@ int rcd_download_unsorted(rcd_handle h, rcd_pair *out, uint64_t cap, uint64_t *n
     return download_impl(h, out, cap, n_out, false);
 }
 
-// twin buffers + copy stream of the pipelined deliveries (allocated at the first use)
+// twin buffers + copy stream of the pipelined deliveries (made at the first use, all or nothing)
 static int delivery_ready(rcd_handle h) {
-    if (!h->out_alt) {
-        CUDA_TRY(h, dev_alloc(&h->out_alt, (size_t)h->max_pairs));
-        CUDA_TRY(h, dev_alloc(&h->counters_alt, 1));
-        CUDA_TRY(h, dev_alloc(&h->risk_count_alt, (size_t)h->cap));
-        CUDA_TRY(h, cudaMallocHost(reinterpret_cast<void **>(&h->pend_counters_host), sizeof(Counters)));
-        CUDA_TRY(h, cudaMallocHost(reinterpret_cast<void **>(&h->pend_alert_counters_host), sizeof(AlertCounters)));
-        CUDA_TRY(h, cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-        CUDA_TRY(h, cudaEventCreateWithFlags(&h->pend_event, cudaEventDisableTiming));
-        {
-            int least = 0, greatest = 0;
-            CUDA_TRY(h, cudaDeviceGetStreamPriorityRange(&least, &greatest));
-            CUDA_TRY(h, cudaStreamCreateWithPriority(&h->alert_stream, cudaStreamNonBlocking, least));
-        }
-        CUDA_TRY(h, cudaEventCreateWithFlags(&h->ev_frame_done, cudaEventDisableTiming));
-        CUDA_TRY(h, cudaEventCreateWithFlags(&h->ev_alert_done, cudaEventDisableTiming));
+    if (h->dl.pend_event) return RCD_OK;
+    FrameBuffers twin;
+    Delivery d;
+    CUDA_TRY(h, twin.out.alloc(h->max_pairs));
+    CUDA_TRY(h, twin.counters.alloc());
+    CUDA_TRY(h, twin.risk_count.alloc(h->cap));
+    CUDA_TRY(h, d.counters_host.alloc());
+    CUDA_TRY(h, d.alert_counters_host.alloc());
+    CUDA_TRY(h, d.copy_stream.create());
+    CUDA_TRY(h, d.pend_event.create());
+    {
+        int least = 0, greatest = 0;
+        CUDA_TRY(h, cudaDeviceGetStreamPriorityRange(&least, &greatest));
+        CUDA_TRY(h, d.alert_stream.create(least));
     }
+    CUDA_TRY(h, d.ev_frame_done.create());
+    CUDA_TRY(h, d.ev_alert_done.create());
+    h->bufs[h->cur ^ 1] = std::move(twin);
+    h->dl = std::move(d);
     return RCD_OK;
 }
 // Order the handle's stream after the alert-table work a summary delivery left on alert_stream.
 static int alerts_join(rcd_handle h) {
     if (h->alert_async) {
-        CUDA_TRY(h, cudaStreamWaitEvent(h->stream, h->ev_alert_done, 0));
+        CUDA_TRY(h, cudaStreamWaitEvent(h->stream, h->dl.ev_alert_done, 0));
         h->alert_async = false;
     }
     return RCD_OK;
-}
-static void counts_out(rcd_handle h, const Counters &c, rcd_counts_t *counts) {
-    h->last_n_pairs = c.n_pairs;
-    h->last_n_detect_end = c.n_detect_end;
-    if (!counts) return;
-    counts->n_objects = h->pend_n;
-    counts->n_owned = h->pend_n_owned;
-    counts->n_candidates = c.n_candidates;
-    counts->n_potential = c.n_potential;
-    counts->n_pairs = c.n_pairs;
-    counts->n_high_risk = c.n_high_risk;
-    counts->n_written = std::min<u64>(c.n_pairs, h->max_pairs);
-    for (int k = 0; k < 4; ++k) counts->n_alerts[k] = c.n_alerts[k];
-    counts->n_exact = c.n_exact;
-    counts->n_fallback = c.n_fallback;
 }
 static int delivery_begin(rcd_handle h, const char *who) {
     if (!h->frame_done) return fail(h, RCD_ESTATE, std::string(who) + ": no frame has been stepped");
@@ -1103,10 +1108,10 @@ static int delivery_begin(rcd_handle h, const char *who) {
 }
 static int delivery_issued(rcd_handle h, cudaStream_t on = nullptr) {  // the frame's totals ride along; later work goes to the twin buffers
     if (!on) on = h->stream;
-    CUDA_TRY(h, cudaMemcpyAsync(h->pend_counters_host, h->counters, sizeof(Counters), cudaMemcpyDeviceToHost, on));
-    CUDA_TRY(h, cudaEventRecord(h->pend_event, on));
-    h->pend_dev = h->out;
-    h->pend_risk = h->risk_count;
+    CUDA_TRY(h, cudaMemcpyAsync(h->dl.counters_host, h->fb().counters, sizeof(Counters), cudaMemcpyDeviceToHost, on));
+    CUDA_TRY(h, cudaEventRecord(h->dl.pend_event, on));
+    h->pend_dev = h->fb().out;
+    h->pend_risk = h->fb().risk_count;
     h->pend_n = h->n;
     h->pend_n_owned = h->n_owned;
     h->download_pending = true;
@@ -1116,8 +1121,7 @@ static int delivery_issued(rcd_handle h, cudaStream_t on = nullptr) {  // the fr
 
 int rcd_download_begin(rcd_handle h, rcd_pair *out, uint64_t cap) {
     if (!h || (cap && !out)) return RCD_EINVAL;
-    int rc = delivery_begin(h, "rcd_download_begin");
-    if (rc) return rc;
+    RC_TRY(delivery_begin(h, "rcd_download_begin"));
     h->pend_kind = 0;
     h->pend_out = out;
     h->pend_cap = cap;
@@ -1126,12 +1130,11 @@ int rcd_download_begin(rcd_handle h, rcd_pair *out, uint64_t cap) {
 
 int rcd_download_begin_compact(rcd_handle h, rcd_pair_compact *out, uint64_t cap) {
     if (!h || (cap && !out)) return RCD_EINVAL;
-    int rc = delivery_begin(h, "rcd_download_begin_compact");
-    if (rc) return rc;
-    if (!h->compact_dev) CUDA_TRY(h, dev_alloc(&h->compact_dev, (size_t)h->max_pairs));
+    RC_TRY(delivery_begin(h, "rcd_download_begin_compact"));
+    if (!h->compact_dev) CUDA_TRY(h, h->compact_dev.alloc(h->max_pairs));
     // (one scratch buffer: the narrowing of frame k + 1 runs on the handle's stream after frame k's copy was issued
     // and waited for by rcd_download_finish -- one delivery in flight at a time)
-    k_compact_pairs<<<(unsigned)h->stage_blocks_sms * 8, 256, 0, h->stream>>>(h->out, h->max_pairs, &h->counters->n_pairs, h->compact_dev);
+    k_compact_pairs<<<(unsigned)h->sms * 8, 256, 0, h->stream>>>(h->fb().out, h->max_pairs, &h->fb().counters->n_pairs, h->compact_dev);
     KERNEL_CHECK(h);
     h->pend_kind = 1;
     h->pend_out_compact = out;
@@ -1143,18 +1146,18 @@ int rcd_download_finish(rcd_handle h, rcd_counts_t *counts, uint64_t *n_out) {
     if (!h || !n_out) return RCD_EINVAL;
     if (!h->download_pending || h->pend_kind == 2) return fail(h, RCD_ESTATE, "rcd_download_finish: no download in flight");
     CUDA_TRY(h, cudaSetDevice(h->device));
-    CUDA_TRY(h, cudaEventSynchronize(h->pend_event));  // the frame is complete; later work keeps running
-    const Counters &c = *h->pend_counters_host;
+    CUDA_TRY(h, cudaEventSynchronize(h->dl.pend_event));  // the frame is complete; later work keeps running
+    const Counters &c = *h->dl.counters_host;
     const u64 m = std::min<u64>(std::min<u64>(c.n_pairs, h->max_pairs), h->pend_cap);
     if (m) {
         if (h->pend_kind == 0)
-            CUDA_TRY(h, cudaMemcpyAsync(h->pend_out, h->pend_dev, (size_t)m * sizeof(rcd_pair), cudaMemcpyDeviceToHost, h->copy_stream));
+            CUDA_TRY(h, cudaMemcpyAsync(h->pend_out, h->pend_dev, (size_t)m * sizeof(rcd_pair), cudaMemcpyDeviceToHost, h->dl.copy_stream));
         else
             CUDA_TRY(h, cudaMemcpyAsync(h->pend_out_compact, h->compact_dev, (size_t)m * sizeof(rcd_pair_compact),
-                                        cudaMemcpyDeviceToHost, h->copy_stream));
-        CUDA_TRY(h, cudaStreamSynchronize(h->copy_stream));
+                                        cudaMemcpyDeviceToHost, h->dl.copy_stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->dl.copy_stream));
     }
-    counts_out(h, c, counts);
+    fill_counts(h, c, h->pend_n, h->pend_n_owned, counts);
     *n_out = m;
     h->download_pending = false;
     return RCD_OK;
@@ -1165,7 +1168,7 @@ int rcd_download_risk_counts(rcd_handle h, uint32_t *out, uint64_t n) {
     if (!h->frame_done) return fail(h, RCD_ESTATE, "rcd_download_risk_counts: no frame has been stepped");
     if (n > h->n) return fail(h, RCD_EINVAL, "rcd_download_risk_counts: n exceeds the object count");
     CUDA_TRY(h, cudaSetDevice(h->device));
-    if (n) CUDA_TRY(h, cudaMemcpyAsync(out, h->risk_count, (size_t)n * sizeof(u32), cudaMemcpyDeviceToHost, h->stream));
+    if (n) CUDA_TRY(h, cudaMemcpyAsync(out, h->fb().risk_count, (size_t)n * sizeof(u32), cudaMemcpyDeviceToHost, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     return RCD_OK;
 }
@@ -1187,47 +1190,33 @@ int rcd_query_radius(rcd_handle h, uint64_t nq, const float *qx, const float *qy
     for (u64 q = 0; q <= nq; ++q) offsets[q] = 0;
     if (nq == 0 || h->n == 0) return RCD_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    {
-        int rcw = wait_upload(h);
-        if (rcw) return rcw;
-    }
+    RC_TRY(wait_upload(h));
     // reuse the index of the last frame if there is one, else build one with the default cell
-    int rc = build_index(h, h->index_valid ? h->index_cell_req : std::max(radius, 1.0f));
-    if (rc) return rc;
-    float *dq = nullptr;
-    uint2 *dhits = nullptr;
-    CUDA_TRY(h, dev_alloc(&dq, 3 * (size_t)nq));
-    cudaError_t e = dev_alloc(&dhits, (size_t)std::max<u64>(cap, 1));
-    if (e != cudaSuccess) { cudaFree(dq); return fail(h, RCD_ENOMEM, "rcd_query_radius: device allocation failed"); }
-    auto cleanup = [&]() { cudaFree(dq); cudaFree(dhits); };
+    RC_TRY(build_index(h, h->idx.valid ? h->idx.cell_req : std::max(radius, 1.0f)));
+    DevBuf<float> dq;
+    DevBuf<uint2> dhits;
+    CUDA_TRY(h, dq.alloc(3 * (size_t)nq));
+    CUDA_TRY(h, dhits.alloc(std::max<u64>(cap, 1)));
     cudaMemcpyAsync(dq, qx, nq * sizeof(float), cudaMemcpyHostToDevice, h->stream);
-    cudaMemcpyAsync(dq + nq, qy, nq * sizeof(float), cudaMemcpyHostToDevice, h->stream);
-    cudaMemcpyAsync(dq + 2 * nq, qz, nq * sizeof(float), cudaMemcpyHostToDevice, h->stream);
-    cudaMemsetAsync(&h->counters->n_query_hits, 0, sizeof(unsigned long long), h->stream);
+    cudaMemcpyAsync(dq.get() + nq, qy, nq * sizeof(float), cudaMemcpyHostToDevice, h->stream);
+    cudaMemcpyAsync(dq.get() + 2 * nq, qz, nq * sizeof(float), cudaMemcpyHostToDevice, h->stream);
+    cudaMemsetAsync(&h->fb().counters->n_query_hits, 0, sizeof(unsigned long long), h->stream);
     const unsigned blocks = (unsigned)((nq * 32 + 127) / 128);
-    k_query_radius<<<blocks, 128, 0, h->stream>>>((u32)nq, dq, dq + nq, dq + 2 * nq, radius, h->grid, (u32)h->n, h->P0,
-                                                   h->cell_begin, h->sorted_slot, dhits, cap, h->counters);
-    e = cudaGetLastError();
+    k_query_radius<<<blocks, 128, 0, h->stream>>>((u32)nq, dq, dq.get() + nq, dq.get() + 2 * nq, radius, h->idx.grid, (u32)h->n,
+                                                   h->P0, h->cell_begin, h->sorted_slot, dhits, cap, h->fb().counters);
+    CUDA_TRY(h, cudaGetLastError());  // (the copies above report their errors here)
     unsigned long long total = 0;
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(&total, &h->counters->n_query_hits, sizeof(total), cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    if (e != cudaSuccess) { cleanup(); return fail(h, RCD_ECUDA, std::string("rcd_query_radius: ") + cudaGetErrorString(e)); }
+    CUDA_TRY(h, cudaMemcpyAsync(&total, &h->fb().counters->n_query_hits, sizeof(total), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     ++h->launches;
     if (total > cap) {
         offsets[nq] = total;  // tells the caller how much room a retry needs
-        cleanup();
         return fail(h, RCD_ECAPACITY, "rcd_query_radius: result buffer too small");
     }
     std::vector<uint2> hits((size_t)total);
-    std::vector<u32> idmap;
-    if (total) e = cudaMemcpy(hits.data(), dhits, (size_t)total * sizeof(uint2), cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) {
-        idmap.resize((size_t)h->n);
-        e = cudaMemcpy(idmap.data(), h->in_id, (size_t)h->n * sizeof(u32), cudaMemcpyDeviceToHost);
-    }
-    cleanup();
-    if (e != cudaSuccess) return fail(h, RCD_ECUDA, std::string("rcd_query_radius: ") + cudaGetErrorString(e));
+    if (total) CUDA_TRY(h, cudaMemcpy(hits.data(), dhits, (size_t)total * sizeof(uint2), cudaMemcpyDeviceToHost));
+    std::vector<u32> idmap((size_t)h->n);
+    CUDA_TRY(h, cudaMemcpy(idmap.data(), h->in_id, (size_t)h->n * sizeof(u32), cudaMemcpyDeviceToHost));
     std::sort(hits.begin(), hits.end(), [](const uint2 &a, const uint2 &b) { return a.x != b.x ? a.x < b.x : a.y < b.y; });
     for (const uint2 &hq : hits) offsets[hq.x + 1]++;
     for (u64 q = 0; q < nq; ++q) offsets[q + 1] += offsets[q];
@@ -1240,24 +1229,19 @@ int rcd_classify_patterns(rcd_handle h, uint64_t n, uint32_t stride, const doubl
     if (!h || (n && (!samples || !count || !pattern_out)) || stride == 0) return RCD_EINVAL;
     if (n == 0) return RCD_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    double *ds = nullptr;
-    u32 *dc = nullptr;
-    uint8_t *dout = nullptr;
     const size_t ns = (size_t)n * stride * 4;
-    cudaError_t e = dev_alloc(&ds, ns);
-    if (e == cudaSuccess) e = dev_alloc(&dc, (size_t)n);
-    if (e == cudaSuccess) e = dev_alloc(&dout, (size_t)n);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(ds, samples, ns * sizeof(double), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dc, count, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) {
-        k_classify_patterns<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>((u32)n, stride, ds, dc, dout);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(pattern_out, dout, (size_t)n, cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    cudaFree(ds); cudaFree(dc); cudaFree(dout);
-    if (e != cudaSuccess) return fail(h, e == cudaErrorMemoryAllocation ? RCD_ENOMEM : RCD_ECUDA,
-                                      std::string("rcd_classify_patterns: ") + cudaGetErrorString(e));
+    DevBuf<double> ds;
+    DevBuf<u32> dc;
+    DevBuf<uint8_t> dout;
+    CUDA_TRY(h, ds.alloc(ns));
+    CUDA_TRY(h, dc.alloc(n));
+    CUDA_TRY(h, dout.alloc(n));
+    CUDA_TRY(h, cudaMemcpyAsync(ds, samples, ns * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(dc, count, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream));
+    k_classify_patterns<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>((u32)n, stride, ds, dc, dout);
+    CUDA_TRY(h, cudaGetLastError());
+    CUDA_TRY(h, cudaMemcpyAsync(pattern_out, dout, (size_t)n, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     ++h->launches;
     return RCD_OK;
 }
@@ -1272,22 +1256,17 @@ int rcd_pair_exact(rcd_handle h, uint64_t n, const rcd_object *a, const rcd_obje
     const double nsteps = std::floor(time_window / time_step);  // int(time_window / time_step), :322
     const int steps = nsteps > 1.0e9 ? 1000000000 : (int)nsteps;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    rcd_object *da = nullptr, *db = nullptr;
-    rcd_pair_exact_result *dout = nullptr;
-    cudaError_t e = dev_alloc(&da, (size_t)n);
-    if (e == cudaSuccess) e = dev_alloc(&db, (size_t)n);
-    if (e == cudaSuccess) e = dev_alloc(&dout, (size_t)n);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(da, a, (size_t)n * sizeof(rcd_object), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(db, b, (size_t)n * sizeof(rcd_object), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) {
-        k_pair_exact<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>((u32)n, da, db, steps, time_step, dout);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, (size_t)n * sizeof(rcd_pair_exact_result), cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    cudaFree(da); cudaFree(db); cudaFree(dout);
-    if (e != cudaSuccess) return fail(h, e == cudaErrorMemoryAllocation ? RCD_ENOMEM : RCD_ECUDA,
-                                      std::string("rcd_pair_exact: ") + cudaGetErrorString(e));
+    DevBuf<rcd_object> da, db;
+    DevBuf<rcd_pair_exact_result> dout;
+    CUDA_TRY(h, da.alloc(n));
+    CUDA_TRY(h, db.alloc(n));
+    CUDA_TRY(h, dout.alloc(n));
+    CUDA_TRY(h, cudaMemcpyAsync(da, a, (size_t)n * sizeof(rcd_object), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(db, b, (size_t)n * sizeof(rcd_object), cudaMemcpyHostToDevice, h->stream));
+    k_pair_exact<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>((u32)n, da, db, steps, time_step, dout);
+    CUDA_TRY(h, cudaGetLastError());
+    CUDA_TRY(h, cudaMemcpyAsync(out, dout, (size_t)n * sizeof(rcd_pair_exact_result), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     ++h->launches;
     return RCD_OK;
 }
@@ -1297,19 +1276,14 @@ int rcd_risk_assessment(rcd_handle h, uint64_t n, const double *in, double *risk
     if (n == 0) return RCD_OK;
     if (n > 0x7fffffffull) return fail(h, RCD_ECAPACITY, "rcd_risk_assessment: too many records");
     CUDA_TRY(h, cudaSetDevice(h->device));
-    double *din = nullptr, *dout = nullptr;
-    cudaError_t e = dev_alloc(&din, 7 * (size_t)n);
-    if (e == cudaSuccess) e = dev_alloc(&dout, (size_t)n);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(din, in, 7 * (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) {
-        k_risk_assessment<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>((u32)n, din, dout);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(risk_out, dout, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    cudaFree(din); cudaFree(dout);
-    if (e != cudaSuccess) return fail(h, e == cudaErrorMemoryAllocation ? RCD_ENOMEM : RCD_ECUDA,
-                                      std::string("rcd_risk_assessment: ") + cudaGetErrorString(e));
+    DevBuf<double> din, dout;
+    CUDA_TRY(h, din.alloc(7 * (size_t)n));
+    CUDA_TRY(h, dout.alloc(n));
+    CUDA_TRY(h, cudaMemcpyAsync(din, in, 7 * (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    k_risk_assessment<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>((u32)n, din, dout);
+    CUDA_TRY(h, cudaGetLastError());
+    CUDA_TRY(h, cudaMemcpyAsync(risk_out, dout, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     ++h->launches;
     return RCD_OK;
 }
@@ -1319,21 +1293,18 @@ int rcd_history_configure(rcd_handle h, uint32_t max_history) {
     if (max_history < 2 || max_history > 4096) return fail(h, RCD_EINVAL, "rcd_history_configure: max_history must be in [2, 4096]");
     CUDA_TRY(h, cudaSetDevice(h->device));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    cudaFree(h->traj); cudaFree(h->traj_count);
-    h->traj = nullptr; h->traj_count = nullptr; h->traj_len = 0;
-    CUDA_TRY(h, dev_alloc(&h->traj, (size_t)max_history * h->cap));
-    CUDA_TRY(h, dev_alloc(&h->traj_count, (size_t)h->cap));
+    h->traj.reset(); h->traj_count.reset(); h->traj_len = 0;
+    CUDA_TRY(h, h->traj.alloc((size_t)max_history * h->cap));
+    CUDA_TRY(h, h->traj_count.alloc(h->cap));
     CUDA_TRY(h, cudaMemsetAsync(h->traj_count, 0, (size_t)h->cap * sizeof(u32), h->stream));
     h->traj_len = max_history;
     return RCD_OK;
 }
 
-static int history_ready(rcd_handle h, const char *who) {
+static int history_ready(rcd_handle h) {
     if (h->traj_len == 0) {
-        int rc = rcd_history_configure(h, 100);  // max_history_length = 100 (collision_detection.py:539)
-        if (rc) return rc;
+        RC_TRY(rcd_history_configure(h, 100));  // max_history_length = 100 (collision_detection.py:539)
     }
-    (void)who;
     return RCD_OK;
 }
 
@@ -1343,24 +1314,19 @@ int rcd_history_append(rcd_handle h, uint64_t n, const uint32_t *slot, const dou
     if (n > h->cap) return fail(h, RCD_ECAPACITY, "rcd_history_append: n exceeds max_objects");
     if (n == 0) return RCD_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    int rc = history_ready(h, "rcd_history_append");
-    if (rc) return rc;
-    double *d = nullptr;
-    u32 *ds = nullptr;
-    CUDA_TRY(h, dev_alloc(&d, 4 * (size_t)n));
-    cudaError_t e = slot ? dev_alloc(&ds, (size_t)n) : cudaSuccess;
+    RC_TRY(history_ready(h));
+    DevBuf<double> d;
+    DevBuf<u32> ds;
+    CUDA_TRY(h, d.alloc(4 * (size_t)n));
+    if (slot) CUDA_TRY(h, ds.alloc(n));
     const double *src[4] = {x, y, z, t};
-    for (int k = 0; k < 4 && e == cudaSuccess; ++k)
-        e = cudaMemcpyAsync(d + (size_t)k * n, src[k], (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess && slot) e = cudaMemcpyAsync(ds, slot, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) {
-        k_history_append<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>((u32)n, ds, d, d + n, d + 2 * n, d + 3 * n, h->traj,
-                                                                             h->traj_count, (u32)h->cap, h->traj_len);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);  // the staging buffers are freed below
-    cudaFree(d); cudaFree(ds);
-    if (e != cudaSuccess) return fail(h, RCD_ECUDA, std::string("rcd_history_append: ") + cudaGetErrorString(e));
+    for (int k = 0; k < 4; ++k)
+        CUDA_TRY(h, cudaMemcpyAsync(d.get() + (size_t)k * n, src[k], (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    if (slot) CUDA_TRY(h, cudaMemcpyAsync(ds, slot, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream));
+    k_history_append<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>((u32)n, ds, d, d.get() + n, d.get() + 2 * n, d.get() + 3 * n,
+                                                                         h->traj, h->traj_count, (u32)h->cap, h->traj_len);
+    CUDA_TRY(h, cudaGetLastError());
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));  // the staging buffers are freed on return
     ++h->launches;
     return RCD_OK;
 }
@@ -1369,18 +1335,13 @@ int rcd_history_reset(rcd_handle h, uint64_t n, const uint32_t *slot) {
     if (!h || (n && !slot)) return RCD_EINVAL;
     if (n == 0) return RCD_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    int rc = history_ready(h, "rcd_history_reset");
-    if (rc) return rc;
-    u32 *ds = nullptr;
-    CUDA_TRY(h, dev_alloc(&ds, (size_t)n));
-    cudaError_t e = cudaMemcpyAsync(ds, slot, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) {
-        k_history_reset<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>((u32)n, ds, h->traj_count, (u32)h->cap);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    cudaFree(ds);
-    if (e != cudaSuccess) return fail(h, RCD_ECUDA, std::string("rcd_history_reset: ") + cudaGetErrorString(e));
+    RC_TRY(history_ready(h));
+    DevBuf<u32> ds;
+    CUDA_TRY(h, ds.alloc(n));
+    CUDA_TRY(h, cudaMemcpyAsync(ds, slot, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream));
+    k_history_reset<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>((u32)n, ds, h->traj_count, (u32)h->cap);
+    CUDA_TRY(h, cudaGetLastError());
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     return RCD_OK;
 }
 
@@ -1389,8 +1350,7 @@ int rcd_history_move(rcd_handle h, uint32_t dst, uint32_t src) {
     if (dst >= h->cap || src >= h->cap) return fail(h, RCD_EINVAL, "rcd_history_move: slot out of range");
     if (dst == src) return RCD_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    int rc = history_ready(h, "rcd_history_move");
-    if (rc) return rc;
+    RC_TRY(history_ready(h));
     k_history_move<<<1, 128, 0, h->stream>>>(dst, src, h->traj, h->traj_count, (u32)h->cap, h->traj_len);
     KERNEL_CHECK(h);
     return RCD_OK;
@@ -1399,10 +1359,8 @@ int rcd_history_move(rcd_handle h, uint32_t dst, uint32_t src) {
 int rcd_history_classify(rcd_handle h, uint8_t *pattern_out) {
     if (!h) return RCD_EINVAL;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    int rc = history_ready(h, "rcd_history_classify");
-    if (rc) return rc;
-    rc = wait_upload(h);
-    if (rc) return rc;
+    RC_TRY(history_ready(h));
+    RC_TRY(wait_upload(h));
     if (h->n) {
         k_history_classify<<<(unsigned)((h->n + 127) / 128), 128, 0, h->stream>>>((u32)h->n, h->traj, h->traj_count,
                                                                                   (u32)h->cap, h->traj_len, h->in_pattern);
@@ -1412,7 +1370,7 @@ int rcd_history_classify(rcd_handle h, uint8_t *pattern_out) {
             CUDA_TRY(h, cudaStreamSynchronize(h->stream));
         }
     }
-    h->index_valid = false;  // the pattern is packed into the cell-ordered state
+    h->idx.valid = false;  // the pattern is packed into the cell-ordered state
     h->frame_done = false;
     return RCD_OK;
 }
@@ -1425,16 +1383,11 @@ int rcd_apply_records(rcd_handle h, uint64_t n, const rcd_record *records, uint3
     if (n > 0xffffffffull / 16) return fail(h, RCD_ECAPACITY, "rcd_apply_records: batch too large");
     CUDA_TRY(h, cudaSetDevice(h->device));
     if (append_history) {
-        int rc = history_ready(h, "rcd_apply_records");
-        if (rc) return rc;
+        RC_TRY(history_ready(h));
     }
-    const bool hist = append_history && h->traj;
-    {
-        int rcw = wait_upload(h);
-        if (rcw) return rcw;
-    }
-    for (int m = 0; m < 3; ++m)
-        for (int s = 0; s < RCD_NUM_STAGES; ++s) h->stages[m][s].used = false;
+    const bool hist = append_history && h->traj.get();
+    RC_TRY(wait_upload(h));
+    reset_stages(h, -1);
     h->stage_mode = 0;
     stage_begin(h, RCD_STAGE_UPLOAD);
     if (n_objects > h->n) {
@@ -1443,36 +1396,24 @@ int rcd_apply_records(rcd_handle h, uint64_t n, const rcd_record *records, uint3
         KERNEL_CHECK(h);
     }
     const unsigned long long *dev = reinterpret_cast<const unsigned long long *>(records);
-    unsigned long long *staged = nullptr;
+    DevBuf<unsigned long long> staged;
     if (n && src == RCD_SRC_HOST) {
-        CUDA_TRY(h, dev_alloc(&staged, (size_t)n * RECORD_WORDS));
-        cudaError_t e = cudaMemcpyAsync(staged, records, (size_t)n * sizeof(rcd_record), cudaMemcpyHostToDevice, h->stream);
-        if (e != cudaSuccess) { cudaFree(staged); return fail(h, RCD_ECUDA, std::string("rcd_apply_records: ") + cudaGetErrorString(e)); }
+        CUDA_TRY(h, staged.alloc((size_t)n * RECORD_WORDS));
+        CUDA_TRY(h, cudaMemcpyAsync(staged, records, (size_t)n * sizeof(rcd_record), cudaMemcpyHostToDevice, h->stream));
         dev = staged;
     }
-    MutableState st;
-    for (int k = 0; k < 11; ++k) st.f[k] = h->in_f[k];
-    st.type = h->in_type; st.pattern = h->in_pattern; st.id = h->in_id;
-    cudaError_t e = cudaSuccess;
-    for (u32 seq = 0; n && seq <= max_seq && e == cudaSuccess; ++seq) {
+    const MutableState st = mutable_state(h);
+    for (u32 seq = 0; n && seq <= max_seq; ++seq) {
         k_apply_records<<<(unsigned)((n + APPLY_THREADS - 1) / APPLY_THREADS), APPLY_THREADS, 0, h->stream>>>(
-            (u32)n, dev, seq, (u32)n_objects, st, hist ? h->traj : nullptr, h->traj_count, (u32)h->cap, h->traj_len);
-        e = cudaGetLastError();
-        ++h->launches;
+            (u32)n, dev, seq, (u32)n_objects, st, hist ? h->traj.get() : nullptr, h->traj_count, (u32)h->cap, h->traj_len);
+        KERNEL_CHECK(h);
     }
     stage_end(h, RCD_STAGE_UPLOAD);
-    if (e == cudaSuccess) {
-        int rcr = release_inputs(h);
-        if (rcr) return rcr;
-    }
-    if (staged) {
-        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);  // the staging buffer is freed below
-        cudaFree(staged);
-    }
-    if (e != cudaSuccess) return fail(h, RCD_ECUDA, std::string("rcd_apply_records: ") + cudaGetErrorString(e));
+    RC_TRY(release_inputs(h));
+    if (staged) CUDA_TRY(h, cudaStreamSynchronize(h->stream));  // the staging buffer is freed on return
     h->n = n_objects;
     h->n_owned = n_objects;
-    h->index_valid = false;
+    h->idx.valid = false;
     h->frame_done = false;
     return RCD_OK;
 }
@@ -1482,31 +1423,21 @@ static int alerts_ready(rcd_handle h, const char *who) {
     if (!h->alert_cap) return fail(h, RCD_ESTATE, std::string(who) + ": call rcd_alerts_configure first");
     return RCD_OK;
 }
-static void alert_stats_out(rcd_handle h, rcd_alert_stats *st) {
-    if (!st) return;
-    const AlertCounters &c = *h->alert_counters_host;
-    st->n_events = c.n_events; st->n_created = c.n_created; st->n_changed = c.n_changed;
-    st->n_refreshed = c.n_refreshed; st->n_expired = c.n_expired; st->n_live = c.n_live; st->n_dropped = c.n_dropped;
-}
 // zero the per-call counters (n_live and next_id persist), run `launch`, bring counters + events back
 extern "C++" {
 template <typename F>
 static int alerts_call(rcd_handle h, rcd_alert_event *events, uint64_t cap, rcd_alert_stats *stats, bool reset_live, F launch) {
     CUDA_TRY(h, cudaSetDevice(h->device));
-    {
-        int rcj = alerts_join(h);
-        if (rcj) return rcj;
-    }
+    RC_TRY(alerts_join(h));
     CUDA_TRY(h, cudaMemsetAsync(h->alert_counters, 0, offsetof(AlertCounters, n_live), h->stream));
     if (reset_live) CUDA_TRY(h, cudaMemsetAsync(&h->alert_counters->n_live, 0, sizeof(unsigned long long), h->stream));
-    int rc = launch();
-    if (rc) return rc;
+    RC_TRY(launch());
     CUDA_TRY(h, cudaMemcpyAsync(h->alert_counters_host, h->alert_counters, sizeof(AlertCounters), cudaMemcpyDeviceToHost, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     const u64 n_ev = std::min<u64>(std::min<u64>(h->alert_counters_host->n_events, h->alert_ev_cap), cap);
     if (n_ev && events)
         CUDA_TRY(h, cudaMemcpy(events, h->alert_ev, (size_t)n_ev * sizeof(rcd_alert_event), cudaMemcpyDeviceToHost));
-    alert_stats_out(h, stats);
+    fill_alert_stats(*h->alert_counters_host, stats);
     return RCD_OK;
 }
 }  // extern "C++"
@@ -1514,20 +1445,19 @@ static int alerts_call(rcd_handle h, rcd_alert_event *events, uint64_t cap, rcd_
 int rcd_alerts_configure(rcd_handle h, uint64_t max_alerts) {
     if (!h || max_alerts == 0 || max_alerts > (1ull << 31)) return h ? fail(h, RCD_EINVAL, "rcd_alerts_configure: max_alerts must be in [1, 2^31]") : RCD_EINVAL;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    if (h->alert_stream) CUDA_TRY(h, cudaStreamSynchronize(h->alert_stream));
+    if (h->dl.alert_stream) CUDA_TRY(h, cudaStreamSynchronize(h->dl.alert_stream));
     h->alert_async = false;
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    cudaFree(h->alert_tab[0]); cudaFree(h->alert_tab[1]); cudaFree(h->alert_ev); cudaFree(h->alert_ev_alt); cudaFree(h->alert_counters);
-    if (h->alert_counters_host) cudaFreeHost(h->alert_counters_host);
-    h->alert_tab[0] = h->alert_tab[1] = nullptr; h->alert_ev = h->alert_ev_alt = nullptr; h->alert_counters = nullptr; h->alert_counters_host = nullptr;
+    h->alert_tab[0].reset(); h->alert_tab[1].reset(); h->alert_ev.reset(); h->alert_ev_alt.reset(); h->alert_counters.reset();
+    h->alert_counters_host.reset();
     h->alert_cap = 0;
     u64 cap = 1024;
     while (cap < 2 * max_alerts) cap <<= 1;  // load factor <= 0.5
-    CUDA_TRY(h, dev_alloc(&h->alert_tab[0], (size_t)cap));
-    CUDA_TRY(h, dev_alloc(&h->alert_tab[1], (size_t)cap));
-    CUDA_TRY(h, dev_alloc(&h->alert_ev, (size_t)max_alerts));
-    CUDA_TRY(h, dev_alloc(&h->alert_counters, 1));
-    CUDA_TRY(h, cudaMallocHost(reinterpret_cast<void **>(&h->alert_counters_host), sizeof(AlertCounters)));
+    CUDA_TRY(h, h->alert_tab[0].alloc(cap));
+    CUDA_TRY(h, h->alert_tab[1].alloc(cap));
+    CUDA_TRY(h, h->alert_ev.alloc(max_alerts));
+    CUDA_TRY(h, h->alert_counters.alloc());
+    CUDA_TRY(h, h->alert_counters_host.alloc());
     CUDA_TRY(h, cudaMemsetAsync(h->alert_tab[0], 0xff, (size_t)cap * sizeof(AlertEntry), h->stream));
     CUDA_TRY(h, cudaMemsetAsync(h->alert_counters, 0, sizeof(AlertCounters), h->stream));
     h->alert_cur = 0;
@@ -1541,9 +1471,7 @@ static int alerts_enqueue_update(rcd_handle h, const rcd_pair *dev_pairs, u64 n_
                                  int32_t report_refreshed, cudaStream_t on = nullptr,
                                  const unsigned long long *n_dev_detect = nullptr /* bound of the detect pass (null: n_dev) */) {
     if (n_max == 0) return RCD_OK;
-    int sms = 0;
-    CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
-    sms = std::max(1, sms);
+    const int sms = h->sms;
     u64 blocks = std::min<u64>((n_max + ALERT_THREADS - 1) / ALERT_THREADS, (u64)sms * 16);
     if (on) {
         // beside the next frame (lower-priority stream): many short-lived blocks -- about one pair per thread, sized from
@@ -1576,26 +1504,22 @@ static int alerts_update_impl(rcd_handle h, const rcd_pair *dev_pairs, u64 n_max
 
 int rcd_summary_begin(rcd_handle h, double now, int32_t report_refreshed) {
     if (!h) return RCD_EINVAL;
-    int rc = alerts_ready(h, "rcd_summary_begin");
-    if (rc) return rc;
-    rc = delivery_begin(h, "rcd_summary_begin");
-    if (rc) return rc;
-    if (!h->alert_ev_alt) CUDA_TRY(h, dev_alloc(&h->alert_ev_alt, (size_t)h->alert_ev_cap));
+    RC_TRY(alerts_ready(h, "rcd_summary_begin"));
+    RC_TRY(delivery_begin(h, "rcd_summary_begin"));
+    if (!h->alert_ev_alt) CUDA_TRY(h, h->alert_ev_alt.alloc(h->alert_ev_cap));
     std::swap(h->alert_ev, h->alert_ev_alt);  // the events of the previous summary may still be on their way to the host
     // the fold runs on alert_stream, after the frame and beside whatever the handle's stream does next (the next
     // frame writes the twin pair buffer and twin totals; other alert calls join alert_stream first)
-    cudaStream_t as = h->alert_stream;
-    CUDA_TRY(h, cudaEventRecord(h->ev_frame_done, h->stream));
-    CUDA_TRY(h, cudaStreamWaitEvent(as, h->ev_frame_done, 0));
+    cudaStream_t as = h->dl.alert_stream;
+    CUDA_TRY(h, cudaEventRecord(h->dl.ev_frame_done, h->stream));
+    CUDA_TRY(h, cudaStreamWaitEvent(as, h->dl.ev_frame_done, 0));
     CUDA_TRY(h, cudaMemsetAsync(h->alert_counters, 0, offsetof(AlertCounters, n_live), as));
-    rc = alerts_enqueue_update(h, h->out, h->max_pairs, &h->counters->n_pairs, now, report_refreshed, as, &h->counters->n_detect_end);
-    if (rc) return rc;
-    CUDA_TRY(h, cudaMemcpyAsync(h->pend_alert_counters_host, h->alert_counters, sizeof(AlertCounters), cudaMemcpyDeviceToHost, as));
+    RC_TRY(alerts_enqueue_update(h, h->fb().out, h->max_pairs, &h->fb().counters->n_pairs, now, report_refreshed, as, &h->fb().counters->n_detect_end));
+    CUDA_TRY(h, cudaMemcpyAsync(h->dl.alert_counters_host, h->alert_counters, sizeof(AlertCounters), cudaMemcpyDeviceToHost, as));
     h->pend_kind = 2;
     h->pend_ev = h->alert_ev;
-    rc = delivery_issued(h, as);
-    if (rc) return rc;
-    CUDA_TRY(h, cudaEventRecord(h->ev_alert_done, as));
+    RC_TRY(delivery_issued(h, as));
+    CUDA_TRY(h, cudaEventRecord(h->dl.ev_alert_done, as));
     h->alert_async = true;
     return RCD_OK;
 }
@@ -1606,18 +1530,15 @@ int rcd_summary_finish(rcd_handle h, rcd_alert_event *events, uint64_t cap, uint
     if (!h->download_pending || h->pend_kind != 2) return fail(h, RCD_ESTATE, "rcd_summary_finish: no summary in flight");
     if (n > h->pend_n) return fail(h, RCD_EINVAL, "rcd_summary_finish: n exceeds the frame's object count");
     CUDA_TRY(h, cudaSetDevice(h->device));
-    CUDA_TRY(h, cudaEventSynchronize(h->pend_event));
-    const AlertCounters &ac = *h->pend_alert_counters_host;
+    CUDA_TRY(h, cudaEventSynchronize(h->dl.pend_event));
+    const AlertCounters &ac = *h->dl.alert_counters_host;
     const u64 n_ev = std::min<u64>(std::min<u64>(ac.n_events, h->alert_ev_cap), cap);
-    if (n_ev) CUDA_TRY(h, cudaMemcpyAsync(events, h->pend_ev, (size_t)n_ev * sizeof(rcd_alert_event), cudaMemcpyDeviceToHost, h->copy_stream));
-    if (n) CUDA_TRY(h, cudaMemcpyAsync(risk_counts, h->pend_risk, (size_t)n * sizeof(u32), cudaMemcpyDeviceToHost, h->copy_stream));
-    if (n_ev || n) CUDA_TRY(h, cudaStreamSynchronize(h->copy_stream));
+    if (n_ev) CUDA_TRY(h, cudaMemcpyAsync(events, h->pend_ev, (size_t)n_ev * sizeof(rcd_alert_event), cudaMemcpyDeviceToHost, h->dl.copy_stream));
+    if (n) CUDA_TRY(h, cudaMemcpyAsync(risk_counts, h->pend_risk, (size_t)n * sizeof(u32), cudaMemcpyDeviceToHost, h->dl.copy_stream));
+    if (n_ev || n) CUDA_TRY(h, cudaStreamSynchronize(h->dl.copy_stream));
     if (n_events) *n_events = n_ev;
-    if (stats) {
-        stats->n_events = ac.n_events; stats->n_created = ac.n_created; stats->n_changed = ac.n_changed;
-        stats->n_refreshed = ac.n_refreshed; stats->n_expired = ac.n_expired; stats->n_live = ac.n_live; stats->n_dropped = ac.n_dropped;
-    }
-    counts_out(h, *h->pend_counters_host, counts);
+    fill_alert_stats(ac, stats);
+    fill_counts(h, *h->dl.counters_host, h->pend_n, h->pend_n_owned, counts);
     h->download_pending = false;
     return RCD_OK;
 }
@@ -1625,39 +1546,31 @@ int rcd_summary_finish(rcd_handle h, rcd_alert_event *events, uint64_t cap, uint
 int rcd_alerts_update(rcd_handle h, double now, int32_t report_refreshed, rcd_alert_event *events, uint64_t cap,
                       rcd_alert_stats *stats) {
     if (!h) return RCD_EINVAL;
-    int rc = alerts_ready(h, "rcd_alerts_update");
-    if (rc) return rc;
+    RC_TRY(alerts_ready(h, "rcd_alerts_update"));
     if (!h->frame_done) return fail(h, RCD_ESTATE, "rcd_alerts_update: no frame has been stepped");
-    return alerts_update_impl(h, h->out, h->max_pairs, &h->counters->n_pairs, now, report_refreshed, events, cap, stats);
+    return alerts_update_impl(h, h->fb().out, h->max_pairs, &h->fb().counters->n_pairs, now, report_refreshed, events, cap, stats);
 }
 
 int rcd_alerts_update_pairs(rcd_handle h, const rcd_pair *pairs, uint64_t n, double now, int32_t report_refreshed,
                             rcd_alert_event *events, uint64_t cap, rcd_alert_stats *stats) {
     if (!h || (n && !pairs)) return RCD_EINVAL;
-    int rc = alerts_ready(h, "rcd_alerts_update_pairs");
-    if (rc) return rc;
+    RC_TRY(alerts_ready(h, "rcd_alerts_update_pairs"));
     CUDA_TRY(h, cudaSetDevice(h->device));
-    rcd_pair *staged = nullptr;
+    DevBuf<rcd_pair> staged;
     if (n) {
-        CUDA_TRY(h, dev_alloc(&staged, (size_t)n));
-        cudaError_t e = cudaMemcpyAsync(staged, pairs, (size_t)n * sizeof(rcd_pair), cudaMemcpyHostToDevice, h->stream);
-        if (e != cudaSuccess) { cudaFree(staged); return fail(h, RCD_ECUDA, std::string("rcd_alerts_update_pairs: ") + cudaGetErrorString(e)); }
+        CUDA_TRY(h, staged.alloc(n));
+        CUDA_TRY(h, cudaMemcpyAsync(staged, pairs, (size_t)n * sizeof(rcd_pair), cudaMemcpyHostToDevice, h->stream));
     }
-    rc = alerts_update_impl(h, staged, n, nullptr, now, report_refreshed, events, cap, stats);  // synchronises
-    cudaFree(staged);
-    return rc;
+    return alerts_update_impl(h, staged, n, nullptr, now, report_refreshed, events, cap, stats);  // (synchronises)
 }
 
 int rcd_alerts_expire(rcd_handle h, double now, double max_age, rcd_alert_event *events, uint64_t cap, rcd_alert_stats *stats) {
     if (!h) return RCD_EINVAL;
-    int rc = alerts_ready(h, "rcd_alerts_expire");
-    if (rc) return rc;
-    rc = alerts_call(h, events, cap, stats, true, [&]() -> int {
+    RC_TRY(alerts_ready(h, "rcd_alerts_expire"));
+    const int rc = alerts_call(h, events, cap, stats, true, [&]() -> int {
         AlertEntry *src = h->alert_tab[h->alert_cur], *dst = h->alert_tab[h->alert_cur ^ 1];
         CUDA_TRY(h, cudaMemsetAsync(dst, 0xff, (size_t)h->alert_cap * sizeof(AlertEntry), h->stream));
-        int sms = 0;
-        CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
-        const unsigned blocks = (unsigned)std::min<u64>((h->alert_cap + ALERT_THREADS - 1) / ALERT_THREADS, (u64)std::max(1, sms) * 8);
+        const unsigned blocks = (unsigned)std::min<u64>((h->alert_cap + ALERT_THREADS - 1) / ALERT_THREADS, (u64)h->sms * 8);
         k_alert_expire<<<blocks, ALERT_THREADS, 0, h->stream>>>(src, h->alert_cap, now, max_age, dst, h->alert_ev, h->alert_ev_cap,
                                                                 h->alert_counters);
         KERNEL_CHECK(h);
@@ -1669,44 +1582,35 @@ int rcd_alerts_expire(rcd_handle h, double now, double max_age, rcd_alert_event 
 
 int rcd_alerts_acknowledge(rcd_handle h, uint64_t n, const uint32_t *i, const uint32_t *j, uint64_t *n_found) {
     if (!h || (n && (!i || !j))) return RCD_EINVAL;
-    int rc = alerts_ready(h, "rcd_alerts_acknowledge");
-    if (rc) return rc;
+    RC_TRY(alerts_ready(h, "rcd_alerts_acknowledge"));
     if (n_found) *n_found = 0;
     if (n == 0) return RCD_OK;
     if (n > 0xffffffffull) return fail(h, RCD_ECAPACITY, "rcd_alerts_acknowledge: too many pairs");
     CUDA_TRY(h, cudaSetDevice(h->device));
-    rc = alerts_join(h);
-    if (rc) return rc;
-    u32 *d = nullptr;
-    CUDA_TRY(h, dev_alloc(&d, 2 * (size_t)n + 1));
-    cudaError_t e = cudaMemcpyAsync(d, i, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d + n, j, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(d + 2 * n, 0, sizeof(u32), h->stream);
-    if (e == cudaSuccess) {
-        k_alert_ack<<<(unsigned)((n + ALERT_THREADS - 1) / ALERT_THREADS), ALERT_THREADS, 0, h->stream>>>(
-            d, d + n, (u32)n, h->alert_tab[h->alert_cur], h->alert_cap - 1, d + 2 * n);
-        e = cudaGetLastError();
-        ++h->launches;
-    }
+    RC_TRY(alerts_join(h));
+    DevBuf<u32> d;
+    CUDA_TRY(h, d.alloc(2 * (size_t)n + 1));
+    u32 *const di = d, *const dj = d.get() + n, *const dfound = d.get() + 2 * n;
+    CUDA_TRY(h, cudaMemcpyAsync(di, i, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(dj, j, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaMemsetAsync(dfound, 0, sizeof(u32), h->stream));
+    k_alert_ack<<<(unsigned)((n + ALERT_THREADS - 1) / ALERT_THREADS), ALERT_THREADS, 0, h->stream>>>(
+        di, dj, (u32)n, h->alert_tab[h->alert_cur], h->alert_cap - 1, dfound);
+    KERNEL_CHECK(h);
     u32 found = 0;
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&found, d + 2 * n, sizeof(u32), cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    cudaFree(d);
-    if (e != cudaSuccess) return fail(h, RCD_ECUDA, std::string("rcd_alerts_acknowledge: ") + cudaGetErrorString(e));
+    CUDA_TRY(h, cudaMemcpyAsync(&found, dfound, sizeof(u32), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     if (n_found) *n_found = found;
     return RCD_OK;
 }
 
 int rcd_alerts_download(rcd_handle h, rcd_alert_event *out, uint64_t cap, uint64_t *n_out) {
     if (!h || !n_out || (cap && !out)) return RCD_EINVAL;
-    int rc = alerts_ready(h, "rcd_alerts_download");
-    if (rc) return rc;
+    RC_TRY(alerts_ready(h, "rcd_alerts_download"));
     CUDA_TRY(h, cudaSetDevice(h->device));
     rcd_alert_stats st;
-    rc = alerts_call(h, out, cap, &st, false, [&]() -> int {
-        int sms = 0;
-        CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
-        const unsigned blocks = (unsigned)std::min<u64>((h->alert_cap + ALERT_THREADS - 1) / ALERT_THREADS, (u64)std::max(1, sms) * 8);
+    const int rc = alerts_call(h, out, cap, &st, false, [&]() -> int {
+        const unsigned blocks = (unsigned)std::min<u64>((h->alert_cap + ALERT_THREADS - 1) / ALERT_THREADS, (u64)h->sms * 8);
         k_alert_dump<<<blocks, ALERT_THREADS, 0, h->stream>>>(h->alert_tab[h->alert_cur], h->alert_cap, h->alert_ev, h->alert_ev_cap,
                                                               h->alert_counters);
         KERNEL_CHECK(h);
@@ -1724,51 +1628,37 @@ int rcd_halo_pack(rcd_handle h, int32_t n_peers, int32_t self, const float *slab
     if (!h || !slab_lo || !slab_hi || !counts || n_peers < 1 || n_peers > MAX_PEERS || self < 0 || self >= n_peers)
         return fail(h, RCD_EINVAL, "rcd_halo_pack: bad arguments");
     CUDA_TRY(h, cudaSetDevice(h->device));
-    {
-        int rcw = wait_upload(h);
-        if (rcw) return rcw;
-    }
+    RC_TRY(wait_upload(h));
     for (int p = 0; p < n_peers; ++p) counts[p] = 0;
     if (h->n_owned == 0) return RCD_OK;
     SlabParams sp;
     sp.n_peers = n_peers; sp.self = self; sp.halo = halo;
     for (int p = 0; p < n_peers; ++p) { sp.lo[p] = slab_lo[p]; sp.hi[p] = slab_hi[p]; }
-    unsigned long long *dcnt = nullptr;
-    CUDA_TRY(h, dev_alloc(&dcnt, 2 * (size_t)MAX_PEERS));
+    DevBuf<unsigned long long> dcnt;  // [MAX_PEERS] counts, then [MAX_PEERS] bases
+    CUDA_TRY(h, dcnt.alloc(2 * (size_t)MAX_PEERS));
+    unsigned long long *const dbase = dcnt.get() + MAX_PEERS;
     unsigned long long host_cnt[MAX_PEERS] = {}, host_base[MAX_PEERS] = {};
     const unsigned blocks = (unsigned)((h->n_owned + 255) / 256);
-    cudaError_t e = cudaMemsetAsync(dcnt, 0, 2 * MAX_PEERS * sizeof(unsigned long long), h->stream);
-    if (e == cudaSuccess) {
-        k_halo_pack<<<blocks, 256, 0, h->stream>>>((u32)h->n_owned, input_state(h), sp, 0, dcnt, dcnt + MAX_PEERS, nullptr, 0);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(host_cnt, dcnt, n_peers * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    CUDA_TRY(h, cudaMemsetAsync(dcnt, 0, 2 * MAX_PEERS * sizeof(unsigned long long), h->stream));
+    k_halo_pack<<<blocks, 256, 0, h->stream>>>((u32)h->n_owned, input_state(h), sp, 0, dcnt, dbase, nullptr, 0);
+    CUDA_TRY(h, cudaGetLastError());
+    CUDA_TRY(h, cudaMemcpyAsync(host_cnt, dcnt, n_peers * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     u64 total = 0;
-    if (e == cudaSuccess) {
-        for (int p = 0; p < n_peers; ++p) { host_base[p] = total; total += host_cnt[p]; counts[p] = host_cnt[p]; }
-        if (!out_records && cap == 0) {  // counting pass only
-            cudaFree(dcnt);
-            ++h->launches;
-            return RCD_OK;
-        }
-        if (total > cap || (total && !out_records)) {
-            cudaFree(dcnt);
-            return fail(h, RCD_ECAPACITY, "rcd_halo_pack: record buffer too small");
-        }
+    for (int p = 0; p < n_peers; ++p) { host_base[p] = total; total += host_cnt[p]; counts[p] = host_cnt[p]; }
+    if (!out_records && cap == 0) {  // counting pass only
+        ++h->launches;
+        return RCD_OK;
     }
-    if (e == cudaSuccess && total) {
-        e = cudaMemsetAsync(dcnt, 0, MAX_PEERS * sizeof(unsigned long long), h->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(dcnt + MAX_PEERS, host_base, n_peers * sizeof(unsigned long long), cudaMemcpyHostToDevice, h->stream);
-        if (e == cudaSuccess) {
-            k_halo_pack<<<blocks, 256, 0, h->stream>>>((u32)h->n_owned, input_state(h), sp, 1, dcnt, dcnt + MAX_PEERS,
-                                                      static_cast<u32 *>(out_records), cap);
-            e = cudaGetLastError();
-        }
-        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    if (total > cap || (total && !out_records)) return fail(h, RCD_ECAPACITY, "rcd_halo_pack: record buffer too small");
+    if (total) {
+        CUDA_TRY(h, cudaMemsetAsync(dcnt, 0, MAX_PEERS * sizeof(unsigned long long), h->stream));
+        CUDA_TRY(h, cudaMemcpyAsync(dbase, host_base, n_peers * sizeof(unsigned long long), cudaMemcpyHostToDevice, h->stream));
+        k_halo_pack<<<blocks, 256, 0, h->stream>>>((u32)h->n_owned, input_state(h), sp, 1, dcnt, dbase,
+                                                  static_cast<u32 *>(out_records), cap);
+        CUDA_TRY(h, cudaGetLastError());
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     }
-    cudaFree(dcnt);
-    if (e != cudaSuccess) return fail(h, RCD_ECUDA, std::string("rcd_halo_pack: ") + cudaGetErrorString(e));
     h->launches += total ? 2 : 1;
     return RCD_OK;
 }
@@ -1779,10 +1669,7 @@ int rcd_halo_pack_async(rcd_handle h, int32_t n_peers, int32_t self, const float
         self < 0 || self >= n_peers)
         return fail(h, RCD_EINVAL, "rcd_halo_pack_async: bad arguments");
     CUDA_TRY(h, cudaSetDevice(h->device));
-    {
-        int rcw = wait_upload(h);
-        if (rcw) return rcw;
-    }
+    RC_TRY(wait_upload(h));
     SlabParams sp;
     sp.n_peers = n_peers; sp.self = self; sp.halo = halo;
     SlabRegions rg;
@@ -1808,22 +1695,14 @@ int rcd_halo_append(rcd_handle h, const void *records, uint64_t n_records) {
     if (h->n + n_records > h->cap) return fail(h, RCD_ECAPACITY, "rcd_halo_append: exceeds max_objects");
     if (n_records == 0) return RCD_OK;
     CUDA_TRY(h, cudaSetDevice(h->device));
-    {
-        int rcw = wait_upload(h);
-        if (rcw) return rcw;
-    }
-    MutableState st;
-    for (int k = 0; k < 11; ++k) st.f[k] = h->in_f[k];
-    st.type = h->in_type; st.pattern = h->in_pattern; st.id = h->in_id;
+    RC_TRY(wait_upload(h));
+    const MutableState st = mutable_state(h);
     k_halo_append<<<(unsigned)((n_records + 255) / 256), 256, 0, h->stream>>>(static_cast<const u32 *>(records),
                                                                              (u32)n_records, (u32)h->n, st);
     KERNEL_CHECK(h);
-    {
-        int rcr = release_inputs(h);
-        if (rcr) return rcr;
-    }
+    RC_TRY(release_inputs(h));
     h->n += n_records;
-    h->index_valid = false;
+    h->idx.valid = false;
     h->frame_done = false;
     return RCD_OK;
 }
@@ -1856,7 +1735,7 @@ int rcd_pair_tests(rcd_handle h, uint64_t *n) {
     if (!h || !n) return RCD_EINVAL;
     if (!h->frame_done) return fail(h, RCD_ESTATE, "rcd_pair_tests: no frame has been stepped");
     CUDA_TRY(h, cudaSetDevice(h->device));
-    CUDA_TRY(h, cudaMemcpyAsync(h->counters_host, h->counters, sizeof(Counters), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(h->counters_host, h->fb().counters, sizeof(Counters), cudaMemcpyDeviceToHost, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     *n = h->counters_host->n_tests;
     return RCD_OK;
@@ -1873,7 +1752,7 @@ int rcd_sync(rcd_handle h) {
     CUDA_TRY(h, cudaSetDevice(h->device));
     CUDA_TRY(h, cudaStreamSynchronize(h->up_stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    if (h->alert_stream) CUDA_TRY(h, cudaStreamSynchronize(h->alert_stream));
+    if (h->dl.alert_stream) CUDA_TRY(h, cudaStreamSynchronize(h->dl.alert_stream));
     return RCD_OK;
 }
 
