@@ -1331,29 +1331,35 @@ __global__ void __launch_bounds__(PAIR_THREADS, SLOW ? 4 : RCD_PAIR_MIN_BLOCKS) 
 // -------------------------------------------------------------------------------------------------
 // k_narrow: QA -> Q3.  A warp takes 32 queued pairs at a time and works through them in phases with
 // different lane assignments, so that every phase runs with (almost) full warps although the pairs
-// carry different numbers of offsets:
-//   1. lane = pair            : gather both objects; detect narrow phase (-> Q3); predict: the time window
-//                               that can hold a hit -> offsets, coefficients of the pair -> shared memory
-//   2. lane = (pair, offset)  : can the offset be hit at all (offset_may_hit)?  is the neighbour within
-//                               100 m of the predicted centre (:801-803)?  survivors -> item list
+// carry different numbers of offsets.  Phase 1 runs on every batch.  Only some of a batch's pairs have
+// offsets to look at, so those wait in a warp-private ring in shared memory, and phases 2-4 run on groups
+// of 32 of them (on what is left once more after the warp's last batch):
+//   1. lane = pair            : gather both objects; detect narrow phase (-> Q3); predict: the offsets whose
+//                               samples can reach the safe distance -> (si, sj, offset mask) into the ring
+//   group start, lane = pair  : gather the pair again (an L1 / L2 hit) and rebuild its coefficients -> shared memory
+//   2. lane = (pair, offset)  : is the neighbour within 100 m of the predicted centre (:801-803)?  survivors ->
+//                               item list
 //   3. lane = surviving item  : the 10 samples of the offset (:322-342) in fp32 -> first sample inside
 //                               safe + band and its squared distance -> shared memory
 //   4. lane = pair            : merge over the offsets (max risk, earliest offset on ties, :848-865)
 //                               -> 0 / RESOLVED | m | k << 8 / mask of the offsets fp64 must decide
+// The ring holds 12 bytes per pair and the coefficients are rebuilt: keeping them in the ring instead would
+// cost 6.4 KB more per warp, and the kernel would lose its 8 blocks per SM.
 // sample_predict() above is the decision of phases 2-4 for one pair on one thread (queue-overflow fallback).
 // -------------------------------------------------------------------------------------------------
 constexpr int STAGE_THREADS = 128;
 constexpr int STAGE_WARPS = STAGE_THREADS / 32;
-constexpr int SC = 27;  // coefficients per pair (odd stride: conflict-free)
-enum { SC_D = 0, SC_CV = 3, SC_CA = 6, SC_RV = 9, SC_RA = 12, SC_UV = 15, SC_UA = 18, SC_HR2 = 21, SC_INVRV2 = 22,
-       SC_LIM2 = 23, SC_SAFEB2 = 24, SC_SAFEIN2 = 25, SC_INVSAFE = 26 };
+constexpr int SC = 25;  // coefficients per pair (odd stride: conflict-free)
+enum { SC_D = 0, SC_CV = 3, SC_CA = 6, SC_RV = 9, SC_RA = 12, SC_UV = 15, SC_UA = 18, SC_SAFEB2 = 21, SC_SAFEIN2 = 22,
+       SC_INVSAFE = 23 };
+constexpr u32 NARROW_RING = 64;  // pending predict pairs of a warp: fewer than 32 left over + one batch
 struct SampleShared {
-    float coef[32][SC];
+    float coef[32][SC];                        // of the group's pairs
     float part[32][PREDICT_OFFSETS];           // offset-dependent part of the risk of a certain hit (< 0: undecided in
                                                // fp32), with the index of the first sample in the 4 lowest mantissa bits
     u32 hit_mask[32];                          // offsets with a sample within safe + band
-    u32 si[32], sj[32];
-    unsigned short items[64];                  // pair | offset << 5
+    QEntry ring[NARROW_RING];                  // predict pairs waiting for phases 2-4: {si, sj, offset mask}
+    unsigned short items[64];                  // pair of the group | offset << 5
 };
 constexpr int QA_BATCHES_PER_BLOCK = QA_BLOCK / 32;
 constexpr u32 SAMPLE_ITEMS = 32u;  // items per pass of the sample phase (two lanes per item, 5 samples each, measured slower)
@@ -1394,6 +1400,7 @@ __global__ void __launch_bounds__(STAGE_THREADS, RCD_NARROW_MIN_BLOCKS) k_narrow
     const unsigned long long wstride = (unsigned long long)gridDim.x * STAGE_WARPS;
     const float R2 = PREDICT_RADIUS * PREDICT_RADIUS;
     u32 n_exact = 0, n_pot = 0;
+    u32 head = 0, n_pend = 0;  // (warp-uniform) the pending pairs are sh.ring[(head + k) % NARROW_RING], k < n_pend
     // the queue entry of a batch (loaded one batch ahead of its use); x = 0xffffffff: none
     auto fetch = [&](unsigned long long batch) {
         uint2 e = make_uint2(0xffffffffu, 0u);
@@ -1403,91 +1410,30 @@ __global__ void __launch_bounds__(STAGE_THREADS, RCD_NARROW_MIN_BLOCKS) k_narrow
         }
         return e;
     };
-    unsigned long long batch = (unsigned long long)blockIdx.x * STAGE_WARPS + (threadIdx.x >> 5);
-    uint2 e_next = fetch(batch);
-    for (; batch < nbatch; batch += wstride) {
-        const uint2 e = e_next;
-        e_next = fetch(batch + wstride);
-        if (!__any_sync(FULL_MASK, e.x != 0xffffffffu)) continue;  // the warp that owned the block stopped before this batch
-        // ---- 1. lane = pair ------------------------------------------------------------------------
-        u32 si = 0, sj = 0, mask = 0, det_word = 0;
-        bool det_keep = false;
-        if (e.x != 0xffffffffu) {
-            si = e.x & QA_SI_MASK;
-            sj = e.y;
-            const bool inr = (e.x & QA_INR) != 0, und = (e.x & QA_UND) != 0;
-            if (si != sj || MODE == RCD_MODE_COMPUTE_NODE) {  // _spatial_filtering strips self (:224-225)
-                const float4 a0 = P.P0[si], a1 = P.P1[si], a2 = P.P2[si];
-                const float4 b0 = P.P0[sj], b1 = P.P1[sj], b2 = P.P2[sj];
-                if (MODE == RCD_MODE_DETECT) {
-                    det_keep = und || narrow_detect(a0, a1, a2, b0, b1, b2, P.T);
-                    det_word = und ? RADIUS_UNDECIDED : 0u;
-                } else if (MODE == RCD_MODE_COMPUTE_NODE) {
-                    det_keep = narrow_compute_node(P, a0, a1, a2, b0, b1, b2, si == sj, und);
-                    det_word = und ? RADIUS_UNDECIDED : 0u;
-                } else {
-                    const u32 pat = meta_pattern(__float_as_uint(a2.w));
-                    const bool nohist = pat == RCD_PAT_NO_HISTORY;
-                    if ((nohist || FUSED) && (inr || und)) {  // detect_collisions(100.0, 10.0): the defaults (:592)
-                        const bool twice = nohist && FUSED;
-                        det_keep = und || narrow_detect(a0, a1, a2, b0, b1, b2, 10.0f);
-                        det_word = (und ? RADIUS_UNDECIDED : 0u) | (twice ? ENTRY_TWICE : 0u);
-                    }
-                    if (!nohist) {
-                        const PredictCoef c = predict_coef(a0, a1, a2, b0, b1, b2, pat);
-                        if (COUNT_CAND) {
-                            mask = predict_mask<true>(P, a0, a1, a2, b0, b1, b2, si, sj, pat, n_exact);
-                        } else {
-                            // the offsets whose 10 samples can come within the safe distance at all (offset_may_hit): the
-                            // samples leave the offset state g(t_m) = centre_i(t_m) - predicted_j(t_m) along rv tau (+ at most
-                            // 0.405 |ra|), tau in [0, 0.9] -- closest point of that segment to the origin, two offsets per
-                            // packed instruction
-                            const float nir = -c.inv_rv2 * (1.0f / 0.9f);
-                            const float r9x = 0.9f * c.rvx, r9y = 0.9f * c.rvy, r9z = 0.9f * c.rvz;
-                            u32 fmask = 0;
-#pragma unroll
-                            for (int m = 0; m < PREDICT_OFFSETS; m += 2) {
-                                const float2 t2 = make_float2(0.5f * (float)m, 0.5f * (float)(m + 1));
-                                const float2 h2 = make_float2(0.125f * (float)(m * m), 0.125f * (float)((m + 1) * (m + 1)));
-                                const float2 gx = fma2(splat2(c.cvx), t2, fma2(splat2(c.cax), h2, splat2(-c.dx)));
-                                const float2 gy = fma2(splat2(c.cvy), t2, fma2(splat2(c.cay), h2, splat2(-c.dy)));
-                                const float2 gz = fma2(splat2(c.cvz), t2, fma2(splat2(c.caz), h2, splat2(-c.dz)));
-                                const float2 dot = fma2(gz, splat2(c.rvz), fma2(gy, splat2(c.rvy), mul2(gx, splat2(c.rvx))));
-                                const float2 sc = make_float2(__saturatef(dot.x * nir), __saturatef(dot.y * nir));  // tau / 0.9
-                                const float2 ex = fma2(splat2(r9x), sc, gx), ey = fma2(splat2(r9y), sc, gy), ez = fma2(splat2(r9z), sc, gz);
-                                const float2 e2 = fma2(ez, ez, fma2(ey, ey, mul2(ex, ex)));
-                                const float2 tf = fma2(e2, splat2(-1.0f), splat2(c.lim2));  // < 0 <=> out of reach
-                                fmask = shift_in_sign(shift_in_sign(fmask, tf.x), tf.y);
-                            }
-                            // offset m failed <=> bit (PREDICT_OFFSETS - 1 - m) of fmask
-                            mask = (~__brev(fmask) >> (32 - PREDICT_OFFSETS)) & ((1u << PREDICT_OFFSETS) - 1u);
-                        }
-                        if (mask) {
-                            float *o = sh.coef[lane];
-                            o[SC_D] = c.dx; o[SC_D + 1] = c.dy; o[SC_D + 2] = c.dz;
-                            o[SC_CV] = c.cvx; o[SC_CV + 1] = c.cvy; o[SC_CV + 2] = c.cvz;
-                            o[SC_CA] = c.cax; o[SC_CA + 1] = c.cay; o[SC_CA + 2] = c.caz;
-                            o[SC_RV] = c.rvx; o[SC_RV + 1] = c.rvy; o[SC_RV + 2] = c.rvz;
-                            o[SC_RA] = a2.x - b2.x; o[SC_RA + 1] = a2.y - b2.y; o[SC_RA + 2] = a2.z - b2.z;
-                            o[SC_UV] = c.uvx; o[SC_UV + 1] = c.uvy; o[SC_UV + 2] = c.uvz;
-                            o[SC_UA] = c.uax; o[SC_UA + 1] = c.uay; o[SC_UA + 2] = c.uaz;
-                            o[SC_SAFEB2] = c.safe_b2;  // (SC_HR2 / SC_INVRV2 / SC_LIM2 were phase 2's: taken in phase 1 now)
-                            const float safe_in = fmaxf(c.safe - (c.safe_b - c.safe), 0.0f);  // safe minus the guard band
-                            o[SC_SAFEIN2] = safe_in * safe_in;
-                            o[SC_INVSAFE] = rcp_fast(c.safe);  // (feeds the fp32 merge key only: ~1e-7 relative)
-                        }
-                    }
-                }
-            }
+
+    // ---- phases 2-4 on the first ng (<= 32) pending pairs: lane (and pr below) = position in the group ------
+    auto run_group = [&](u32 ng) {
+        u32 si = 0, sj = 0, mask = 0;
+        if (lane < ng) {
+            const QEntry q = sh.ring[(head + lane) % NARROW_RING];
+            si = q.si; sj = q.sj; mask = q.mask;
+            const float4 a0 = P.P0[si], a1 = P.P1[si], a2 = P.P2[si];
+            const float4 b0 = P.P0[sj], b1 = P.P1[sj], b2 = P.P2[sj];
+            const PredictCoef c = predict_coef(a0, a1, a2, b0, b1, b2, meta_pattern(__float_as_uint(a2.w)));
+            float *o = sh.coef[lane];
+            o[SC_D] = c.dx; o[SC_D + 1] = c.dy; o[SC_D + 2] = c.dz;
+            o[SC_CV] = c.cvx; o[SC_CV + 1] = c.cvy; o[SC_CV + 2] = c.cvz;
+            o[SC_CA] = c.cax; o[SC_CA + 1] = c.cay; o[SC_CA + 2] = c.caz;
+            o[SC_RV] = c.rvx; o[SC_RV + 1] = c.rvy; o[SC_RV + 2] = c.rvz;
+            o[SC_RA] = a2.x - b2.x; o[SC_RA + 1] = a2.y - b2.y; o[SC_RA + 2] = a2.z - b2.z;
+            o[SC_UV] = c.uvx; o[SC_UV + 1] = c.uvy; o[SC_UV + 2] = c.uvz;
+            o[SC_UA] = c.uax; o[SC_UA + 1] = c.uay; o[SC_UA + 2] = c.uaz;
+            o[SC_SAFEB2] = c.safe_b2;
+            const float safe_in = fmaxf(c.safe - (c.safe_b - c.safe), 0.0f);  // safe minus the guard band
+            o[SC_SAFEIN2] = safe_in * safe_in;
+            o[SC_INVSAFE] = rcp_fast(c.safe);  // (feeds the fp32 merge key only: ~1e-7 relative)
         }
-        if (!push_detect(P, det_keep, si, sj, det_word))
-            n_pot += finish_entry_inline<MODE>(P, si, sj, det_word);  // queue full: decide here
-        if (!PRED) continue;
-        mask &= (1u << PREDICT_OFFSETS) - 1u;
-        if (!__any_sync(FULL_MASK, mask != 0)) continue;
         sh.hit_mask[lane] = 0;
-        sh.si[lane] = si;
-        sh.sj[lane] = sj;
         const u32 cnt = (u32)__popc(mask);
         u32 off = cnt;
 #pragma unroll
@@ -1565,8 +1511,8 @@ __global__ void __launch_bounds__(STAGE_THREADS, RCD_NARROW_MIN_BLOCKS) k_narrow
                         pass = c2 <= R2 * (1.0f + BAND_R2);
                         if (pass && c2 >= R2 * (1.0f - BAND_R2)) {
                             ++n_exact;
-                            const u32 psi = sh.si[pr], psj = sh.sj[pr];
-                            pass = exact_predict_radius(P, psi, psj, meta_pattern(__float_as_uint(P.P2[psi].w)), (int)m);
+                            const QEntry q = sh.ring[(head + pr) % NARROW_RING];
+                            pass = exact_predict_radius(P, q.si, q.sj, meta_pattern(__float_as_uint(P.P2[q.si].w)), (int)m);
                         }
                     }
                 }
@@ -1604,7 +1550,91 @@ __global__ void __launch_bounds__(STAGE_THREADS, RCD_NARROW_MIN_BLOCKS) k_narrow
         }
         if (!push_predict(P, word != 0, si, sj, word))
             finish_entry_inline<RCD_MODE_PREDICT>(P, si, sj, word);
-        __syncwarp();  // the next batch overwrites this warp's shared memory
+        __syncwarp();  // the next group overwrites this warp's shared memory (and the next batch these ring slots)
+    };
+
+    unsigned long long batch = (unsigned long long)blockIdx.x * STAGE_WARPS + (threadIdx.x >> 5);
+    uint2 e_next = fetch(batch);
+    for (;; batch += wstride) {
+        const bool more = batch < nbatch;  // false: one more pass, for the pairs still in the ring
+        const uint2 e = e_next;
+        if (more) e_next = fetch(batch + wstride);
+        // (no entry in the batch: the warp that owned the block stopped before it)
+        if (more && __any_sync(FULL_MASK, e.x != 0xffffffffu)) {
+            // ---- 1. lane = pair ------------------------------------------------------------------------
+            u32 si = 0, sj = 0, mask = 0, det_word = 0;
+            bool det_keep = false;
+            if (e.x != 0xffffffffu) {
+                si = e.x & QA_SI_MASK;
+                sj = e.y;
+                const bool inr = (e.x & QA_INR) != 0, und = (e.x & QA_UND) != 0;
+                if (si != sj || MODE == RCD_MODE_COMPUTE_NODE) {  // _spatial_filtering strips self (:224-225)
+                    const float4 a0 = P.P0[si], a1 = P.P1[si], a2 = P.P2[si];
+                    const float4 b0 = P.P0[sj], b1 = P.P1[sj], b2 = P.P2[sj];
+                    if (MODE == RCD_MODE_DETECT) {
+                        det_keep = und || narrow_detect(a0, a1, a2, b0, b1, b2, P.T);
+                        det_word = und ? RADIUS_UNDECIDED : 0u;
+                    } else if (MODE == RCD_MODE_COMPUTE_NODE) {
+                        det_keep = narrow_compute_node(P, a0, a1, a2, b0, b1, b2, si == sj, und);
+                        det_word = und ? RADIUS_UNDECIDED : 0u;
+                    } else {
+                        const u32 pat = meta_pattern(__float_as_uint(a2.w));
+                        const bool nohist = pat == RCD_PAT_NO_HISTORY;
+                        if ((nohist || FUSED) && (inr || und)) {  // detect_collisions(100.0, 10.0): the defaults (:592)
+                            const bool twice = nohist && FUSED;
+                            det_keep = und || narrow_detect(a0, a1, a2, b0, b1, b2, 10.0f);
+                            det_word = (und ? RADIUS_UNDECIDED : 0u) | (twice ? ENTRY_TWICE : 0u);
+                        }
+                        if (!nohist) {
+                            if (COUNT_CAND) {
+                                mask = predict_mask<true>(P, a0, a1, a2, b0, b1, b2, si, sj, pat, n_exact);
+                            } else {
+                                // the offsets whose 10 samples can come within the safe distance at all (offset_may_hit): the
+                                // samples leave the offset state g(t_m) = centre_i(t_m) - predicted_j(t_m) along rv tau (+ at most
+                                // 0.405 |ra|), tau in [0, 0.9] -- closest point of that segment to the origin, two offsets per
+                                // packed instruction
+                                const PredictCoef c = predict_coef(a0, a1, a2, b0, b1, b2, pat);
+                                const float nir = -c.inv_rv2 * (1.0f / 0.9f);
+                                const float r9x = 0.9f * c.rvx, r9y = 0.9f * c.rvy, r9z = 0.9f * c.rvz;
+                                u32 fmask = 0;
+#pragma unroll
+                                for (int m = 0; m < PREDICT_OFFSETS; m += 2) {
+                                    const float2 t2 = make_float2(0.5f * (float)m, 0.5f * (float)(m + 1));
+                                    const float2 h2 = make_float2(0.125f * (float)(m * m), 0.125f * (float)((m + 1) * (m + 1)));
+                                    const float2 gx = fma2(splat2(c.cvx), t2, fma2(splat2(c.cax), h2, splat2(-c.dx)));
+                                    const float2 gy = fma2(splat2(c.cvy), t2, fma2(splat2(c.cay), h2, splat2(-c.dy)));
+                                    const float2 gz = fma2(splat2(c.cvz), t2, fma2(splat2(c.caz), h2, splat2(-c.dz)));
+                                    const float2 dot = fma2(gz, splat2(c.rvz), fma2(gy, splat2(c.rvy), mul2(gx, splat2(c.rvx))));
+                                    const float2 sc = make_float2(__saturatef(dot.x * nir), __saturatef(dot.y * nir));  // tau / 0.9
+                                    const float2 ex = fma2(splat2(r9x), sc, gx), ey = fma2(splat2(r9y), sc, gy), ez = fma2(splat2(r9z), sc, gz);
+                                    const float2 e2 = fma2(ez, ez, fma2(ey, ey, mul2(ex, ex)));
+                                    const float2 tf = fma2(e2, splat2(-1.0f), splat2(c.lim2));  // < 0 <=> out of reach
+                                    fmask = shift_in_sign(shift_in_sign(fmask, tf.x), tf.y);
+                                }
+                                // offset m failed <=> bit (PREDICT_OFFSETS - 1 - m) of fmask
+                                mask = (~__brev(fmask) >> (32 - PREDICT_OFFSETS)) & ((1u << PREDICT_OFFSETS) - 1u);
+                            }
+                        }
+                    }
+                }
+            }
+            if (!push_detect(P, det_keep, si, sj, det_word))
+                n_pot += finish_entry_inline<MODE>(P, si, sj, det_word);  // queue full: decide here
+            if (PRED) {  // the pairs with offsets to look at join the ring
+                mask &= (1u << PREDICT_OFFSETS) - 1u;
+                const u32 bal = __ballot_sync(FULL_MASK, mask != 0);
+                if (mask) sh.ring[(head + n_pend + (u32)__popc(bal & lanemask_lt())) % NARROW_RING] = QEntry{si, sj, mask};
+                n_pend += (u32)__popc(bal);
+            }
+        }
+        if (PRED && (n_pend >= 32u || (!more && n_pend != 0u))) {
+            __syncwarp();  // the ring entries are written
+            const u32 ng = min(n_pend, 32u);
+            run_group(ng);
+            head = (head + ng) % NARROW_RING;
+            n_pend -= ng;
+        }
+        if (!more) break;
     }
     unsigned long long ex = warp_sum((unsigned long long)n_exact);
     unsigned long long pt = warp_sum((unsigned long long)n_pot);
