@@ -171,6 +171,25 @@ int rcd_set_patterns(rcd_handle h, uint64_t n, const uint8_t *pattern, int32_t s
  * shard: they are neighbours only (spatial slabs, SURVEY.md 8e).  Default: all owned. */
 int rcd_set_owned(rcd_handle h, uint64_t n_owned);
 
+/* Query only the listed objects in the following rcd_step calls; every object stays a neighbour.
+ * The reference's partitioned queries (collision_system.py:437-446).  slots: upload-order indices,
+ * each < n_owned, no repeats, any order; host or device memory (src), copied.  NULL: back to every
+ * owned object.  n = 0 with a non-NULL list: no queries.
+ *   - A step with query set Q emits exactly the records the same step without a list emits for i in Q
+ *     (the same bytes after rcd_download's sort).  rcd_counts_t.n_owned is |Q|; n_candidates,
+ *     n_potential, n_pairs, n_high_risk and n_alerts are the totals over Q; the per-object candidate
+ *     and risk counts are zero for objects outside Q.
+ *   - A slot >= n_owned (a halo copy) or a repeated slot: RCD_EINVAL, and the previous set stays.
+ *     Host lists are checked on the host; device lists by a kernel with one 4-byte readback, so
+ *     such a call synchronises.
+ *   - The set stays in force across steps.  rcd_upload, rcd_set_owned and rcd_truncate reset it to
+ *     every owned object; rcd_halo_append, rcd_apply_records, rcd_set_patterns, rcd_invalidate and
+ *     rcd_set_compute_node_params keep it.
+ *   - The spatial index is kept: a new set only rebuilds the query order, O(|Q|).  Like
+ *     rcd_set_owned, the call ends the frame (a following RCD_STEP_APPEND gets RCD_ESTATE).
+ *   - The first call with a list allocates about 8 bytes of device memory per object. */
+int rcd_set_queries(rcd_handle h, uint64_t n, const uint32_t *slots, int32_t src);
+
 /* Run one frame for every owned object, asynchronously on the handle's stream.
  * search_radius / time_window: the arguments of detect_collisions (collision_detection.py:110-111);
  * predict mode always uses 100.0 / 1.0 like the reference (:802, :821) and ignores them except
@@ -378,7 +397,10 @@ typedef struct {
 int rcd_alerts_configure(rcd_handle h, uint64_t max_alerts);
 /* process_collision_risks on every pair the last rcd_step(s) of this frame emitted (risk >= 0.3 only,
  * :273), with time.time() = now.  events (host, may be NULL with cap 0) receives the CREATED and
- * PRIORITY_CHANGED events, plus the REFRESHED ones if report_refreshed != 0; order is not deterministic. */
+ * PRIORITY_CHANGED events, plus the REFRESHED ones if report_refreshed != 0; order is not deterministic.
+ * After a step with a query list (rcd_set_queries) only the pairs of listed objects are folded in: the alerts
+ * of the other objects are not refreshed and age towards expiry, as the reference's alerts do for the vehicles
+ * a shard does not process. */
 int rcd_alerts_update(rcd_handle h, double now, int32_t report_refreshed, rcd_alert_event *events, uint64_t cap,
                       rcd_alert_stats *stats);
 /* The same for an explicit list of risks (host array of rcd_pair; i, j, ttc, risk, distance, priority and predicted

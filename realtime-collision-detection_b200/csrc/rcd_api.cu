@@ -100,6 +100,7 @@ struct IndexState {
     int sorted_buf = 0;
     int qorder_kind = 0;   // 0 none, 1 balls (radius queries), 2 capsules (predict queries)
     int q_sorted_buf = 0;
+    bool slot_pos = false; // q_pos holds the inverse of sorted_slot (built for a query list only)
 };
 
 // What a frame writes.  A pending delivery still reads the previous frame's set, so the handle keeps a twin.
@@ -157,13 +158,14 @@ const FrameKernels FRAME_KERNELS[5] = {
 struct StepKey {
     int32_t mode = -1;
     float R = 0, T = 0, pt = 0, thr = 0, index_cell_req = 0;
-    u64 n = 0, n_owned = 0;
-    int index_valid = 0, sorted_buf = 0, frame_done = 0, qorder_kind = 0, q_sorted_buf = 0;
+    u64 n = 0, n_owned = 0;  // n_owned: queries (the length of a query list)
+    int index_valid = 0, sorted_buf = 0, frame_done = 0, qorder_kind = 0, q_sorted_buf = 0, listed = 0, slot_pos = 0;
     const void *out = nullptr;
     bool operator==(const StepKey &o) const {
         return mode == o.mode && R == o.R && T == o.T && pt == o.pt && thr == o.thr && index_cell_req == o.index_cell_req &&
                n == o.n && n_owned == o.n_owned && index_valid == o.index_valid && sorted_buf == o.sorted_buf &&
-               frame_done == o.frame_done && qorder_kind == o.qorder_kind && q_sorted_buf == o.q_sorted_buf && out == o.out;
+               frame_done == o.frame_done && qorder_kind == o.qorder_kind && q_sorted_buf == o.q_sorted_buf &&
+               listed == o.listed && slot_pos == o.slot_pos && out == o.out;
     }
 };
 
@@ -206,6 +208,16 @@ struct rcd_handle_s {
     u32 cells_cap = 0;
     float cell_scale = 0.5f;    // grid cell edge (x, y) as a fraction of the query radius
     DevBuf<u32> qkeys[2], qvals[2];  // query order: Morton keys of the query volumes + permutation
+    // rcd_set_queries: the listed query set.  Made at the first call with a list (about 8 B per object).
+    DevBuf<u32> q_list;      // [cap] upload slots of the listed queries
+    DevBuf<u32> q_pos;       // [cap] upload slot -> position in cell order (IndexState::slot_pos)
+    DevBuf<u32> q_seen;      // [cap / 32 + 2] bitmap of the device-list check, then its error word
+    HostBuf<u32> q_host;     // [cap] pinned copy of a host list on its way to q_list
+    Event q_copied;          // q_host is free again
+    bool q_listed = false;
+    u64 q_n = 0;
+    // the objects a frame queries
+    u64 queried() const { return q_listed ? q_n : n_owned; }
 
     bool world_static = false;
     float wmin[3] = {}, wmax[3] = {};
@@ -437,6 +449,7 @@ int build_index(rcd_handle h, float cell_req) {
     if (h->idx.valid && h->idx.cell_req == cell_req) return RCD_OK;
     h->idx.valid = false;
     h->idx.qorder_kind = 0;
+    h->idx.slot_pos = false;
     RC_TRY(wait_upload(h));
     if (n == 0) {
         float z[3] = {0, 0, 0};
@@ -501,11 +514,13 @@ int build_index(rcd_handle h, float cell_req) {
 
 // Query order for the pair kernel (k_query_keys + the same onesweep passes): tiles of 32 queries whose
 // volumes overlap.  kind 1: balls about the objects; kind 2: capsules of the predict queries.
+// With a query list only the listed objects are keyed and sorted (k_query_keys_list): O(k) instead of O(n).
 int build_query_order(rcd_handle h, int kind) {
     const u32 n = (u32)h->n;
     if (h->idx.qorder_kind == kind || n == 0) return RCD_OK;
     const GridParams g = h->idx.grid;
-    const u32 tiles = (n + SORT_TILE - 1) / SORT_TILE;
+    const u32 nq = h->q_listed ? (u32)h->q_n : n;  // keys to sort
+    const u32 tiles = (nq + SORT_TILE - 1) / SORT_TILE;
     stage_begin(h, RCD_STAGE_QORDER);
     CUDA_TRY(h, cudaMemsetAsync(h->hist, 0, MAX_PASSES * RADIX * sizeof(u32), h->stream));
     CUDA_TRY(h, cudaMemsetAsync(h->tile_status, 0, (size_t)QKEY_PASSES * tiles * RADIX * sizeof(u32), h->stream));
@@ -524,13 +539,24 @@ int build_query_order(rcd_handle h, int kind) {
     q.bits_lo = std::min(bits_x, bits_y);
     q.x_longer = bits_x > bits_y ? 1 : 0;
     q.capsule = kind == 2 ? 1 : 0;
-    const int blocks = (int)std::min<u64>(((u64)n + KEYS_THREADS - 1) / KEYS_THREADS, 148 * 8);
-    k_query_keys<<<blocks, KEYS_THREADS, 0, h->stream>>>(h->P0, h->P1, h->P2, n, q, h->qkeys[0], h->hist);
+    const int blocks = (int)std::min<u64>(((u64)nq + KEYS_THREADS - 1) / KEYS_THREADS, 148 * 8);
+    if (h->q_listed) {
+        if (!h->idx.slot_pos) {  // once per index build
+            k_slot_pos<<<(n + 255) / 256, 256, 0, h->stream>>>(h->sorted_slot, n, h->q_pos);
+            KERNEL_CHECK(h);
+            h->idx.slot_pos = true;
+        }
+        k_query_keys_list<<<blocks, KEYS_THREADS, 0, h->stream>>>(h->P0, h->P1, h->P2, h->q_list, h->q_pos, nq, q,
+                                                                   h->qkeys[0], h->qvals[0], h->hist);
+    } else {
+        k_query_keys<<<blocks, KEYS_THREADS, 0, h->stream>>>(h->P0, h->P1, h->P2, n, q, h->qkeys[0], h->hist);
+    }
     KERNEL_CHECK(h);
     k_scan_hist<<<1, RADIX, 0, h->stream>>>(h->hist, QKEY_PASSES);
     KERNEL_CHECK(h);
     u32 *const keys[2] = {h->qkeys[0], h->qkeys[1]}, *const vals[2] = {h->qvals[0], h->qvals[1]};
-    const int cur = launch_onesweep(keys, vals, n, QKEY_PASSES, h->hist, h->tile_status, h->tile_counter, h->stream);
+    const int cur = launch_onesweep(keys, vals, nq, QKEY_PASSES, h->hist, h->tile_status, h->tile_counter, h->stream,
+                                    !h->q_listed);
     KERNEL_CHECK(h);
     stage_end(h, RCD_STAGE_QORDER);
     h->idx.q_sorted_buf = cur;
@@ -714,6 +740,7 @@ int rcd_upload(rcd_handle h, uint64_t n, const float *px, const float *py, const
     RC_TRY(upload_issued(h, on));
     h->n = n;
     h->n_owned = n;
+    h->q_listed = false;
     h->idx.valid = false;
     h->frame_done = false;
     return RCD_OK;
@@ -739,7 +766,74 @@ int rcd_set_owned(rcd_handle h, uint64_t n_owned) {
     if (!h) return RCD_EINVAL;
     if (n_owned > h->n) return fail(h, RCD_EINVAL, "rcd_set_owned: n_owned exceeds the object count");
     h->n_owned = n_owned;
+    h->q_listed = false;
     h->idx.valid = false;
+    h->frame_done = false;
+    return RCD_OK;
+}
+
+// the list, inverse-map, bitmap and staging buffers of rcd_set_queries (all or nothing)
+static int queries_ready(rcd_handle h) {
+    if (h->q_list) return RCD_OK;
+    DevBuf<u32> list, pos, seen;
+    HostBuf<u32> host;
+    Event copied;
+    CUDA_TRY(h, list.alloc(h->cap));
+    CUDA_TRY(h, pos.alloc(h->cap));
+    CUDA_TRY(h, seen.alloc(h->cap / 32 + 2));
+    CUDA_TRY(h, host.alloc(h->cap));
+    CUDA_TRY(h, copied.create());
+    h->q_list = std::move(list);
+    h->q_pos = std::move(pos);
+    h->q_seen = std::move(seen);
+    h->q_host = std::move(host);
+    h->q_copied = std::move(copied);
+    return RCD_OK;
+}
+
+int rcd_set_queries(rcd_handle h, uint64_t n, const uint32_t *slots, int32_t src) {
+    if (!h) return RCD_EINVAL;
+    if (!slots) {
+        if (h->q_listed) h->idx.qorder_kind = 0;
+        h->q_listed = false;
+        h->frame_done = false;
+        return RCD_OK;
+    }
+    const u64 owned = h->n_owned;
+    if (n > owned) return fail(h, RCD_EINVAL, "rcd_set_queries: more slots than owned objects");
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    RC_TRY(queries_ready(h));
+    if (n && src == RCD_SRC_DEVICE) {
+        const u64 words = (owned + 31) / 32;
+        u32 *const err = h->q_seen.get() + words;
+        CUDA_TRY(h, cudaMemsetAsync(h->q_seen, 0, (words + 1) * sizeof(u32), h->stream));
+        k_check_queries<<<(unsigned)std::min<u64>((n + 255) / 256, (u64)h->sms * 8), 256, 0, h->stream>>>(
+            slots, (u32)n, (u32)owned, h->q_seen, err);
+        KERNEL_CHECK(h);
+        u32 bad = 0;
+        CUDA_TRY(h, cudaMemcpyAsync(&bad, err, sizeof(u32), cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+        if (bad & 1u) return fail(h, RCD_EINVAL, "rcd_set_queries: a slot is not an owned object");
+        if (bad & 2u) return fail(h, RCD_EINVAL, "rcd_set_queries: a slot is listed twice");
+        CUDA_TRY(h, cudaMemcpyAsync(h->q_list, slots, (size_t)n * sizeof(u32), cudaMemcpyDeviceToDevice, h->stream));
+    } else if (n) {
+        std::vector<uint64_t> seen((size_t)((owned + 63) / 64), 0);
+        for (u64 t = 0; t < n; ++t) {
+            const u32 s = slots[t];
+            if (s >= owned) return fail(h, RCD_EINVAL, "rcd_set_queries: slot " + std::to_string(s) + " is not an owned object");
+            const uint64_t bit = 1ull << (s & 63u);
+            if (seen[s >> 6] & bit) return fail(h, RCD_EINVAL, "rcd_set_queries: slot " + std::to_string(s) + " is listed twice");
+            seen[s >> 6] |= bit;
+        }
+        // (the previous list's copy out of the pinned buffer has to be done before it is overwritten)
+        CUDA_TRY(h, cudaEventSynchronize(h->q_copied));
+        std::memcpy(h->q_host.get(), slots, (size_t)n * sizeof(u32));
+        CUDA_TRY(h, cudaMemcpyAsync(h->q_list, h->q_host, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream));
+        CUDA_TRY(h, cudaEventRecord(h->q_copied, h->stream));
+    }
+    h->q_listed = true;
+    h->q_n = n;
+    h->idx.qorder_kind = 0;  // the index stays; only the query order is rebuilt
     h->frame_done = false;
     return RCD_OK;
 }
@@ -772,17 +866,17 @@ static int step_impl(rcd_handle h, int32_t mode, float search_radius, float time
     const float cell_req = (mode == RCD_MODE_PREDICT) ? PREDICT_RADIUS : search_radius;
     RC_TRY(build_index(h, cell_req));
 
-    if (h->n && h->n_owned) {
+    if (h->n && h->queried()) {
         RC_TRY(build_query_order(h, mode == RCD_MODE_PREDICT ? 2 : 1));
     }
     stage_begin(h, RCD_STAGE_PAIRS);
     if (!append) CUDA_TRY(h, cudaMemsetAsync(h->fb().counters, 0, sizeof(Counters), h->stream));
     if (h->n) CUDA_TRY(h, cudaMemsetAsync(h->cand_count, 0, (size_t)h->n * sizeof(u32), h->stream));
     if (h->n && !append) CUDA_TRY(h, cudaMemsetAsync(h->fb().risk_count, 0, (size_t)h->n * sizeof(u32), h->stream));
-    if (h->n && h->n_owned) {
+    if (h->n && h->queried()) {
         PairParams P;
         P.n = (u32)h->n;
-        P.n_owned = (u32)h->n_owned;
+        P.n_owned = (u32)h->queried();
         P.g = h->idx.grid;
         P.P0 = h->P0; P.P1 = h->P1; P.P2 = h->P2;
         P.qorder = h->qvals[h->idx.q_sorted_buf];
@@ -809,7 +903,7 @@ static int step_impl(rcd_handle h, int32_t mode, float search_radius, float time
         P.counters = h->fb().counters;
         P.cand_count = h->cand_count;
         P.risk_count = h->fb().risk_count;
-        P.ntiles = (u32)((h->n_owned + TQ - 1) / TQ);
+        P.ntiles = (u32)((P.n_owned + TQ - 1) / TQ);
         P.tile_counter = h->pair_tile_counter;
         P.qa = h->qa; P.qa_fill = h->qa_fill; P.qa_blocks_cap = h->qa_blocks_cap;
         P.ovf = h->ovf; P.ovf_cap = h->ovf_cap;
@@ -878,7 +972,9 @@ static StepKey step_key(rcd_handle h, int32_t mode, float search_radius, float t
     StepKey key;
     key.mode = mode; key.R = search_radius; key.T = time_window;
     key.pt = h->cn_prediction_time; key.thr = h->cn_risk_threshold;
-    key.n = h->n; key.n_owned = h->n_owned;
+    key.n = h->n; key.n_owned = h->queried();
+    key.listed = h->q_listed ? 1 : 0;
+    key.slot_pos = (ix.valid && ix.slot_pos) ? 1 : 0;
     key.index_valid = ix.valid ? 1 : 0;
     key.index_cell_req = ix.valid ? ix.cell_req : 0.0f;
     key.sorted_buf = ix.valid ? ix.sorted_buf : 0;
@@ -895,7 +991,7 @@ static StepKey step_key(rcd_handle h, int32_t mode, float search_radius, float t
 int rcd_step(rcd_handle h, int32_t mode, float search_radius, float time_window) {
     if (!h) return RCD_EINVAL;
     const bool want = (h->flags & RCD_FLAG_GRAPH) && !(h->flags & RCD_FLAG_PROFILE) && h->world_static && !h->graph_broken &&
-                      h->n > 0 && h->n_owned > 0;
+                      h->n > 0 && h->queried() > 0;
     if (!want) return step_impl(h, mode, search_radius, time_window);
     const bool append = (mode & RCD_STEP_APPEND) != 0;
     const bool flip = !append && h->flip_pending;
@@ -999,6 +1095,7 @@ int rcd_truncate(rcd_handle h, uint64_t n) {
     if (n > h->n) return fail(h, RCD_EINVAL, "rcd_truncate: n exceeds the object count");
     h->n = n;
     h->n_owned = n;
+    h->q_listed = false;
     h->idx.valid = false;
     h->frame_done = false;
     return RCD_OK;
@@ -1030,7 +1127,7 @@ int rcd_counts(rcd_handle h, rcd_counts_t *out) {
     CUDA_TRY(h, cudaSetDevice(h->device));
     CUDA_TRY(h, cudaMemcpyAsync(h->counters_host, h->fb().counters, sizeof(Counters), cudaMemcpyDeviceToHost, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    fill_counts(h, *h->counters_host, h->n, h->n_owned, out);
+    fill_counts(h, *h->counters_host, h->n, h->queried(), out);
     return RCD_OK;
 }
 
@@ -1113,7 +1210,7 @@ static int delivery_issued(rcd_handle h, cudaStream_t on = nullptr) {  // the fr
     h->pend_dev = h->fb().out;
     h->pend_risk = h->fb().risk_count;
     h->pend_n = h->n;
-    h->pend_n_owned = h->n_owned;
+    h->pend_n_owned = h->queried();
     h->download_pending = true;
     h->flip_pending = true;
     return RCD_OK;

@@ -319,13 +319,14 @@ k_onesweep_pass(const u32 *__restrict__ keys_in, const u32 *__restrict__ vals_in
                                        s_warp_hist, s_digit_excl, s_global_base, s_scan, s_kv);
 }
 
-// all passes of one sort: (keys[0], identity) -> (keys[cur], vals[cur]); returns cur
+// all passes of one sort: (keys[0], identity) -> (keys[cur], vals[cur]); returns cur.
+// identity = false: the values start in vals[0].
 inline int launch_onesweep(u32 *const keys[2], u32 *const vals[2], u32 n, int passes, const u32 *hist, u32 *tile_status,
-                           u32 *tile_counter, cudaStream_t stream) {
+                           u32 *tile_counter, cudaStream_t stream, bool identity = true) {
     const u32 tiles = (n + SORT_TILE - 1) / SORT_TILE;
     int cur = 0;
     for (int p = 0; p < passes; ++p) {
-        if (p == 0)
+        if (p == 0 && identity)
             k_onesweep_pass<true><<<tiles, SORT_THREADS, 0, stream>>>(keys[0], nullptr, keys[1], vals[1], n, 0, hist, tile_status,
                                                                     tile_counter);
         else
@@ -477,6 +478,26 @@ struct QueryKeyParams {
     int capsule;           // 1: predict queries are keyed by the middle of their chord
 };
 
+// Morton key of the query volume of the object at cell position s (p0 = P0[s], p2 = P2[s]; P1[s] is read only for
+// capsules).  Shared by k_query_keys and k_query_keys_list, so a listed query lands in the same key as unlisted.
+__device__ __forceinline__ u32 query_key(const float4 &p0, const float4 &p2, const float4 *__restrict__ P1, u32 s,
+                                         const QueryKeyParams &q) {
+    float x = p0.x, y = p0.y;
+    const u32 pattern = meta_pattern(__float_as_uint(p2.w));
+    if (q.capsule && pattern != RCD_PAT_NO_HISTORY) {
+        const float4 p1 = P1[s];
+        const float fv = (pattern >= RCD_PAT_CONSTANT_VELOCITY) ? 4.75f : 0.0f;
+        const float fa = (pattern == RCD_PAT_ACCELERATING) ? 22.5625f : 0.0f;
+        const float mx = x + p1.x * fv + p2.x * fa, my = y + p1.y * fv + p2.y * fa;
+        if (fabsf(mx) < 1.0e30f && fabsf(my) < 1.0e30f) { x = mx; y = my; }
+    }
+    const u32 ix = (u32)fminf(fmaxf((x - q.ox) * q.inv_res_x, 0.0f), q.max_x);  // NaN -> 0
+    const u32 iy = (u32)fminf(fmaxf((y - q.oy) * q.inv_res_y, 0.0f), q.max_y);
+    const u32 lo_mask = (1u << q.bits_lo) - 1u;
+    return spread_bits_2d(ix & lo_mask) | (spread_bits_2d(iy & lo_mask) << 1) |
+           (((q.x_longer ? ix : iy) >> q.bits_lo) << (2 * q.bits_lo));
+}
+
 __global__ void __launch_bounds__(KEYS_THREADS)
 k_query_keys(const float4 *__restrict__ P0, const float4 *__restrict__ P1, const float4 *__restrict__ P2, u32 n,
              QueryKeyParams q, u32 *__restrict__ keys, u32 *__restrict__ hist) {
@@ -489,22 +510,7 @@ k_query_keys(const float4 *__restrict__ P0, const float4 *__restrict__ P1, const
         const float4 p2 = P2[s];
         const u32 meta = __float_as_uint(p2.w);
         u32 key = QKEY_NOT_QUERIED;
-        if (meta & META_OWNED) {
-            float x = p0.x, y = p0.y;
-            const u32 pattern = meta_pattern(meta);
-            if (q.capsule && pattern != RCD_PAT_NO_HISTORY) {
-                const float4 p1 = P1[s];
-                const float fv = (pattern >= RCD_PAT_CONSTANT_VELOCITY) ? 4.75f : 0.0f;
-                const float fa = (pattern == RCD_PAT_ACCELERATING) ? 22.5625f : 0.0f;
-                const float mx = x + p1.x * fv + p2.x * fa, my = y + p1.y * fv + p2.y * fa;
-                if (fabsf(mx) < 1.0e30f && fabsf(my) < 1.0e30f) { x = mx; y = my; }
-            }
-            const u32 ix = (u32)fminf(fmaxf((x - q.ox) * q.inv_res_x, 0.0f), q.max_x);  // NaN -> 0
-            const u32 iy = (u32)fminf(fmaxf((y - q.oy) * q.inv_res_y, 0.0f), q.max_y);
-            const u32 lo_mask = (1u << q.bits_lo) - 1u;
-            key = spread_bits_2d(ix & lo_mask) | (spread_bits_2d(iy & lo_mask) << 1) |
-                  (((q.x_longer ? ix : iy) >> q.bits_lo) << (2 * q.bits_lo));
-        }
+        if (meta & META_OWNED) key = query_key(p0, p2, P1, s, q);
         keys[s] = key;
 #pragma unroll
         for (int p = 0; p < QKEY_PASSES; ++p) atomicAdd(&s_hist[p][(key >> (p * RADIX_BITS)) & (RADIX - 1)], 1u);
@@ -513,6 +519,57 @@ k_query_keys(const float4 *__restrict__ P0, const float4 *__restrict__ P1, const
     for (int k = threadIdx.x; k < QKEY_PASSES * RADIX; k += KEYS_THREADS) {
         u32 c = (&s_hist[0][0])[k];
         if (c) atomicAdd(&hist[k], c);
+    }
+}
+
+// -------------------------------------------------------------------------------------------------
+// K6 for a listed query set (rcd_set_queries): keys of the k listed objects only, with their cell positions as
+// the values of the sort (every onesweep pass then reads them, none is the identity pass).  The list holds upload
+// slots; slot_pos (k_slot_pos, once per index build) turns them into cell positions.  Bytes: 8 k + 48 k read
+// (gathers) + 8 k written.
+// -------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(KEYS_THREADS)
+k_query_keys_list(const float4 *__restrict__ P0, const float4 *__restrict__ P1, const float4 *__restrict__ P2,
+                  const u32 *__restrict__ list, const u32 *__restrict__ slot_pos, u32 k, QueryKeyParams q,
+                  u32 *__restrict__ keys, u32 *__restrict__ vals, u32 *__restrict__ hist) {
+    __shared__ u32 s_hist[QKEY_PASSES][RADIX];
+    for (int t = threadIdx.x; t < QKEY_PASSES * RADIX; t += KEYS_THREADS) (&s_hist[0][0])[t] = 0;
+    __syncthreads();
+    const u32 stride = gridDim.x * KEYS_THREADS;
+    for (u32 t = blockIdx.x * KEYS_THREADS + threadIdx.x; t < k; t += stride) {
+        const u32 s = slot_pos[list[t]];
+        const u32 key = query_key(P0[s], P2[s], P1, s, q);
+        keys[t] = key;
+        vals[t] = s;
+#pragma unroll
+        for (int p = 0; p < QKEY_PASSES; ++p) atomicAdd(&s_hist[p][(key >> (p * RADIX_BITS)) & (RADIX - 1)], 1u);
+    }
+    __syncthreads();
+    for (int t = threadIdx.x; t < QKEY_PASSES * RADIX; t += KEYS_THREADS) {
+        u32 c = (&s_hist[0][0])[t];
+        if (c) atomicAdd(&hist[t], c);
+    }
+}
+
+// upload slot -> position in cell order: the inverse of sorted_slot (k_reorder)
+__global__ void __launch_bounds__(256)
+k_slot_pos(const u32 *__restrict__ sorted_slot, u32 n, u32 *__restrict__ slot_pos) {
+    const u32 s = blockIdx.x * 256 + threadIdx.x;
+    if (s < n) slot_pos[sorted_slot[s]] = s;
+}
+
+// Checks a query list in device memory: err |= 1 for a slot >= n_owned, |= 2 for a slot listed twice.
+// seen: a zeroed bitmap of n_owned bits.
+__global__ void __launch_bounds__(256)
+k_check_queries(const u32 *__restrict__ list, u32 k, u32 n_owned, u32 *__restrict__ seen, u32 *__restrict__ err) {
+    for (u32 t = blockIdx.x * 256 + threadIdx.x; t < k; t += gridDim.x * 256) {
+        const u32 s = list[t];
+        if (s >= n_owned) {
+            atomicOr(err, 1u);
+            continue;
+        }
+        const u32 bit = 1u << (s & 31u);
+        if (atomicOr(&seen[s >> 5], bit) & bit) atomicOr(err, 2u);
     }
 }
 

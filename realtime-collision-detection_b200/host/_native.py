@@ -30,7 +30,7 @@ HALO_RECORD_WORDS = 13
 # list and against the header itself)
 SYMBOLS = (
     "rcd_version", "rcd_last_error", "rcd_create", "rcd_destroy", "rcd_upload", "rcd_set_patterns",
-    "rcd_set_owned", "rcd_step", "rcd_build_index", "rcd_set_compute_node_params", "rcd_truncate", "rcd_invalidate", "rcd_counts", "rcd_download", "rcd_download_unsorted",
+    "rcd_set_owned", "rcd_set_queries", "rcd_step", "rcd_build_index", "rcd_set_compute_node_params", "rcd_truncate", "rcd_invalidate", "rcd_counts", "rcd_download", "rcd_download_unsorted",
     "rcd_download_candidate_counts", "rcd_query_radius", "rcd_classify_patterns", "rcd_halo_pack",
     "rcd_halo_pack_async", "rcd_halo_append", "rcd_history_configure", "rcd_history_append", "rcd_history_reset", "rcd_history_move",
     "rcd_history_classify", "rcd_stage_ms", "rcd_get_stream", "rcd_launch_count", "rcd_pair_tests", "rcd_sync",
@@ -125,6 +125,8 @@ def load() -> ctypes.CDLL:
     L.rcd_upload.argtypes = [vp, u64] + [vp] * 13 + [i32]
     L.rcd_set_patterns.argtypes = [vp, u64, vp, i32]
     L.rcd_set_owned.argtypes = [vp, u64]
+    if hasattr(L, "rcd_set_queries"):
+        L.rcd_set_queries.argtypes = [vp, u64, vp, i32]
     L.rcd_step.argtypes = [vp, i32, f32, f32]
     L.rcd_build_index.argtypes = [vp, f32]
     L.rcd_set_compute_node_params.argtypes = [vp, f32, f32]

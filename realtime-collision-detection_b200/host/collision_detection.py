@@ -95,6 +95,19 @@ def _risks_from_pairs(pairs: np.ndarray, ids: List[str], tag: Optional[str] = No
     return RiskList(pairs, ids, tag, time.time())
 
 
+def _rows_for(spatial_index: SpatialIndex, vehicle_ids, kind: str, frame) -> Dict[str, List[CollisionRisk]]:
+    """{id: risks} for the known ids among `vehicle_ids`, from frame(slots) = (pairs, starts, counts)."""
+    table = spatial_index._table
+    slots = sorted({table.slot_of[v] for v in vehicle_ids if v in table.slot_of})
+    if not slots:
+        return {}
+    sl = np.asarray(slots, np.uint32)
+    pairs, starts, _ = frame(sl)
+    tag = f"{kind}{spatial_index._frames.frames_run:x}"
+    return {table.ids[s]: _risks_from_pairs(pairs[starts[s]:starts[s + 1]], table.ids, f"{tag}-{s:x}")
+            for s in slots if starts[s + 1] > starts[s]}
+
+
 class CollisionDetector:
     def __init__(self, spatial_index: SpatialIndex):
         self.spatial_index = spatial_index
@@ -137,11 +150,11 @@ class CollisionDetector:
             risks.pop(vehicle_id, None)
 
     # -- queries --------------------------------------------------------------------------------
-    def _frame(self, search_radius: float, time_window: float):
+    def _frame(self, search_radius: float, time_window: float, slots: Optional[np.ndarray] = None):
         frames = self.spatial_index._frames
         t0 = time.perf_counter()
         ran_before = frames.frames_run
-        pairs, starts, counts = frames.run(N.MODE_DETECT, search_radius, time_window)
+        pairs, starts, counts = frames.run(N.MODE_DETECT, search_radius, time_window, slots=slots)
         if frames.frames_run != ran_before:  # a new frame was computed: fold its totals into the stats
             ms = (time.perf_counter() - t0) * 1e3
             n = max(1, self.spatial_index._table.n)
@@ -179,6 +192,14 @@ class CollisionDetector:
         for s in np.flatnonzero(np.diff(starts)):
             out[table.ids[int(s)]] = _risks_from_pairs(pairs[starts[s]:starts[s + 1]], table.ids, f"{tag}-{int(s):x}")
         return out
+
+    def detect_for(self, vehicle_ids, search_radius: float = 100.0, time_window: float = 10.0) -> Dict[str, List[CollisionRisk]]:
+        """Additive batch API: the risks of the listed vehicles only, keyed like ``detect_all`` (vehicles without a
+        risk are left out); unknown ids are skipped.  A whole frame memoised with the same parameters answers
+        without GPU work; otherwise one GPU frame queries just these vehicles (every vehicle stays a neighbour) --
+        the partitioned queries of CollisionDetectionSystem._process_shard (collision_system.py:423-459)."""
+        return _rows_for(self.spatial_index, vehicle_ids, "d",
+                         lambda slots: self._frame(search_radius, time_window, slots))
 
     def get_collision_risks(self, vehicle_id: str) -> List[CollisionRisk]:
         return list(self.collision_risks.get(vehicle_id, {}).values())
@@ -369,11 +390,11 @@ class CollisionPredictionModel:
             self._pattern_key = key
         return self._patterns
 
-    def _frame(self):
+    def _frame(self, slots: Optional[np.ndarray] = None):
         frames = self.collision_detector.spatial_index._frames
         if self._ordered:
-            return frames.run(N.MODE_PREDICT, 100.0, 10.0, prepare=self._classify_on_device)
-        return frames.run(N.MODE_PREDICT, 100.0, 10.0, flags=self.trajectory_patterns())
+            return frames.run(N.MODE_PREDICT, 100.0, 10.0, prepare=self._classify_on_device, slots=slots)
+        return frames.run(N.MODE_PREDICT, 100.0, 10.0, flags=self.trajectory_patterns(), slots=slots)
 
     def predict_collisions(self, vehicle_id: str) -> List[CollisionRisk]:
         det = self.collision_detector
@@ -401,6 +422,10 @@ class CollisionPredictionModel:
         for s in np.flatnonzero(np.diff(starts)):
             out[table.ids[int(s)]] = _risks_from_pairs(pairs[starts[s]:starts[s + 1]], table.ids, f"{tag}-{int(s):x}")
         return out
+
+    def predict_for(self, vehicle_ids) -> Dict[str, List[CollisionRisk]]:
+        """``predict_all`` for the listed vehicles only (see ``CollisionDetector.detect_for``)."""
+        return _rows_for(self.collision_detector.spatial_index, vehicle_ids, "p", self._frame)
 
     def get_stats(self) -> Dict[str, Any]:
         return {**self.stats, "trajectory_history_count": len(self.trajectory_history)}

@@ -127,6 +127,20 @@ class FrameEngine:
     def set_owned(self, n_owned: int) -> None:
         N.check(self._lib.rcd_set_owned(self._h, int(n_owned)), self._h)
 
+    def set_queries(self, slots: Optional[np.ndarray]) -> None:
+        """Query only the listed upload slots (each < n_owned, no repeats) in the following steps; every object
+        stays a neighbour.  None: back to every owned object.  The spatial index is kept (rcd_set_queries)."""
+        if slots is None:
+            N.check(self._lib.rcd_set_queries(self._h, 0, None, N.SRC_HOST), self._h)
+            return
+        s = _as(slots, np.uint32)
+        buf = s if s.shape[0] else np.zeros(1, np.uint32)  # (n = 0 still needs a non-NULL list)
+        N.check(self._lib.rcd_set_queries(self._h, int(s.shape[0]), _vp(buf), N.SRC_HOST), self._h)
+
+    def set_queries_device(self, n: int, ptr: int) -> None:
+        """Same, from n uint32 slots in device memory (checked on the device; synchronises)."""
+        N.check(self._lib.rcd_set_queries(self._h, int(n), ctypes.c_void_p(int(ptr)), N.SRC_DEVICE), self._h)
+
     def set_compute_node_params(self, prediction_time: float = 5.0, risk_threshold: float = 0.5) -> None:
         N.check(self._lib.rcd_set_compute_node_params(self._h, float(prediction_time), float(risk_threshold)), self._h)
 
@@ -141,7 +155,7 @@ class FrameEngine:
     # -- frames -----------------------------------------------------------------------------
     def step(self, mode: int, search_radius: float = 100.0, time_window: float = 10.0, append: bool = False,
              with_detect: bool = False) -> None:
-        """One frame for every owned object.  ``append``: keep the pairs / totals of the previous step of this
+        """One frame for every owned object (or the set_queries list).  ``append``: keep the pairs / totals of the previous step of this
         frame.  ``with_detect`` (predict mode): also run detect_collisions(search_radius, time_window) in the
         same pass -- the result of step(DETECT) + step(PREDICT, append=True) for one sweep over the data."""
         m = int(mode) | (N.STEP_APPEND if append else 0) | (N.STEP_WITH_DETECT if with_detect else 0)

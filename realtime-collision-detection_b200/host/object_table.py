@@ -150,18 +150,24 @@ class FrameCache:
             self._results.clear()
 
     def run(self, mode: int, radius: float = 100.0, window: float = 10.0, flags: Optional[np.ndarray] = None,
-            prepare=None):
+            prepare=None, slots: Optional[np.ndarray] = None):
         """(pairs sorted by slot i, CSR starts per slot, counts) of one frame, memoised until the
         objects change.  `prepare(cache)` runs after the objects are on the device and again whenever
-        the handle had to be replaced (it sets device-side flags)."""
+        the handle had to be replaced (it sets device-side flags).  `slots` (sorted, unique uint32):
+        only these objects need their rows -- a memoised whole frame answers, else one frame queries
+        just them (rcd_set_queries; its counts are the totals over the slots), memoised per set."""
         self.sync_objects(flags)
         if prepare is not None:
             prepare(self)
         key = (mode, float(radius), float(window))
         hit = self._results.get(key)
+        if hit is None and slots is not None:
+            key += (slots.tobytes(),)
+            hit = self._results.get(key)
         if hit is not None:
             return hit
         eng = self.engine
+        eng.set_queries(slots)
         eng.step(mode, radius, window)
         while True:
             counts = eng.counts()
@@ -178,6 +184,7 @@ class FrameCache:
             if prepare is not None:
                 prepare(self)
             eng = self.engine
+            eng.set_queries(slots)
             eng.step(mode, radius, window)
         pairs = eng.download()
         starts = np.searchsorted(pairs["i"], np.arange(self.table.n + 1, dtype=np.uint32), side="left")
