@@ -355,12 +355,21 @@ int rcd_ingest_rejected(rcd_ingest g, uint64_t *n);
 int rcd_ingest_id_name(rcd_ingest g, uint32_t slot, const char **name, uint32_t *len);
 int rcd_ingest_type_name(rcd_ingest g, uint32_t code, const char **name, uint32_t *len);
 int rcd_ingest_lookup(rcd_ingest g, const char *id, uint32_t len, uint32_t *slot); /* RCD_ESTATE if unknown */
+/* Forget the ids of the listed slots (vehicles retired with rcd_retire / rcd_retire_stale); the next new ids take the
+ * freed slots, lowest first, before any fresh slot.  The id limit (rcd_ingest_set_limit) then counts live ids;
+ * rcd_ingest_counts' n_ids stays "slots handed out" (the frame size to pass to rcd_apply_records).  *n_live = ids
+ * interned afterwards (may be NULL).  A free or out-of-range slot, or a repeat: RCD_EINVAL, nothing changes.  After a
+ * release, rcd_ingest_lookup of a released id gives RCD_ESTATE and rcd_ingest_id_name of a free slot RCD_EINVAL.
+ * Records decoded before a release must be applied before it. */
+int rcd_ingest_release(rcd_ingest g, uint64_t n, const uint32_t *slots, uint64_t *n_live);
 
 /* Apply n decoded records to the frame: state[slot] = record for every record, in seq order
  * (N x CollisionDetector.update_vehicle, collision_detection.py:74-85), and -- if the trajectory rings
  * are configured (rcd_history_configure) and append_history != 0 -- one ring sample per record
  * (N x update_trajectory, :553-570).  n_objects = frame size afterwards (>= every slot + 1, >= the
- * current size; objects without a record keep their state).  records: host or device memory (src). */
+ * current size; objects without a record keep their state).  records: host or device memory (src).
+ * The timestamp of each slot's newest record is kept for rcd_retire_stale (8 bytes of device memory per
+ * object, allocated at the first call).  A record for a retired slot brings it back as a fresh vehicle. */
 int rcd_apply_records(rcd_handle h, uint64_t n, const rcd_record *records, uint32_t max_seq,
                       uint64_t n_objects, int32_t append_history, int32_t src);
 
@@ -427,6 +436,39 @@ int rcd_alerts_download(rcd_handle h, rcd_alert_event *out, uint64_t cap, uint64
 int rcd_summary_begin(rcd_handle h, double now, int32_t report_refreshed);
 int rcd_summary_finish(rcd_handle h, rcd_alert_event *events, uint64_t cap, uint64_t *n_events, rcd_alert_stats *stats,
                        uint32_t *risk_counts, uint64_t n, rcd_counts_t *counts);
+/* ---- retiring departed vehicles ----------------------------------------------------------------------
+ * CollisionDetector.remove_vehicle / SpatialIndex.remove_vehicle (collision_detection.py:74-108,
+ * spatial_index.py:202-227) and compute_node.SpatialIndex.remove for the device-resident frame.  A retired slot:
+ *   - has no position (the all-bits-set ghost state of rcd_halo_pack_async), type 0, the default pattern
+ *     (RCD_PAT_ACCELERATING), an empty trajectory ring and no record time; its caller id stays;
+ *   - is nobody's neighbour and is never queried: it emits nothing and is counted nowhere -- its candidate and risk
+ *     counts are 0, it adds nothing to n_candidates / n_potential / n_pairs / n_high_risk / n_alerts, and it is never
+ *     a hit of rcd_query_radius;
+ *   - keeps its place in the frame: n_objects / n_owned still count slots, retired ones included; nothing is compacted.
+ * A later record for the slot (rcd_apply_records) brings it back as a fresh vehicle whose ring starts from 0.
+ * Equivalence: a step on a frame whose live slots are L -- any mode, with or without a query list (a listed retired
+ * slot emits nothing) or graph replay -- emits the same records (byte for byte after mapping upload index to slot)
+ * with the same totals, and takes the same number of pair tests (rcd_pair_tests), as the same step on a frame
+ * uploaded with only the vehicles of L, in slot order, with the same world bounds.
+ * Alerts: when rcd_alerts_configure was called, every alert whose i or j is the caller id of a retired slot is
+ * dropped and reported as an RCD_ALERT_EXPIRED event (n_expired / n_live follow), after an in-flight summary fold,
+ * like rcd_alerts_expire; a recycled slot never inherits the previous vehicle's alerts.  events / cap / stats are
+ * those of rcd_alerts_expire (NULL / 0 when alerts are not configured).
+ * Both calls end the frame (a following RCD_STEP_APPEND gets RCD_ESTATE), invalidate the spatial index, keep the
+ * query list of rcd_set_queries, and synchronise. */
+/* Retire the listed slots (host array; each < n_objects; repeats and already-retired slots are no-ops).  A slot out
+ * of range: RCD_EINVAL and nothing changes. */
+int rcd_retire(rcd_handle h, uint64_t n, const uint32_t *slots, rcd_alert_event *events, uint64_t cap,
+               rcd_alert_stats *stats);
+/* Retire every live slot whose newest applied record has now - timestamp > max_age (strict, the form of the alert
+ * expiry) and write those slots in ascending order to slots_out; *n_retired = how many.  More than slots_cap of them:
+ * RCD_ECAPACITY, nothing is retired, *n_retired = how many there are (the rcd_ingest_decode_json convention).  Slots
+ * with no record time (never written by a record, or retired) are never reported, so a second call at the same `now`
+ * retires nothing.  A frame whose slots were not all written by rcd_apply_records since the last rcd_upload /
+ * rcd_halo_append (an rcd_upload of 0 objects starts a record-built frame): RCD_ESTATE. */
+int rcd_retire_stale(rcd_handle h, double now, double max_age, uint32_t *slots_out, uint64_t slots_cap,
+                     uint64_t *n_retired, rcd_alert_event *events, uint64_t cap, rcd_alert_stats *stats);
+
 /* Spatial-slab support (SURVEY.md 8e): pack every owned object whose x lies within `halo` of
  * peer p's slab [slab_lo[p], slab_hi[p]) -- p != self -- into 52-byte records
  * (11 floats, meta u32 = type | pattern << 8, id u32), grouped by peer.  out_records is a DEVICE

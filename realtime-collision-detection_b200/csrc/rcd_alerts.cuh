@@ -12,7 +12,7 @@
 //   second DRAM access for the quarter of the 40-byte entries of the first layout that straddled a line -- is gone);
 //   then timestamp (float64 like time.time()), risk, ttc, distance.  The state word is read and written whole (an
 //   update never needs a fence).
-// Expiry rebuilds the table into its twin (no tombstones).
+// Expiry and the purge of retired vehicles rebuild the table into its twin (no tombstones).
 #pragma once
 #include <cstddef>
 #include "rcd_common.cuh"
@@ -214,11 +214,36 @@ k_alert_update(const rcd_pair *__restrict__ pairs, unsigned long long n_max, con
     }
 }
 
-// _cleanup_expired_alerts (:488-517): acknowledged or now - timestamp > max_age -> EXPIRED event;
-// everything else moves to the twin table.
+// _cleanup_expired_alerts (:488-517): acknowledged or now - timestamp > max_age
+struct AlertTooOld {
+    double now, max_age;
+    __device__ __forceinline__ bool operator()(const AlertEntry &a) const { return a.acked || __dsub_rn(now, a.ts) > max_age; }
+};
+
+// rcd_retire: i or j is the caller id of a retired slot.  ids: sorted, distinct (any u32 values: upload-built frames
+// carry the caller's ids); a binary search per entry, retire batches being small next to the table.
+struct AlertOfRetired {
+    const u32 *ids;
+    u32 n;
+    __device__ __forceinline__ bool has(u32 v) const {
+        u32 lo = 0, hi = n;
+        while (lo < hi) {
+            const u32 mid = (lo + hi) >> 1;
+            if (__ldg(ids + mid) < v) lo = mid + 1; else hi = mid;
+        }
+        return lo < n && __ldg(ids + lo) == v;
+    }
+    __device__ __forceinline__ bool operator()(const AlertEntry &a) const {
+        return has((u32)(a.key >> 32)) || has((u32)(a.key & 0xffffffffu));
+    }
+};
+
+// Rebuild the table into its twin (no tombstones): every entry `drop` selects -> EXPIRED event; everything else moves
+// to the twin table.  Drop = AlertTooOld: rcd_alerts_expire; AlertOfRetired: the purge of rcd_retire.
+template <typename Drop>
 __global__ void __launch_bounds__(ALERT_THREADS)
-k_alert_expire(const AlertEntry *__restrict__ src, unsigned long long cap, double now, double max_age, AlertEntry *dst,
-               rcd_alert_event *ev, unsigned long long ev_cap, AlertCounters *c) {
+k_alert_rebuild(const AlertEntry *__restrict__ src, unsigned long long cap, Drop drop, AlertEntry *dst,
+                rcd_alert_event *ev, unsigned long long ev_cap, AlertCounters *c) {
     const unsigned long long stride = (unsigned long long)gridDim.x * ALERT_THREADS;
     const unsigned long long rounds = (cap + stride - 1) / stride;
     u32 expired = 0, live = 0;
@@ -231,7 +256,7 @@ k_alert_expire(const AlertEntry *__restrict__ src, unsigned long long cap, doubl
         if (k < cap) {
             const AlertEntry a = src[k];
             if (a.key != ALERT_EMPTY) {
-                if (a.acked || __dsub_rn(now, a.ts) > max_age) {
+                if (drop(a)) {
                     e.i = (u32)(a.key >> 32); e.j = (u32)(a.key & 0xffffffffu); e.alert_id = a.alert_id;
                     e.risk = a.risk; e.ttc = a.ttc; e.distance = a.distance; e.priority = e.old_priority = a.priority; e.acknowledged = a.acked;
                     e.timestamp = a.ts;

@@ -252,6 +252,11 @@ struct rcd_handle_s {
     DevBuf<Sample64> traj;  // trajectory rings, [max_history][cap]
     DevBuf<u32> traj_count;
     u32 traj_len = 0;
+    // rcd_retire_stale: per slot, the timestamp of the newest applied record (no_record_time(): none).  Made at the
+    // first rcd_apply_records (8 B per object).  records_only: every slot of the frame came from rcd_apply_records
+    // (rcd_upload of a non-empty frame and rcd_halo_append clear it, rcd_upload of an empty one sets it).
+    DevBuf<double> last_seen;
+    bool records_only = true;
     u64 launches = 0;
     // CUDA-graph replay of rcd_step (RCD_FLAG_GRAPH)
     StepGraph graphs[4];
@@ -740,6 +745,7 @@ int rcd_upload(rcd_handle h, uint64_t n, const float *px, const float *py, const
     RC_TRY(upload_issued(h, on));
     h->n = n;
     h->n_owned = n;
+    h->records_only = n == 0;
     h->q_listed = false;
     h->idx.valid = false;
     h->frame_done = false;
@@ -1483,13 +1489,20 @@ int rcd_apply_records(rcd_handle h, uint64_t n, const rcd_record *records, uint3
         RC_TRY(history_ready(h));
     }
     const bool hist = append_history && h->traj.get();
+    if (!h->last_seen) {
+        DevBuf<double> ls;
+        CUDA_TRY(h, ls.alloc(h->cap));
+        CUDA_TRY(h, cudaMemsetAsync(ls, 0xff, (size_t)h->cap * sizeof(double), h->stream));  // no record time
+        h->last_seen = std::move(ls);
+    }
     RC_TRY(wait_upload(h));
     reset_stages(h, -1);
     h->stage_mode = 0;
     stage_begin(h, RCD_STAGE_UPLOAD);
     if (n_objects > h->n) {
         const u32 fresh = (u32)(n_objects - h->n);
-        k_init_slots<<<(fresh + 255) / 256, 256, 0, h->stream>>>((u32)h->n, (u32)n_objects, h->in_id, h->in_pattern);
+        k_init_slots<<<(fresh + 255) / 256, 256, 0, h->stream>>>((u32)h->n, (u32)n_objects, h->in_id, h->in_pattern,
+                                                                 h->last_seen);
         KERNEL_CHECK(h);
     }
     const unsigned long long *dev = reinterpret_cast<const unsigned long long *>(records);
@@ -1502,7 +1515,8 @@ int rcd_apply_records(rcd_handle h, uint64_t n, const rcd_record *records, uint3
     const MutableState st = mutable_state(h);
     for (u32 seq = 0; n && seq <= max_seq; ++seq) {
         k_apply_records<<<(unsigned)((n + APPLY_THREADS - 1) / APPLY_THREADS), APPLY_THREADS, 0, h->stream>>>(
-            (u32)n, dev, seq, (u32)n_objects, st, hist ? h->traj.get() : nullptr, h->traj_count, (u32)h->cap, h->traj_len);
+            (u32)n, dev, seq, (u32)n_objects, st, hist ? h->traj.get() : nullptr, h->traj_count, (u32)h->cap, h->traj_len,
+            h->last_seen);
         KERNEL_CHECK(h);
     }
     stage_end(h, RCD_STAGE_UPLOAD);
@@ -1668,8 +1682,8 @@ int rcd_alerts_expire(rcd_handle h, double now, double max_age, rcd_alert_event 
         AlertEntry *src = h->alert_tab[h->alert_cur], *dst = h->alert_tab[h->alert_cur ^ 1];
         CUDA_TRY(h, cudaMemsetAsync(dst, 0xff, (size_t)h->alert_cap * sizeof(AlertEntry), h->stream));
         const unsigned blocks = (unsigned)std::min<u64>((h->alert_cap + ALERT_THREADS - 1) / ALERT_THREADS, (u64)h->sms * 8);
-        k_alert_expire<<<blocks, ALERT_THREADS, 0, h->stream>>>(src, h->alert_cap, now, max_age, dst, h->alert_ev, h->alert_ev_cap,
-                                                                h->alert_counters);
+        k_alert_rebuild<<<blocks, ALERT_THREADS, 0, h->stream>>>(src, h->alert_cap, AlertTooOld{now, max_age}, dst, h->alert_ev,
+                                                                 h->alert_ev_cap, h->alert_counters);
         KERNEL_CHECK(h);
         return RCD_OK;
     });
@@ -1717,6 +1731,107 @@ int rcd_alerts_download(rcd_handle h, rcd_alert_event *out, uint64_t cap, uint64
     const u64 n = std::min<u64>(std::min<u64>(st.n_events, h->alert_ev_cap), cap);
     std::sort(out, out + n, [](const rcd_alert_event &a, const rcd_alert_event &b) { return a.i != b.i ? a.i < b.i : a.j < b.j; });
     *n_out = n;
+    return RCD_OK;
+}
+
+// ---- retirement (rcd_retire, rcd_retire_stale) -------------------------------------------------------------
+// Retire the n slots of the device list d_slots (checked: each < h->n); d_ids has room for n caller ids.  Both entry
+// points end the frame and invalidate the index; the query list stays (a listed retired slot emits nothing).
+static int retire_slots(rcd_handle h, u64 n, const u32 *d_slots, u32 *d_ids, rcd_alert_event *events, uint64_t cap,
+                        rcd_alert_stats *stats) {
+    if (stats) *stats = rcd_alert_stats{};
+    h->idx.valid = false;
+    h->frame_done = false;
+    if (n) {
+        RC_TRY(wait_upload(h));
+        k_retire_slots<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(d_slots, (u32)n, mutable_state(h),
+                                                                           h->traj_count.get(), h->last_seen.get(), d_ids);
+        KERNEL_CHECK(h);
+        RC_TRY(release_inputs(h));
+    }
+    if (!h->alert_cap) return RCD_OK;
+    // the purge: every alert of a retired caller id, after an in-flight summary fold (like rcd_alerts_expire)
+    RC_TRY(alerts_join(h));
+    std::vector<u32> ids((size_t)n);
+    if (n) CUDA_TRY(h, cudaMemcpyAsync(ids.data(), d_ids, (size_t)n * sizeof(u32), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaMemcpyAsync(h->alert_counters_host, h->alert_counters, sizeof(AlertCounters), cudaMemcpyDeviceToHost,
+                                h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    const u64 live = h->alert_counters_host->n_live;
+    std::sort(ids.begin(), ids.end());
+    ids.erase(std::unique(ids.begin(), ids.end()), ids.end());
+    if (ids.empty() || live == 0) {  // nothing can match: no rebuild
+        if (stats) stats->n_live = live;
+        return RCD_OK;
+    }
+    CUDA_TRY(h, cudaMemcpyAsync(d_ids, ids.data(), ids.size() * sizeof(u32), cudaMemcpyHostToDevice, h->stream));
+    const int rc = alerts_call(h, events, cap, stats, true, [&]() -> int {
+        AlertEntry *src = h->alert_tab[h->alert_cur], *dst = h->alert_tab[h->alert_cur ^ 1];
+        CUDA_TRY(h, cudaMemsetAsync(dst, 0xff, (size_t)h->alert_cap * sizeof(AlertEntry), h->stream));
+        const unsigned blocks = (unsigned)std::min<u64>((h->alert_cap + ALERT_THREADS - 1) / ALERT_THREADS, (u64)h->sms * 8);
+        k_alert_rebuild<<<blocks, ALERT_THREADS, 0, h->stream>>>(src, h->alert_cap, AlertOfRetired{d_ids, (u32)ids.size()}, dst,
+                                                                 h->alert_ev, h->alert_ev_cap, h->alert_counters);
+        KERNEL_CHECK(h);
+        return RCD_OK;
+    });
+    if (rc == RCD_OK) h->alert_cur ^= 1;
+    return rc;
+}
+
+int rcd_retire(rcd_handle h, uint64_t n, const uint32_t *slots, rcd_alert_event *events, uint64_t cap, rcd_alert_stats *stats) {
+    if (!h || (n && !slots) || (cap && !events)) return RCD_EINVAL;
+    for (u64 k = 0; k < n; ++k)
+        if (slots[k] >= h->n) return fail(h, RCD_EINVAL, "rcd_retire: slot " + std::to_string(slots[k]) + " is not in the frame");
+    if (n > 0xffffffffull) return fail(h, RCD_ECAPACITY, "rcd_retire: too many slots");
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    DevBuf<u32> d;  // [n] slots, [n] caller ids
+    if (n) {
+        CUDA_TRY(h, d.alloc(2 * (size_t)n));
+        CUDA_TRY(h, cudaMemcpyAsync(d, slots, (size_t)n * sizeof(u32), cudaMemcpyHostToDevice, h->stream));
+    }
+    RC_TRY(retire_slots(h, n, d, d.get() + n, events, cap, stats));
+    if (n) CUDA_TRY(h, cudaStreamSynchronize(h->stream));  // d is freed on return
+    return RCD_OK;
+}
+
+int rcd_retire_stale(rcd_handle h, double now, double max_age, uint32_t *slots_out, uint64_t slots_cap, uint64_t *n_retired,
+                     rcd_alert_event *events, uint64_t cap, rcd_alert_stats *stats) {
+    if (!h || !n_retired || (slots_cap && !slots_out) || (cap && !events)) return RCD_EINVAL;
+    if (!h->records_only)
+        return fail(h, RCD_ESTATE, "rcd_retire_stale: the frame has objects that rcd_apply_records did not write (rcd_upload / "
+                                   "rcd_halo_append): they have no record time");
+    *n_retired = 0;
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    const u32 n = (u32)h->n;
+    u64 total = 0;
+    DevBuf<u32> tiles_buf, d;
+    if (n && h->last_seen) {
+        RC_TRY(wait_upload(h));
+        const u32 tiles = (n + STALE_TILE - 1) / STALE_TILE;
+        CUDA_TRY(h, tiles_buf.alloc((size_t)tiles + 1));
+        k_stale_count<<<tiles, STALE_THREADS, 0, h->stream>>>(h->last_seen, n, now, max_age, tiles_buf);
+        KERNEL_CHECK(h);
+        k_scan_tiles<<<1, 1024, 0, h->stream>>>(tiles_buf, tiles);
+        KERNEL_CHECK(h);
+        u32 count = 0;
+        CUDA_TRY(h, cudaMemcpyAsync(&count, tiles_buf.get() + tiles, sizeof(u32), cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+        total = count;
+        *n_retired = total;
+        if (total > slots_cap) {
+            if (stats) *stats = rcd_alert_stats{};
+            return fail(h, RCD_ECAPACITY, "rcd_retire_stale: " + std::to_string(total) + " stale slots, room for " +
+                                              std::to_string(slots_cap));
+        }
+        if (total) {
+            CUDA_TRY(h, d.alloc(2 * (size_t)total));  // [total] slots, ascending, [total] caller ids
+            k_stale_scatter<<<tiles, STALE_THREADS, 0, h->stream>>>(h->last_seen, n, now, max_age, tiles_buf, d);
+            KERNEL_CHECK(h);
+            CUDA_TRY(h, cudaMemcpyAsync(slots_out, d, (size_t)total * sizeof(u32), cudaMemcpyDeviceToHost, h->stream));
+        }
+    }
+    RC_TRY(retire_slots(h, total, d, d.get() + total, events, cap, stats));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));  // slots_out is complete; the scratch buffers are freed on return
     return RCD_OK;
 }
 
@@ -1799,6 +1914,7 @@ int rcd_halo_append(rcd_handle h, const void *records, uint64_t n_records) {
     KERNEL_CHECK(h);
     RC_TRY(release_inputs(h));
     h->n += n_records;
+    h->records_only = false;
     h->idx.valid = false;
     h->frame_done = false;
     return RCD_OK;

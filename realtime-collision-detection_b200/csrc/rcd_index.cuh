@@ -454,10 +454,11 @@ k_cell_table(const u32 *__restrict__ keys, u32 n, u32 ncells, u32 *__restrict__ 
 // code of the centre of their volume -- the object itself for radius queries, the middle of the chord
 // of the predicted centre path (collision_detection.py:728-741) for predict queries -- and sorted;
 // consecutive 32 objects are then a compact tile at any density.  Halo copies (not queried) get the
-// top key and end up behind the last tile.  Bytes: 48 N read + 4 N written, then the sort passes.
+// top key and end up behind the last tile.  Owned objects without a position come just before them.  Bytes: 48 N read + 4 N written, then the sort passes.
 // -------------------------------------------------------------------------------------------------
 constexpr int QKEY_BITS = 23;                       // both axes together, split so that the key lattice is (nearly) square
-constexpr u32 QKEY_NOT_QUERIED = 1u << QKEY_BITS;   // bit 23: sorts behind every query
+constexpr u32 QKEY_NO_POSITION = 1u << QKEY_BITS;   // an owned object without a position (retired): behind every live query
+constexpr u32 QKEY_NOT_QUERIED = QKEY_NO_POSITION + 1u;  // halo copies: behind everything
 constexpr int QKEY_PASSES = 3;                      // 24 bits
 
 __device__ __forceinline__ u32 spread_bits_2d(u32 v) {  // 16 bits -> every other bit
@@ -480,8 +481,12 @@ struct QueryKeyParams {
 
 // Morton key of the query volume of the object at cell position s (p0 = P0[s], p2 = P2[s]; P1[s] is read only for
 // capsules).  Shared by k_query_keys and k_query_keys_list, so a listed query lands in the same key as unlisted.
+// An object without a position (a retired slot, rcd_retire) gets QKEY_NO_POSITION: such queries form the trailing
+// tiles of the query order, which k_tile_plan leaves empty, and the live queries are tiled exactly as in a frame
+// without them (the sort is stable and their cell positions come first).
 __device__ __forceinline__ u32 query_key(const float4 &p0, const float4 &p2, const float4 *__restrict__ P1, u32 s,
                                          const QueryKeyParams &q) {
+    if (p0.x != p0.x) return QKEY_NO_POSITION;
     float x = p0.x, y = p0.y;
     const u32 pattern = meta_pattern(__float_as_uint(p2.w));
     if (q.capsule && pattern != RCD_PAT_NO_HISTORY) {

@@ -9,7 +9,8 @@
 // rcd_apply_records scatters into the device-resident frame state and trajectory rings:
 //   - numbers are converted with std::from_chars (correctly rounded, like Python's float()); NaN / Infinity /
 //     -Infinity are accepted like json.loads does;
-//   - id and type strings are unescaped to UTF-8 and interned: id -> dense slot (first seen first),
+//   - id and type strings are unescaped to UTF-8 and interned: id -> dense slot (first seen first; slots freed by
+//     rcd_ingest_release are handed out again, lowest first, before any fresh slot),
 //     type -> small code (only equality of types is ever used, collision_detection.py:498-513);
 //   - a message that is not valid JSON, or lacks one of the fields the reference reads, is skipped and
 //     counted (the reference logs and drops it, warning_system.py:677-678);
@@ -21,6 +22,8 @@
 #include <cstdint>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
+#include <queue>
 #include <string>
 #include <thread>
 #include <unordered_map>
@@ -281,11 +284,14 @@ struct Ingest {
     std::vector<std::string> id_names, type_names;
     std::vector<uint32_t> batch_stamp;  // per slot: batch number of the last message
     std::vector<uint8_t> batch_seq;     // per slot: messages seen in that batch
+    std::vector<uint8_t> slot_free;     // per slot: released, no id (rcd_ingest_release)
+    std::priority_queue<uint32_t, std::vector<uint32_t>, std::greater<uint32_t>> free_slots;  // lowest first
     uint32_t batch = 0;
-    uint64_t max_ids = ~0ull;           // new ids beyond this are rejected (rcd_ingest_set_limit)
+    uint64_t max_ids = ~0ull;           // live ids beyond this are rejected (rcd_ingest_set_limit)
     uint64_t n_rejected = 0;            // messages dropped since creation: unknown id with the table full,
                                         // or more than 255 messages of one vehicle in one call
     std::string err;
+    uint64_t n_live() const { return id_names.size() - free_slots.size(); }
 };
 constexpr uint32_t TYPE_CODE_OTHER = 255;  // every type string beyond the first 255 distinct ones
 
@@ -355,16 +361,26 @@ int rcd_ingest_decode_json(rcd_ingest g, const char *buf, uint64_t len, int32_t 
                 auto it = g->ids.find(m.id);
                 uint32_t slot;
                 if (it == g->ids.end()) {
-                    if (g->id_names.size() >= g->max_ids) {  // table full: known vehicles keep being served
+                    if (g->n_live() >= g->max_ids) {  // table full: known vehicles keep being served
                         ++n_bad;
                         ++g->n_rejected;
                         continue;
                     }
-                    slot = (uint32_t)g->id_names.size();
+                    if (!g->free_slots.empty()) {  // a released slot, lowest first
+                        slot = g->free_slots.top();
+                        g->free_slots.pop();
+                        g->slot_free[slot] = 0;
+                        g->id_names[slot] = m.id;
+                        g->batch_stamp[slot] = 0;
+                        g->batch_seq[slot] = 0;
+                    } else {
+                        slot = (uint32_t)g->id_names.size();
+                        g->id_names.push_back(m.id);
+                        g->batch_stamp.push_back(0);
+                        g->batch_seq.push_back(0);
+                        g->slot_free.push_back(0);
+                    }
                     g->ids.emplace(m.id, slot);
-                    g->id_names.push_back(m.id);
-                    g->batch_stamp.push_back(0);
-                    g->batch_seq.push_back(0);
                 } else slot = it->second;
                 auto tt = g->types.find(m.type);
                 uint32_t code;
@@ -433,7 +449,7 @@ int rcd_ingest_counts(rcd_ingest g, uint64_t *n_ids, uint64_t *n_types) {
     return RCD_OK;
 }
 int rcd_ingest_id_name(rcd_ingest g, uint32_t slot, const char **name, uint32_t *len) {
-    if (!g || !name || !len || slot >= g->id_names.size()) return RCD_EINVAL;
+    if (!g || !name || !len || slot >= g->id_names.size() || g->slot_free[slot]) return RCD_EINVAL;
     *name = g->id_names[slot].data();
     *len = (uint32_t)g->id_names[slot].size();
     return RCD_OK;
@@ -455,6 +471,33 @@ int rcd_ingest_lookup(rcd_ingest g, const char *id, uint32_t len, uint32_t *slot
     auto it = g->ids.find(std::string(id, len));
     if (it == g->ids.end()) return RCD_ESTATE;
     *slot = it->second;
+    return RCD_OK;
+}
+
+int rcd_ingest_release(rcd_ingest g, uint64_t n, const uint32_t *slots, uint64_t *n_live) {
+    if (!g || (n && !slots)) return RCD_EINVAL;
+    try {
+        // every slot is checked before anything changes
+        std::vector<uint8_t> seen(n ? g->id_names.size() : 0, 0);
+        for (uint64_t k = 0; k < n; ++k) {
+            const uint32_t s = slots[k];
+            if (s >= g->id_names.size()) { g->err = "rcd_ingest_release: slot " + std::to_string(s) + " was never handed out"; return RCD_EINVAL; }
+            if (g->slot_free[s]) { g->err = "rcd_ingest_release: slot " + std::to_string(s) + " is free"; return RCD_EINVAL; }
+            if (seen[s]) { g->err = "rcd_ingest_release: slot " + std::to_string(s) + " is listed twice"; return RCD_EINVAL; }
+            seen[s] = 1;
+        }
+        for (uint64_t k = 0; k < n; ++k) {
+            const uint32_t s = slots[k];
+            g->ids.erase(g->id_names[s]);
+            std::string().swap(g->id_names[s]);
+            g->slot_free[s] = 1;
+            g->free_slots.push(s);
+        }
+    } catch (const std::bad_alloc &) {
+        g->err = "out of host memory";
+        return RCD_ENOMEM;
+    }
+    if (n_live) *n_live = g->n_live();
     return RCD_OK;
 }
 

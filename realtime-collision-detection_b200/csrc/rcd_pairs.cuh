@@ -836,13 +836,23 @@ __global__ void __launch_bounds__(128) k_tile_plan(PairParams P) {
     const u32 nwarps = gridDim.x * (blockDim.x >> 5);
     for (u32 tile = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); tile < P.ntiles; tile += nwarps) {
         const u32 qi = tile * TQ + lane;
-        const bool valid = qi < P.n_owned;
         float4 p0 = make_float4(0.f, 0.f, 0.f, 0.f), p1 = p0, p2 = p0;
-        if (valid) {
+        if (qi < P.n_owned) {
             const u32 s = P.qorder[qi];
             p0 = P.P0[s];
             p1 = P.P1[s];
             p2 = P.P2[s];
+        }
+        // a query without a position (retired slot, NaN) is a lane past the queries: it widens no box.  A tile of them
+        // only (the trailing tiles of the query order, query_key) gets an empty box -- no rows, no work items; the
+        // clamped box of "no lane" would be inverted, {nx-1..0, ny-1..0, nz-1..0}, with (2-ny)(2-nz) rows
+        const bool valid = qi < P.n_owned && p0.x == p0.x;
+        if (!__any_sync(FULL_MASK, valid)) {
+            if (lane == 0) {
+                P.tile_box[2 * (size_t)tile] = make_int4(1, 0, 1, 0);
+                P.tile_box[2 * (size_t)tile + 1] = make_int4(1, 0, 0, 0);
+            }
+            continue;
         }
         const QueryVolume v = query_volume<MODE>(p1, p2, meta_pattern(__float_as_uint(p2.w)), Rq);
         // cells of the bounding box of the tile's query volumes (cell_coord is monotone, so a

@@ -38,7 +38,7 @@ SYMBOLS = (
     "rcd_ingest_counts", "rcd_ingest_set_limit", "rcd_ingest_rejected", "rcd_ingest_id_name", "rcd_ingest_type_name", "rcd_ingest_lookup", "rcd_apply_records",
     "rcd_alerts_configure", "rcd_alerts_update", "rcd_alerts_update_pairs", "rcd_alerts_expire",
     "rcd_alerts_acknowledge", "rcd_alerts_download", "rcd_download_begin", "rcd_download_finish", "rcd_graph_replays", "rcd_pair_exact", "rcd_risk_assessment", "rcd_download_begin_compact", "rcd_summary_begin", "rcd_summary_finish",
-    "rcd_download_risk_counts",
+    "rcd_download_risk_counts", "rcd_retire", "rcd_retire_stale", "rcd_ingest_release",
 )
 
 
@@ -181,6 +181,7 @@ def load() -> ctypes.CDLL:
     L.rcd_ingest_type_name.argtypes = [vp, u32, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(u32)]
     L.rcd_ingest_lookup.argtypes = [vp, ctypes.c_char_p, u32, ctypes.POINTER(u32)]
     L.rcd_apply_records.argtypes = [vp, u64, vp, u32, u64, i32, i32]
+    L.rcd_ingest_release.argtypes = [vp, u64, vp, ctypes.POINTER(u64)]
     f64 = ctypes.c_double
     L.rcd_alerts_configure.argtypes = [vp, u64]
     L.rcd_alerts_update.argtypes = [vp, f64, i32, vp, u64, ctypes.POINTER(RcdAlertStats)]
@@ -188,6 +189,8 @@ def load() -> ctypes.CDLL:
     L.rcd_alerts_expire.argtypes = [vp, f64, f64, vp, u64, ctypes.POINTER(RcdAlertStats)]
     L.rcd_alerts_acknowledge.argtypes = [vp, u64, vp, vp, ctypes.POINTER(u64)]
     L.rcd_alerts_download.argtypes = [vp, vp, u64, ctypes.POINTER(u64)]
+    L.rcd_retire.argtypes = [vp, u64, vp, vp, u64, ctypes.POINTER(RcdAlertStats)]
+    L.rcd_retire_stale.argtypes = [vp, f64, f64, vp, u64, ctypes.POINTER(u64), vp, u64, ctypes.POINTER(RcdAlertStats)]
     for name in SYMBOLS:
         if not hasattr(L, name) and os.environ.get("RCD_B200_LIB"):
             continue  # an older build loaded for an A/B kernel experiment

@@ -152,6 +152,28 @@ class FrameEngine:
     def invalidate(self) -> None:
         N.check(self._lib.rcd_invalidate(self._h), self._h)
 
+    # -- retiring departed vehicles (rcd_retire, rcd_retire_stale) -------------------------------------
+    def _retire_events(self) -> np.ndarray:
+        return self._alert_events(None) if getattr(self, "_alert_cap", 0) else np.zeros(0, N.ALERT_EVENT_DTYPE)
+
+    def retire(self, slots) -> Tuple[np.ndarray, np.ndarray, Dict[str, int]]:
+        """remove_vehicle for the listed slots: they keep their place in the frame but have no position, are nobody's
+        neighbour and emit nothing; their alerts are dropped.  Returns (slots, EXPIRED events, alert stats)."""
+        s = _as(slots, np.uint32)
+        ev, st = self._retire_events(), N.RcdAlertStats()
+        N.check(self._lib.rcd_retire(self._h, int(s.shape[0]), _vp(s) if s.shape[0] else None, _vp(ev) if ev.shape[0] else None,
+                                     ev.shape[0], ctypes.byref(st)), self._h)
+        return s, ev[: min(int(st.n_events), ev.shape[0])], self._alert_stats(st)
+
+    def retire_stale(self, now: float, max_age: float) -> Tuple[np.ndarray, np.ndarray, Dict[str, int]]:
+        """Retire every slot whose newest applied record is older than max_age at `now` (now - t > max_age).
+        Returns (retired slots ascending, EXPIRED events, alert stats).  Record-built frames only."""
+        ev, st, n = self._retire_events(), N.RcdAlertStats(), ctypes.c_uint64(0)
+        out = np.empty(max(1, self.n), np.uint32)  # (written up to n_retired)
+        N.check(self._lib.rcd_retire_stale(self._h, float(now), float(max_age), _vp(out), out.shape[0], ctypes.byref(n),
+                                           _vp(ev) if ev.shape[0] else None, ev.shape[0], ctypes.byref(st)), self._h)
+        return out[: int(n.value)], ev[: min(int(st.n_events), ev.shape[0])], self._alert_stats(st)
+
     # -- frames -----------------------------------------------------------------------------
     def step(self, mode: int, search_radius: float = 100.0, time_window: float = 10.0, append: bool = False,
              with_detect: bool = False) -> None:

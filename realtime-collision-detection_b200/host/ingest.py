@@ -20,7 +20,8 @@ from . import _native as N
 
 
 class VehicleIngest:
-    """Decoder + id table.  Slot ``k`` of the frame is the k-th distinct vehicle id ever seen."""
+    """Decoder + id table.  A new vehicle id takes the lowest released slot (``release``), else the next fresh one:
+    without releases, slot ``k`` of the frame is the k-th distinct vehicle id ever seen."""
 
     def __init__(self, threads: int = 0):
         self._lib = N.load()
@@ -84,6 +85,15 @@ class VehicleIngest:
         """At most ``max_ids`` distinct vehicles: messages of further (unknown) vehicles are dropped and counted
         (``bad_messages``, ``rejected``) while the known ones keep being served."""
         self._check(self._lib.rcd_ingest_set_limit(self._g, int(max_ids)))
+
+    def release(self, slots) -> int:
+        """Forget the ids of the listed slots (retired vehicles): new ids take them, lowest first, and the id limit
+        counts live ids.  ``n_objects`` (slots handed out) does not change.  Returns the number of live ids."""
+        s = np.ascontiguousarray(slots, dtype=np.uint32)
+        live = ctypes.c_uint64()
+        self._check(self._lib.rcd_ingest_release(self._g, int(s.shape[0]), s.ctypes.data_as(ctypes.c_void_p) if s.shape[0]
+                                                 else None, ctypes.byref(live)))
+        return int(live.value)
 
     @property
     def rejected(self) -> int:
@@ -158,6 +168,29 @@ class VehiclePositionStream:
             self.engine.apply_records(rec, self.ingest.n_objects, max_seq, history=True)
             self.messages_applied += len(rec)
         return len(rec)
+
+    def _retired(self, slots: np.ndarray, events: np.ndarray, alerts) -> List[str]:
+        # the alert manager drops the events while id_of still names the departed vehicles; then the slots are freed
+        ids = [self.ingest.id_of(int(k)) for k in slots]
+        if alerts is not None:
+            alerts.retire_vehicles(events, ids)
+        if len(slots):
+            self.ingest.release(slots)
+        return ids
+
+    def remove_vehicles(self, ids, alerts=None) -> List[str]:
+        """``remove_vehicle`` for the listed vehicle ids (unknown ids are skipped): their slots stop taking part in
+        frames and are handed to the next new vehicles.  ``alerts``: the ``AlertManager`` attached to this engine,
+        whose alerts of the departed vehicles are dropped too.  Returns the ids that were removed."""
+        slots = sorted({s for s in (self.ingest.slot_of(v) for v in ids) if s is not None})
+        _, ev, _ = self.engine.retire(np.asarray(slots, np.uint32))
+        return self._retired(np.asarray(slots, np.uint32), ev, alerts)
+
+    def retire_stale(self, now: float, max_age: float, alerts=None) -> List[str]:
+        """Remove every vehicle whose newest message is older than ``max_age`` at ``now`` (now - timestamp >
+        max_age); returns their ids in slot order."""
+        slots, ev, _ = self.engine.retire_stale(now, max_age)
+        return self._retired(slots, ev, alerts)
 
     def detect_all_vehicles(self, predict: bool = True) -> np.ndarray:
         """``predict_collisions`` (or ``detect_collisions``) for every vehicle: pairs with i / j = slots

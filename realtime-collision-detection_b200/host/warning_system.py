@@ -226,12 +226,26 @@ class AlertManager:
         self.stats["active_alerts"] = st["n_live"]
         return out
 
+    def _drop_events(self, ev) -> List[Tuple[str, str]]:
+        """Drop the alerts of the device table's EXPIRED events from the host dicts; returns their (vehicle, other) keys."""
+        self._drop([self._by_number.pop(int(e["alert_id"]), None) for e in ev])
+        return [(self._id_of(int(e["i"])), self._id_of(int(e["j"]))) for e in ev]
+
     def cleanup_expired(self, now: Optional[float] = None, max_age: float = ALERT_MAX_AGE) -> List[Tuple[str, str]]:
         """_cleanup_expired_alerts (:488-517) on the device table; returns the (vehicle, other) keys that were dropped."""
         ev, st = self._engine.alerts_expire(time.time() if now is None else now, max_age)
-        self._drop([self._by_number.pop(int(e["alert_id"]), None) for e in ev])
+        keys = self._drop_events(ev)
         self.stats["active_alerts"] = st["n_live"]
-        return [(self._id_of(int(e["i"])), self._id_of(int(e["j"]))) for e in ev]
+        return keys
+
+    def retire_vehicles(self, ev, vehicle_ids) -> List[Tuple[str, str]]:
+        """The host side of retiring vehicles on the attached engine (``FrameEngine.retire`` / ``retire_stale``): drop
+        the alerts of its EXPIRED events -- call while ``id_of`` still names the departed vehicles -- and forget the
+        departed vehicles' per-vehicle entries.  Returns the (vehicle, other) keys that were dropped."""
+        keys = self._drop_events(ev)
+        for v in vehicle_ids:
+            self.vehicle_alerts.pop(v, None)
+        return keys
 
     def acknowledge(self, vehicle_id_index: int, other_vehicle_index: int) -> bool:
         """acknowledge_alert (:199-213) addressed by the pair's caller ids (device table)."""

@@ -77,6 +77,6 @@ for order in ("slot order", "random order"):
                 e.sync()
                 ms.append(e.stage_ms(N.MODE_DETECT)["upload"])
             t = float(np.median(ms[2:]))
-            alg = n * (72 + 50 + (32 + 8 if hist else 0))
+            alg = n * (72 + 58 + (32 + 8 if hist else 0))  # (58: the state and the record time)
             print(json.dumps({"what": f"k_apply_records, {order}, history={hist}", "records": n, "ms": round(t, 4),
                               "alg_bytes": alg, "GBps": round(alg / t / 1e6, 1), "frac_of_measured_peak": round(alg / t / 1e6 / peak, 3)}))
