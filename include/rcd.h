@@ -152,6 +152,28 @@ const char *rcd_last_error(rcd_handle h); /* h may be NULL: last error of rcd_cr
 int rcd_create(const rcd_config *cfg, rcd_handle *out);
 int rcd_destroy(rcd_handle h);
 
+/* ---- growing a handle in place ------------------------------------------------------------------------
+ * Grow the handle to max_objects objects and / or max_pairs emitted pairs.  0 keeps the current value, and so does a
+ * value below it: the handle never shrinks.  A call that changes neither is a no-op.
+ *   - Kept: the first n entries (owned and halo) of the object state, type, pattern and caller id; n, n_owned, the
+ *     record-built flag (rcd_retire_stale), the record times, the trajectory rings and their counts, the query list
+ *     of rcd_set_queries, the compute-node parameters, the world bounds, the alert table with its counters and alert
+ *     numbering, and the slot layout rcd_apply_records writes to.  A step after rcd_reserve, with no other call in
+ *     between, emits exactly what the same step would have emitted without it.
+ *   - Slots in [n, new max_objects) start as rcd_create and rcd_history_configure leave them: zero state, no ring
+ *     samples, no record time.
+ *   - Every buffer is sized exactly as in a handle created at the final size, so such a handle and a grown one step
+ *     alike, pair-test counts (rcd_pair_tests) included.
+ *   - Ends the frame, like rcd_set_queries: rcd_counts, rcd_download*, rcd_pair_tests and rcd_alerts_update return
+ *     RCD_ESTATE until the next rcd_step, and so does a following RCD_STEP_APPEND.  The spatial index is rebuilt by
+ *     the next step and every captured step graph (RCD_FLAG_GRAPH) is dropped, to be captured again.
+ *   - RCD_ESTATE while a download or summary delivery is in flight (finish it first).  Otherwise the call first waits
+ *     for the handle's streams, the alert stream included, and synchronises again before it returns.
+ *   - Old and new buffers coexist during the call: peak device memory is the old set plus the new one.  The new set
+ *     is complete before it replaces the old one, so a failure leaves the handle untouched and usable: RCD_ENOMEM for
+ *     a refused allocation, RCD_EINVAL for max_objects >= 2^30 (as in rcd_create). */
+int rcd_reserve(rcd_handle h, uint64_t max_objects, uint64_t max_pairs);
+
 /* Replace the frame's object state.  Replaces N x CollisionDetector.update_vehicle +
  * SpatialIndex.insert_vehicle (collision_detection.py:74-85, spatial_index.py:162-200) and
  * compute_node.SpatialIndex.insert (compute_node.py:55-72).  All arrays have n entries; id may be
@@ -404,6 +426,13 @@ typedef struct {
 } rcd_alert_stats;
 /* Allocate (or reset) the table for up to max_alerts live alerts. */
 int rcd_alerts_configure(rcd_handle h, uint64_t max_alerts);
+/* Grow the table to max_alerts live alerts, keeping every live alert (unlike rcd_alerts_configure, which empties it):
+ * each keeps its alert number, timestamp, risk / ttc / distance, priority and acknowledged flag, and the next created
+ * alert gets the next number.  The event buffers grow to max_alerts.  max_alerts <= the current size: no-op.
+ * RCD_ESTATE if the table was never configured or while a summary delivery is in flight; max_alerts > 2^31:
+ * RCD_EINVAL.  Old and new tables coexist during the call; a refused allocation (RCD_ENOMEM) leaves the table as it
+ * was.  Synchronises. */
+int rcd_alerts_reserve(rcd_handle h, uint64_t max_alerts);
 /* process_collision_risks on every pair the last rcd_step(s) of this frame emitted (risk >= 0.3 only,
  * :273), with time.time() = now.  events (host, may be NULL with cap 0) receives the CREATED and
  * PRIORITY_CHANGED events, plus the REFRESHED ones if report_refreshed != 0; order is not deterministic.

@@ -238,8 +238,20 @@ struct AlertOfRetired {
     }
 };
 
-// Rebuild the table into its twin (no tombstones): every entry `drop` selects -> EXPIRED event; everything else moves
-// to the twin table.  Drop = AlertTooOld: rcd_alerts_expire; AlertOfRetired: the purge of rcd_retire.
+// rcd_alerts_reserve: every entry moves to a larger table of dst_mask + 1 slots
+struct AlertKeep {
+    unsigned long long dst_mask;
+    __device__ __forceinline__ bool operator()(const AlertEntry &) const { return false; }
+};
+// The slot mask of the table a rebuild writes: the twin of the same size, unless the predicate brings its own.  (A
+// compile-time choice: the expire and purge rebuilds keep the registers they had before rcd_alerts_reserve.)
+template <typename Drop>
+__device__ __forceinline__ unsigned long long rebuild_dst_mask(const Drop &, unsigned long long cap) { return cap - 1; }
+__device__ __forceinline__ unsigned long long rebuild_dst_mask(const AlertKeep &k, unsigned long long) { return k.dst_mask; }
+
+// Rebuild the table into an empty one (no tombstones): every entry `drop` selects -> EXPIRED event; everything else
+// moves to dst.  Drop = AlertTooOld: rcd_alerts_expire; AlertOfRetired: the purge of rcd_retire (both into the twin);
+// AlertKeep: rcd_alerts_reserve (into a larger table).
 template <typename Drop>
 __global__ void __launch_bounds__(ALERT_THREADS)
 k_alert_rebuild(const AlertEntry *__restrict__ src, unsigned long long cap, Drop drop, AlertEntry *dst,
@@ -265,7 +277,8 @@ k_alert_rebuild(const AlertEntry *__restrict__ src, unsigned long long cap, Drop
                 } else {
                     bool inserted = false;
                     unsigned long long st_unused = 0;
-                    AlertEntry *d = alert_find_or_insert(dst, cap - 1, a.key, inserted, st_unused);  // same capacity: always fits
+                    AlertEntry *d = alert_find_or_insert(dst, rebuild_dst_mask(drop, cap), a.key, inserted,
+                                                         st_unused);  // at least as large: always fits
                     d->ts = a.ts; d->risk = a.risk; d->ttc = a.ttc; d->distance = a.distance; d->alert_id = a.alert_id;
                     d->priority = a.priority; d->acked = a.acked; d->pad = 0; d->pad2 = 0;
                     ++live;

@@ -177,42 +177,73 @@ struct StepGraph {
     u64 launches = 0;
 };
 
-}  // namespace
-
-struct rcd_handle_s {
-    int device = 0;
-    u32 flags = 0;
-    int sms = 1;  // multiprocessors of the device
-    Stream stream;
+// Every buffer whose size follows from the handle's capacity (max_objects, max_pairs).  rcd_create makes one set
+// (size_buffers); rcd_reserve makes a larger one the same way and swaps it in whole.  The optional parts, made at
+// their first use, are sized by the same functions.
+struct Sized {
     u64 cap = 0, max_pairs = 0;
-    u64 n = 0, n_owned = 0;
 
     DevBuf<float> in_f[11];
     DevBuf<uint8_t> in_type, in_pattern;
     DevBuf<u32> in_id;
 
     DevBuf<u32> keys[2], vals[2];
-    DevBuf<u32> hist, tile_status, tile_counter;
+    DevBuf<u32> tile_status;
     size_t tile_status_words = 0;
 
     DevBuf<float4> P0, P1, P2;
     DevBuf<float4> U;  // packed 48-byte records in upload order
     DevBuf<u32> sorted_slot;
     DevBuf<u32> sorted_id;   // caller ids in cell order (the frame kernels never touch the upload buffers)
-    // uploads from host memory run on their own stream and overlap the previous frame: the upload buffers are
-    // free again as soon as that frame's index is built (k_pack_keys + k_reorder have consumed them)
-    Stream up_stream;
-    Event ev_upload_done, ev_inputs_free;
-    bool upload_pending = false, inputs_busy = false, capturing = false;
     DevBuf<u32> cell_begin;  // [cells_cap + 1] dense cell table
     u32 cells_cap = 0;
-    float cell_scale = 0.5f;    // grid cell edge (x, y) as a fraction of the query radius
     DevBuf<u32> qkeys[2], qvals[2];  // query order: Morton keys of the query volumes + permutation
     // rcd_set_queries: the listed query set.  Made at the first call with a list (about 8 B per object).
     DevBuf<u32> q_list;      // [cap] upload slots of the listed queries
     DevBuf<u32> q_pos;       // [cap] upload slot -> position in cell order (IndexState::slot_pos)
     DevBuf<u32> q_seen;      // [cap / 32 + 2] bitmap of the device-list check, then its error word
     HostBuf<u32> q_host;     // [cap] pinned copy of a host list on its way to q_list
+
+    FrameBuffers bufs[2];  // the current set and the twin of the pipelined deliveries (made at their first use)
+    DevBuf<u32> cand_count;
+    DevBuf<QEntry> q3;
+    u32 qcap = 0;
+    DevBuf<uint2> qa;        // pair queue k_pairs -> k_narrow
+    DevBuf<u32> qa_fill;
+    u32 qa_blocks_cap = 0;
+    DevBuf<uint4> ovf;       // work items (or rests of them) left to the overflow pass of k_pairs
+    u32 ovf_cap = 0;
+    DevBuf<uint4> items;     // work items of k_pairs (k_tile_plan)
+    u32 items_cap = 0;
+    DevBuf<int4> tile_box;   // [2 * tiles]
+    DevBuf<uint2> tile_rowx; // [TILE_ROWS * tiles]
+    DevBuf<rcd_pair_compact> compact_dev;    // scratch of rcd_download_begin_compact
+
+    DevBuf<Sample64> traj;  // trajectory rings, [max_history][cap]
+    DevBuf<u32> traj_count;
+    u32 traj_len = 0;
+    // rcd_retire_stale: per slot, the timestamp of the newest applied record (no_record_time(): none).  Made at the
+    // first rcd_apply_records (8 B per object).
+    DevBuf<double> last_seen;
+};
+
+}  // namespace
+
+struct rcd_handle_s : Sized {
+    int device = 0;
+    u32 flags = 0;
+    int sms = 1;  // multiprocessors of the device
+    Stream stream;
+    u64 n = 0, n_owned = 0;
+
+    DevBuf<u32> hist, tile_counter;
+
+    // uploads from host memory run on their own stream and overlap the previous frame: the upload buffers are
+    // free again as soon as that frame's index is built (k_pack_keys + k_reorder have consumed them)
+    Stream up_stream;
+    Event ev_upload_done, ev_inputs_free;
+    bool upload_pending = false, inputs_busy = false, capturing = false;
+    float cell_scale = 0.5f;    // grid cell edge (x, y) as a fraction of the query radius
     Event q_copied;          // q_host is free again
     bool q_listed = false;
     u64 q_n = 0;
@@ -225,22 +256,9 @@ struct rcd_handle_s {
     HostBuf<int> bbox_host;
     IndexState idx;
 
-    FrameBuffers bufs[2];  // the current set and the twin of the pipelined deliveries
     int cur = 0;
     HostBuf<Counters> counters_host;
-    DevBuf<u32> cand_count;
     DevBuf<u32> pair_tile_counter;
-    DevBuf<QEntry> q3;
-    u32 qcap = 0;
-    DevBuf<uint2> qa;        // pair queue k_pairs -> k_narrow
-    DevBuf<u32> qa_fill;
-    u32 qa_blocks_cap = 0;
-    DevBuf<uint4> ovf;       // work items (or rests of them) left to the overflow pass of k_pairs
-    u32 ovf_cap = 0;
-    DevBuf<uint4> items;     // work items of k_pairs (k_tile_plan)
-    u32 items_cap = 0;
-    DevBuf<int4> tile_box;   // [2 * tiles]
-    DevBuf<uint2> tile_rowx; // [TILE_ROWS * tiles]
     int narrow_blocks[5] = {0, 0, 0, 0, 0};
     int pair_blocks[5] = {0, 0, 0, 0, 0};  // resident blocks per SM x SMs, per kernel variant
     bool frame_done = false;
@@ -249,13 +267,8 @@ struct rcd_handle_s {
     Stage stages[3][RCD_NUM_STAGES];  // per frame mode
     int stage_mode = 0;
     float cn_prediction_time = 5.0f, cn_risk_threshold = 0.5f;
-    DevBuf<Sample64> traj;  // trajectory rings, [max_history][cap]
-    DevBuf<u32> traj_count;
-    u32 traj_len = 0;
-    // rcd_retire_stale: per slot, the timestamp of the newest applied record (no_record_time(): none).  Made at the
-    // first rcd_apply_records (8 B per object).  records_only: every slot of the frame came from rcd_apply_records
-    // (rcd_upload of a non-empty frame and rcd_halo_append clear it, rcd_upload of an empty one sets it).
-    DevBuf<double> last_seen;
+    // records_only: every slot of the frame came from rcd_apply_records (rcd_upload of a non-empty frame and
+    // rcd_halo_append clear it, rcd_upload of an empty one sets it).
     bool records_only = true;
     u64 launches = 0;
     // CUDA-graph replay of rcd_step (RCD_FLAG_GRAPH)
@@ -273,7 +286,6 @@ struct rcd_handle_s {
     rcd_pair *pend_dev = nullptr, *pend_out = nullptr;
     u64 pend_cap = 0, pend_n = 0, pend_n_owned = 0;
     int pend_kind = 0;                       // 0 pairs, 1 compact pairs, 2 summary (alert events + risk counts)
-    DevBuf<rcd_pair_compact> compact_dev;    // scratch of rcd_download_begin_compact
     rcd_pair_compact *pend_out_compact = nullptr;
     u32 *pend_risk = nullptr;
     rcd_alert_event *pend_ev = nullptr;
@@ -384,6 +396,94 @@ MutableState mutable_state(rcd_handle h) {
     for (int k = 0; k < 11; ++k) st.f[k] = h->in_f[k];
     st.type = h->in_type; st.pattern = h->in_pattern; st.id = h->in_id;
     return st;
+}
+
+// ---- sizing: every capacity-dependent buffer is made by one of these (h may be null: errors of rcd_create) ----------
+// The pair buffer, totals and per-object risk counts of one frame.
+int alloc_frame_buffers(rcd_handle h, u64 cap, u64 max_pairs, FrameBuffers &fb) {
+    CUDA_TRY(h, fb.out.alloc(max_pairs));
+    CUDA_TRY(h, fb.counters.alloc());
+    CUDA_TRY(h, fb.risk_count.alloc(cap));
+    return RCD_OK;
+}
+// rcd_set_queries: the list, the inverse map, the bitmap of the device-list check and the pinned staging copy.
+int alloc_queries(rcd_handle h, u64 cap, Sized &s) {
+    CUDA_TRY(h, s.q_list.alloc(cap));
+    CUDA_TRY(h, s.q_pos.alloc(cap));
+    CUDA_TRY(h, s.q_seen.alloc(cap / 32 + 2));
+    CUDA_TRY(h, s.q_host.alloc(cap));
+    return RCD_OK;
+}
+// Trajectory rings [len][cap], every ring empty.
+int alloc_history(rcd_handle h, u64 cap, u32 len, cudaStream_t on, Sized &s) {
+    CUDA_TRY(h, s.traj.alloc((size_t)len * cap));
+    CUDA_TRY(h, s.traj_count.alloc(cap));
+    CUDA_TRY(h, cudaMemsetAsync(s.traj_count, 0, (size_t)cap * sizeof(u32), on));
+    s.traj_len = len;
+    return RCD_OK;
+}
+// rcd_retire_stale's record times, none yet.
+int alloc_last_seen(rcd_handle h, u64 cap, cudaStream_t on, Sized &s) {
+    CUDA_TRY(h, s.last_seen.alloc(cap));
+    CUDA_TRY(h, cudaMemsetAsync(s.last_seen, 0xff, (size_t)cap * sizeof(double), on));  // no record time
+    return RCD_OK;
+}
+
+// The whole set for (cap, max_pairs), every buffer as rcd_create leaves it; `like` (rcd_reserve: the set being
+// replaced) adds the optional parts it has.  The memsets run on `on`.
+int size_buffers(rcd_handle h, u64 cap, u64 max_pairs, const Sized *like, cudaStream_t on, Sized &s) {
+    s.cap = cap;
+    s.max_pairs = max_pairs;
+    s.cells_cap = (u32)std::min<u64>(std::max<u64>(4 * cap, CELLS_CAP_MIN), CELLS_CAP_MAX);
+    for (int k = 0; k < 11; ++k) {
+        CUDA_TRY(h, s.in_f[k].alloc(cap));
+        CUDA_TRY(h, cudaMemsetAsync(s.in_f[k], 0, cap * sizeof(float), on));
+    }
+    CUDA_TRY(h, s.in_type.alloc(cap));
+    CUDA_TRY(h, s.in_pattern.alloc(cap));
+    CUDA_TRY(h, s.in_id.alloc(cap));
+    for (int k = 0; k < 2; ++k) {
+        CUDA_TRY(h, s.keys[k].alloc(cap + 4));
+        CUDA_TRY(h, s.vals[k].alloc(cap + 4));
+    }
+    s.tile_status_words = (size_t)MAX_PASSES * ((cap + SORT_TILE - 1) / SORT_TILE) * RADIX;
+    CUDA_TRY(h, s.tile_status.alloc(s.tile_status_words));
+    CUDA_TRY(h, s.P0.alloc(cap));
+    CUDA_TRY(h, s.P1.alloc(cap));
+    CUDA_TRY(h, s.P2.alloc(cap));
+    CUDA_TRY(h, s.U.alloc(4 * (cap + 4)));
+    CUDA_TRY(h, s.sorted_slot.alloc(cap));
+    CUDA_TRY(h, s.sorted_id.alloc(cap));
+    CUDA_TRY(h, s.cell_begin.alloc((size_t)s.cells_cap + 2));
+    for (int k = 0; k < 2; ++k) {
+        CUDA_TRY(h, s.qkeys[k].alloc(cap + 4));
+        CUDA_TRY(h, s.qvals[k].alloc(cap + 4));
+    }
+    for (int k = 0; k < 2; ++k)  // (the twin exists once a delivery made it; the current set is bufs[0] until then)
+        if (k == 0 || (like && like->bufs[k].out)) RC_TRY(alloc_frame_buffers(h, cap, max_pairs, s.bufs[k]));
+    CUDA_TRY(h, s.cand_count.alloc(cap));
+    // the fp32 stages forward about 5 candidate entries per emitted pair on clustered frames; a full
+    // queue is not an error (the pair is then finished in place) but it is slower
+    s.qcap = (u32)std::min<u64>(6 * max_pairs + 65536, (1ull << 31) - (1ull << 24));  // (32-bit entry indices)
+    CUDA_TRY(h, s.q3.alloc(s.qcap));
+    // the S1 filter forwards ~60 (predict) / ~20 (detect) pairs per object at the density of the bench frame;
+    // the pair queue is handed out in blocks of QA_BLOCK entries, one per warp at a time
+    // (+ one partly filled block per resident warp of k_pairs)
+    s.qa_blocks_cap = (u32)(s.qcap / QA_BLOCK + 148 * 8 * PAIR_WARPS);
+    CUDA_TRY(h, s.qa.alloc((size_t)s.qa_blocks_cap * QA_BLOCK));
+    CUDA_TRY(h, s.qa_fill.alloc(s.qa_blocks_cap));
+    s.items_cap = (u32)((cap / TQ + 1) * ITEMS_PER_TILE_CAP);  // k_tile_plan never makes more
+    CUDA_TRY(h, s.items.alloc(s.items_cap));
+    CUDA_TRY(h, s.tile_box.alloc(2 * (cap / TQ + 1)));
+    CUDA_TRY(h, s.tile_rowx.alloc((size_t)TILE_ROWS * (cap / TQ + 1)));
+    s.ovf_cap = s.items_cap;  // every work item is handed over at most once
+    CUDA_TRY(h, s.ovf.alloc(s.ovf_cap));
+    if (!like) return RCD_OK;
+    if (like->compact_dev) CUDA_TRY(h, s.compact_dev.alloc(max_pairs));
+    if (like->q_list) RC_TRY(alloc_queries(h, cap, s));
+    if (like->traj_len) RC_TRY(alloc_history(h, cap, like->traj_len, on, s));
+    if (like->last_seen) RC_TRY(alloc_last_seen(h, cap, on, s));
+    return RCD_OK;
 }
 
 // A frame's totals reached the host: they size the next alert fold's grid, and fill `out` unless it is null.
@@ -620,11 +720,8 @@ int rcd_create(const rcd_config *cfg, rcd_handle *out) {
     if (!h) return fail(nullptr, RCD_ENOMEM, "rcd_create: out of host memory");
     h->device = cfg->device;
     h->flags = cfg->flags;
-    h->cap = cfg->max_objects;
-    h->max_pairs = std::max<u64>(cfg->max_pairs, 1);
     h->world_static = cfg->world_min[0] <= cfg->world_max[0];
     for (int d = 0; d < 3; ++d) { h->wmin[d] = cfg->world_min[d]; h->wmax[d] = cfg->world_max[d]; }
-    h->cells_cap = (u32)std::min<u64>(std::max<u64>(4 * h->cap, CELLS_CAP_MIN), CELLS_CAP_MAX);
 
     CUDA_TRY(nullptr, cudaSetDevice(h->device));
     {
@@ -640,61 +737,17 @@ int rcd_create(const rcd_config *cfg, rcd_handle *out) {
     CUDA_TRY(nullptr, h->up_stream.create());
     CUDA_TRY(nullptr, h->ev_upload_done.create());
     CUDA_TRY(nullptr, h->ev_inputs_free.create());
-    const size_t cap = (size_t)h->cap;
-    for (int k = 0; k < 11; ++k) {
-        CUDA_TRY(nullptr, h->in_f[k].alloc(cap));
-        CUDA_TRY(nullptr, cudaMemsetAsync(h->in_f[k], 0, cap * sizeof(float), h->stream));
-    }
-    CUDA_TRY(nullptr, h->in_type.alloc(cap));
-    CUDA_TRY(nullptr, h->in_pattern.alloc(cap));
-    CUDA_TRY(nullptr, h->in_id.alloc(cap));
-    for (int k = 0; k < 2; ++k) {
-        CUDA_TRY(nullptr, h->keys[k].alloc(cap + 4));
-        CUDA_TRY(nullptr, h->vals[k].alloc(cap + 4));
-    }
+    RC_TRY(size_buffers(nullptr, cfg->max_objects, std::max<u64>(cfg->max_pairs, 1), nullptr, h->stream, *h));
     CUDA_TRY(nullptr, h->hist.alloc(MAX_PASSES * RADIX));
-    h->tile_status_words = (size_t)MAX_PASSES * ((cap + SORT_TILE - 1) / SORT_TILE) * RADIX;
-    CUDA_TRY(nullptr, h->tile_status.alloc(h->tile_status_words));
     CUDA_TRY(nullptr, h->tile_counter.alloc(MAX_PASSES));
-    CUDA_TRY(nullptr, h->P0.alloc(cap));
-    CUDA_TRY(nullptr, h->P1.alloc(cap));
-    CUDA_TRY(nullptr, h->P2.alloc(cap));
-    CUDA_TRY(nullptr, h->U.alloc(4 * (cap + 4)));
-    CUDA_TRY(nullptr, h->sorted_slot.alloc(cap));
-    CUDA_TRY(nullptr, h->sorted_id.alloc(cap));
-    CUDA_TRY(nullptr, h->cell_begin.alloc((size_t)h->cells_cap + 2));
-    for (int k = 0; k < 2; ++k) {
-        CUDA_TRY(nullptr, h->qkeys[k].alloc(cap + 4));
-        CUDA_TRY(nullptr, h->qvals[k].alloc(cap + 4));
-    }
     if (const char *e = getenv("RCD_CELL_SCALE")) {  // kernel-tuning experiments only
         const double v = atof(e);
         if (v >= 0.05 && v <= 4.0) h->cell_scale = (float)v;
     }
     CUDA_TRY(nullptr, h->bbox_dev.alloc(6));
     CUDA_TRY(nullptr, h->bbox_host.alloc(6));
-    CUDA_TRY(nullptr, h->bufs[0].out.alloc(h->max_pairs));
-    CUDA_TRY(nullptr, h->bufs[0].counters.alloc());
     CUDA_TRY(nullptr, h->counters_host.alloc());
-    CUDA_TRY(nullptr, h->cand_count.alloc(cap));
-    CUDA_TRY(nullptr, h->bufs[0].risk_count.alloc(cap));
     CUDA_TRY(nullptr, h->pair_tile_counter.alloc(2));
-    // the fp32 stages forward about 5 candidate entries per emitted pair on clustered frames; a full
-    // queue is not an error (the pair is then finished in place) but it is slower
-    h->qcap = (u32)std::min<u64>(6 * h->max_pairs + 65536, (1ull << 31) - (1ull << 24));  // (32-bit entry indices)
-    CUDA_TRY(nullptr, h->q3.alloc(h->qcap));
-    // the S1 filter forwards ~60 (predict) / ~20 (detect) pairs per object at the density of the bench frame;
-    // the pair queue is handed out in blocks of QA_BLOCK entries, one per warp at a time
-    // (+ one partly filled block per resident warp of k_pairs)
-    h->qa_blocks_cap = (u32)(h->qcap / QA_BLOCK + 148 * 8 * PAIR_WARPS);
-    CUDA_TRY(nullptr, h->qa.alloc((size_t)h->qa_blocks_cap * QA_BLOCK));
-    CUDA_TRY(nullptr, h->qa_fill.alloc(h->qa_blocks_cap));
-    h->items_cap = (u32)((cap / TQ + 1) * ITEMS_PER_TILE_CAP);  // k_tile_plan never makes more
-    CUDA_TRY(nullptr, h->items.alloc(h->items_cap));
-    CUDA_TRY(nullptr, h->tile_box.alloc(2 * (cap / TQ + 1)));
-    CUDA_TRY(nullptr, h->tile_rowx.alloc((size_t)TILE_ROWS * (cap / TQ + 1)));
-    h->ovf_cap = h->items_cap;  // every work item is handed over at most once
-    CUDA_TRY(nullptr, h->ovf.alloc(h->ovf_cap));
     for (auto &mode : h->stages)
         for (Stage &st : mode) {
             CUDA_TRY(nullptr, st.begin.create(cudaEventDefault));
@@ -707,6 +760,53 @@ int rcd_create(const rcd_config *cfg, rcd_handle *out) {
 
 int rcd_destroy(rcd_handle h) {
     delete h;
+    return RCD_OK;
+}
+
+int rcd_reserve(rcd_handle h, uint64_t max_objects, uint64_t max_pairs) {
+    if (!h) return RCD_EINVAL;
+    if (max_objects >= (1ull << 30)) return fail(h, RCD_EINVAL, "rcd_reserve: max_objects must be below 2^30");
+    const u64 cap = std::max<u64>(h->cap, max_objects), pairs = std::max<u64>(h->max_pairs, max_pairs);
+    if (cap == h->cap && pairs == h->max_pairs) return RCD_OK;
+    if (h->download_pending) return fail(h, RCD_ESTATE, "rcd_reserve: a delivery is in flight");
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    CUDA_TRY(h, cudaStreamSynchronize(h->up_stream));
+    if (h->dl.alert_stream) CUDA_TRY(h, cudaStreamSynchronize(h->dl.alert_stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    Sized s;
+    int rc = size_buffers(h, cap, pairs, h, h->stream, s);
+    // the state the handle keeps: the first n slots of every per-object buffer, the query list
+    const size_t n = (size_t)h->n;
+    auto check = [&](cudaError_t e) {
+        if (rc == RCD_OK && e != cudaSuccess) rc = fail(h, RCD_ECUDA, std::string("rcd_reserve: ") + cudaGetErrorString(e));
+    };
+    auto copy = [&](void *dst, const void *src, size_t bytes) {
+        if (rc == RCD_OK && bytes) check(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, h->stream));
+    };
+    for (int k = 0; k < 11; ++k) copy(s.in_f[k], h->in_f[k], n * sizeof(float));
+    copy(s.in_type, h->in_type, n);
+    copy(s.in_pattern, h->in_pattern, n);
+    copy(s.in_id, h->in_id, n * sizeof(u32));
+    if (h->traj_len) {
+        copy(s.traj_count, h->traj_count, n * sizeof(u32));
+        if (rc == RCD_OK && n)  // sample-major rings [traj_len][cap]: the row pitch grows with the capacity
+            check(cudaMemcpy2DAsync(s.traj, cap * sizeof(Sample64), h->traj, h->cap * sizeof(Sample64), n * sizeof(Sample64),
+                                    h->traj_len, cudaMemcpyDeviceToDevice, h->stream));
+    }
+    if (h->last_seen) copy(s.last_seen, h->last_seen, n * sizeof(double));
+    if (h->q_listed) copy(s.q_list, h->q_list, (size_t)h->q_n * sizeof(u32));
+    // swap only a complete set, and only when nothing in flight touches either set any more
+    check(cudaStreamSynchronize(h->stream));
+    if (rc != RCD_OK) {
+        (void)cudaGetLastError();  // (a refused allocation is not a fault of the handle)
+        return rc;
+    }
+    static_cast<Sized &>(*h) = std::move(s);
+    // the index, the frame and every captured step graph referred to the old buffers
+    h->idx = IndexState{};
+    h->frame_done = false;
+    for (StepGraph &g : h->graphs) g = StepGraph{};
+    for (StepKey &k : h->graph_candidates) k = StepKey{};
     return RCD_OK;
 }
 
@@ -781,18 +881,14 @@ int rcd_set_owned(rcd_handle h, uint64_t n_owned) {
 // the list, inverse-map, bitmap and staging buffers of rcd_set_queries (all or nothing)
 static int queries_ready(rcd_handle h) {
     if (h->q_list) return RCD_OK;
-    DevBuf<u32> list, pos, seen;
-    HostBuf<u32> host;
+    Sized s;
     Event copied;
-    CUDA_TRY(h, list.alloc(h->cap));
-    CUDA_TRY(h, pos.alloc(h->cap));
-    CUDA_TRY(h, seen.alloc(h->cap / 32 + 2));
-    CUDA_TRY(h, host.alloc(h->cap));
+    RC_TRY(alloc_queries(h, h->cap, s));
     CUDA_TRY(h, copied.create());
-    h->q_list = std::move(list);
-    h->q_pos = std::move(pos);
-    h->q_seen = std::move(seen);
-    h->q_host = std::move(host);
+    h->q_list = std::move(s.q_list);
+    h->q_pos = std::move(s.q_pos);
+    h->q_seen = std::move(s.q_seen);
+    h->q_host = std::move(s.q_host);
     h->q_copied = std::move(copied);
     return RCD_OK;
 }
@@ -1177,9 +1273,7 @@ static int delivery_ready(rcd_handle h) {
     if (h->dl.pend_event) return RCD_OK;
     FrameBuffers twin;
     Delivery d;
-    CUDA_TRY(h, twin.out.alloc(h->max_pairs));
-    CUDA_TRY(h, twin.counters.alloc());
-    CUDA_TRY(h, twin.risk_count.alloc(h->cap));
+    RC_TRY(alloc_frame_buffers(h, h->cap, h->max_pairs, twin));
     CUDA_TRY(h, d.counters_host.alloc());
     CUDA_TRY(h, d.alert_counters_host.alloc());
     CUDA_TRY(h, d.copy_stream.create());
@@ -1397,11 +1491,7 @@ int rcd_history_configure(rcd_handle h, uint32_t max_history) {
     CUDA_TRY(h, cudaSetDevice(h->device));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     h->traj.reset(); h->traj_count.reset(); h->traj_len = 0;
-    CUDA_TRY(h, h->traj.alloc((size_t)max_history * h->cap));
-    CUDA_TRY(h, h->traj_count.alloc(h->cap));
-    CUDA_TRY(h, cudaMemsetAsync(h->traj_count, 0, (size_t)h->cap * sizeof(u32), h->stream));
-    h->traj_len = max_history;
-    return RCD_OK;
+    return alloc_history(h, h->cap, max_history, h->stream, *h);
 }
 
 static int history_ready(rcd_handle h) {
@@ -1489,12 +1579,7 @@ int rcd_apply_records(rcd_handle h, uint64_t n, const rcd_record *records, uint3
         RC_TRY(history_ready(h));
     }
     const bool hist = append_history && h->traj.get();
-    if (!h->last_seen) {
-        DevBuf<double> ls;
-        CUDA_TRY(h, ls.alloc(h->cap));
-        CUDA_TRY(h, cudaMemsetAsync(ls, 0xff, (size_t)h->cap * sizeof(double), h->stream));  // no record time
-        h->last_seen = std::move(ls);
-    }
+    if (!h->last_seen) RC_TRY(alloc_last_seen(h, h->cap, h->stream, *h));
     RC_TRY(wait_upload(h));
     reset_stages(h, -1);
     h->stage_mode = 0;
@@ -1572,6 +1657,49 @@ int rcd_alerts_configure(rcd_handle h, uint64_t max_alerts) {
     CUDA_TRY(h, cudaMemsetAsync(h->alert_tab[0], 0xff, (size_t)cap * sizeof(AlertEntry), h->stream));
     CUDA_TRY(h, cudaMemsetAsync(h->alert_counters, 0, sizeof(AlertCounters), h->stream));
     h->alert_cur = 0;
+    h->alert_cap = cap;
+    h->alert_ev_cap = max_alerts;
+    return RCD_OK;
+}
+
+int rcd_alerts_reserve(rcd_handle h, uint64_t max_alerts) {
+    if (!h) return RCD_EINVAL;
+    RC_TRY(alerts_ready(h, "rcd_alerts_reserve"));
+    if (max_alerts > (1ull << 31)) return fail(h, RCD_EINVAL, "rcd_alerts_reserve: max_alerts must be at most 2^31");
+    if (max_alerts <= h->alert_ev_cap) return RCD_OK;
+    if (h->download_pending && h->pend_kind == 2) return fail(h, RCD_ESTATE, "rcd_alerts_reserve: a summary is in flight");
+    CUDA_TRY(h, cudaSetDevice(h->device));
+    if (h->dl.alert_stream) CUDA_TRY(h, cudaStreamSynchronize(h->dl.alert_stream));
+    h->alert_async = false;
+    u64 cap = 1024;
+    while (cap < 2 * max_alerts) cap <<= 1;  // load factor <= 0.5, as in rcd_alerts_configure
+    // the new table, its twin and the event buffers exist before anything of the old ones changes
+    DevBuf<AlertEntry> tab, twin;
+    DevBuf<rcd_alert_event> ev, ev_alt;
+    auto make = [&]() -> int {
+        CUDA_TRY(h, tab.alloc(cap));
+        CUDA_TRY(h, twin.alloc(cap));
+        CUDA_TRY(h, ev.alloc(max_alerts));
+        if (h->alert_ev_alt) CUDA_TRY(h, ev_alt.alloc(max_alerts));
+        return RCD_OK;
+    };
+    if (const int rc = make()) {
+        (void)cudaGetLastError();  // (a refused allocation is not a fault of the handle)
+        return rc;
+    }
+    // every live entry is rehashed into the new table; n_live is recounted, the alert numbering goes on
+    CUDA_TRY(h, cudaMemsetAsync(tab, 0xff, (size_t)cap * sizeof(AlertEntry), h->stream));
+    CUDA_TRY(h, cudaMemsetAsync(&h->alert_counters->n_live, 0, sizeof(unsigned long long), h->stream));
+    const unsigned blocks = (unsigned)std::min<u64>((h->alert_cap + ALERT_THREADS - 1) / ALERT_THREADS, (u64)h->sms * 8);
+    k_alert_rebuild<<<blocks, ALERT_THREADS, 0, h->stream>>>(h->alert_tab[h->alert_cur], h->alert_cap, AlertKeep{cap - 1}, tab, ev, 0,
+                                                             h->alert_counters);
+    KERNEL_CHECK(h);
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    h->alert_tab[0] = std::move(tab);
+    h->alert_tab[1] = std::move(twin);
+    h->alert_cur = 0;
+    h->alert_ev = std::move(ev);
+    if (h->alert_ev_alt) h->alert_ev_alt = std::move(ev_alt);
     h->alert_cap = cap;
     h->alert_ev_cap = max_alerts;
     return RCD_OK;

@@ -38,7 +38,8 @@ SYMBOLS = (
     "rcd_ingest_counts", "rcd_ingest_set_limit", "rcd_ingest_rejected", "rcd_ingest_id_name", "rcd_ingest_type_name", "rcd_ingest_lookup", "rcd_apply_records",
     "rcd_alerts_configure", "rcd_alerts_update", "rcd_alerts_update_pairs", "rcd_alerts_expire",
     "rcd_alerts_acknowledge", "rcd_alerts_download", "rcd_download_begin", "rcd_download_finish", "rcd_graph_replays", "rcd_pair_exact", "rcd_risk_assessment", "rcd_download_begin_compact", "rcd_summary_begin", "rcd_summary_finish",
-    "rcd_download_risk_counts", "rcd_retire", "rcd_retire_stale", "rcd_ingest_release",
+    "rcd_download_risk_counts", "rcd_retire", "rcd_retire_stale", "rcd_ingest_release", "rcd_reserve",
+    "rcd_alerts_reserve",
 )
 
 
@@ -184,6 +185,8 @@ def load() -> ctypes.CDLL:
     L.rcd_ingest_release.argtypes = [vp, u64, vp, ctypes.POINTER(u64)]
     f64 = ctypes.c_double
     L.rcd_alerts_configure.argtypes = [vp, u64]
+    L.rcd_alerts_reserve.argtypes = [vp, u64]
+    L.rcd_reserve.argtypes = [vp, u64, u64]
     L.rcd_alerts_update.argtypes = [vp, f64, i32, vp, u64, ctypes.POINTER(RcdAlertStats)]
     L.rcd_alerts_update_pairs.argtypes = [vp, vp, u64, f64, i32, vp, u64, ctypes.POINTER(RcdAlertStats)]
     L.rcd_alerts_expire.argtypes = [vp, f64, f64, vp, u64, ctypes.POINTER(RcdAlertStats)]

@@ -115,11 +115,12 @@ class CollisionDetector:
         self._engine: Optional[FrameEngine] = None
 
     def _eng(self, n: int) -> FrameEngine:
-        if self._engine is None or self._engine.max_objects < n:
-            if self._engine is not None:
-                self._engine.close()
-            self._engine = FrameEngine(max(1024, 2 * n), device=self.device)
+        cap = max(1024, 2 * n)
+        if self._engine is None:
+            self._engine = FrameEngine(cap, device=self.device)
             self._engine.set_compute_node_params(self.prediction_time, self.risk_threshold)
+        elif self._engine.max_objects < n:  # grow in place (the parameters stay), FrameEngine's default pair buffer
+            self._engine.reserve(cap, max(4096, 16 * cap))
         return self._engine
 
     def detect_collisions(self, vehicle: VehicleState, nearby_vehicles: Dict[str, VehicleState]) -> List[CollisionRisk]:

@@ -67,6 +67,13 @@ class FrameEngine:
     def __exit__(self, *exc):
         self.close()
 
+    def reserve(self, max_objects: Optional[int] = None, max_pairs: Optional[int] = None) -> None:
+        """Grow the handle in place (rcd_reserve): None or a value below the current one keeps it.  The objects,
+        patterns, trajectory rings, record times, query list and alert table stay on the device; the frame ends."""
+        N.check(self._lib.rcd_reserve(self._h, int(max_objects or 0), int(max_pairs or 0)), self._h)
+        self.max_objects = max(self.max_objects, int(max_objects or 0))
+        self.max_pairs = max(self.max_pairs, int(max_pairs or 0))
+
     # -- state ------------------------------------------------------------------------------
     def upload(self, frame: Dict[str, np.ndarray], ids: Optional[np.ndarray] = None) -> None:
         """N x update_vehicle (collision_detection.py:74-85) as one SoA copy."""
@@ -341,6 +348,11 @@ class FrameEngine:
     def alerts_configure(self, max_alerts: int) -> None:
         N.check(self._lib.rcd_alerts_configure(self._h, int(max_alerts)), self._h)
         self._alert_cap = int(max_alerts)
+
+    def alerts_reserve(self, max_alerts: int) -> None:
+        """Grow the alert table to max_alerts live alerts, keeping every live alert and the alert numbering."""
+        N.check(self._lib.rcd_alerts_reserve(self._h, int(max_alerts)), self._h)
+        self._alert_cap = max(self._alert_cap, int(max_alerts))
 
     @staticmethod
     def _alert_stats(st: "N.RcdAlertStats") -> Dict[str, int]:

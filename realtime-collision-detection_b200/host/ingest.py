@@ -161,6 +161,15 @@ class VehiclePositionStream:
     def __exit__(self, *exc):
         self.close()
 
+    def reserve(self, max_objects: Optional[int] = None, max_pairs: Optional[int] = None,
+                max_alerts: Optional[int] = None) -> None:
+        """Grow the frame (vehicles, pair buffer) and the alert table in place: every ring, record time and live alert
+        stays on the device.  The ingest id limit follows ``max_objects``, so new vehicles are taken again."""
+        self.engine.reserve(max_objects, max_pairs)
+        if max_alerts is not None:
+            self.engine.alerts_reserve(max_alerts)
+        self.ingest.set_limit(self.engine.max_objects)
+
     def handle_messages(self, data) -> int:
         """Decode and apply a buffer of vehicle messages; returns how many were applied."""
         rec, max_seq = self.ingest.decode(data)

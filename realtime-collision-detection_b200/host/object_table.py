@@ -115,17 +115,19 @@ class FrameCache:
         self._flags_uploaded = None
         self._results: Dict[Tuple, Tuple[np.ndarray, np.ndarray, Dict]] = {}
         self.frames_run = 0
-        self.engine_generation = 0  # bumps whenever a new handle replaces the old one (device state is lost)
+        self.engine_generation = 0  # bumps when a handle is made (a new handle has no device state)
 
     def _ensure_engine(self):
         need = max(self.table.n, 1)
-        if self.engine is None or self.engine.max_objects < need:
-            if self.engine is not None:
-                self.engine.close()
-            cap = max(1024, 2 * need)
+        if self.engine is not None and self.engine.max_objects >= need:
+            return
+        cap = max(1024, 2 * need)
+        if self.engine is None:
             self.engine = FrameEngine(cap, max_pairs=max(1 << 16, 32 * cap), device=self.device)
             self.engine_generation += 1
             self._uploaded = -1
+        else:  # grown in place: the objects, patterns and rings stay on the device
+            self.engine.reserve(cap, max(1 << 16, 32 * cap))
 
     def sync_objects(self, flags: Optional[np.ndarray] = None):
         self._ensure_engine()
@@ -152,10 +154,10 @@ class FrameCache:
     def run(self, mode: int, radius: float = 100.0, window: float = 10.0, flags: Optional[np.ndarray] = None,
             prepare=None, slots: Optional[np.ndarray] = None):
         """(pairs sorted by slot i, CSR starts per slot, counts) of one frame, memoised until the
-        objects change.  `prepare(cache)` runs after the objects are on the device and again whenever
-        the handle had to be replaced (it sets device-side flags).  `slots` (sorted, unique uint32):
-        only these objects need their rows -- a memoised whole frame answers, else one frame queries
-        just them (rcd_set_queries; its counts are the totals over the slots), memoised per set."""
+        objects change.  `prepare(cache)` runs after the objects are on the device (it sets device-side
+        flags).  `slots` (sorted, unique uint32): only these objects need their rows -- a memoised whole
+        frame answers, else one frame queries just them (rcd_set_queries; its counts are the totals over
+        the slots), memoised per set."""
         self.sync_objects(flags)
         if prepare is not None:
             prepare(self)
@@ -169,23 +171,13 @@ class FrameCache:
         eng = self.engine
         eng.set_queries(slots)
         eng.step(mode, radius, window)
-        while True:
-            counts = eng.counts()
-            if counts["n_pairs"] <= eng.max_pairs:
-                break
-            # the pair buffer overflowed: grow it and run the frame again (counts stay exact)
-            self.engine.close()
-            cap = self.engine.max_objects
-            self.engine = FrameEngine(cap, max_pairs=int(counts["n_pairs"] * 1.5) + 1024, device=self.device)
-            self.engine_generation += 1
-            self._uploaded = -1
-            self._flags_uploaded = None
-            self.sync_objects(flags)
-            if prepare is not None:
-                prepare(self)
-            eng = self.engine
-            eng.set_queries(slots)
+        counts = eng.counts()
+        if counts["n_pairs"] > eng.max_pairs:
+            # the pair buffer overflowed (the counts are exact): grow it in place and run the frame again; the
+            # objects, flags and query list are still on the device
+            eng.reserve(max_pairs=int(counts["n_pairs"] * 1.5) + 1024)
             eng.step(mode, radius, window)
+            counts = eng.counts()
         pairs = eng.download()
         starts = np.searchsorted(pairs["i"], np.arange(self.table.n + 1, dtype=np.uint32), side="left")
         self.frames_run += 1
