@@ -319,9 +319,10 @@ int rcd_classify_patterns(rcd_handle h, uint64_t n, uint32_t stride, const doubl
 /* Trajectory history on the device: replaces CollisionPredictionModel.update_trajectory +
  * _analyze_trajectory_pattern (collision_detection.py:553-570, 623-711) without re-staging every
  * vehicle's samples from the host each frame.  The handle keeps a ring of the last `max_history`
- * (default 100, :539) float64 (x, y, z, t) samples per object slot (= upload order index).
- * Samples of one object must arrive with non-decreasing timestamps (the reference sorts by
- * timestamp before classifying; callers with out-of-order samples use rcd_classify_patterns). */
+ * (default 100, :539) float64 (x, y, z, t) samples per object slot (= upload order index): the
+ * last max_history samples in arrival order, which may be in any timestamp order.  Classifying
+ * sorts them by timestamp first (stable: equal timestamps keep their arrival order), as the
+ * reference does (:638); rings that arrived in timestamp order take a single streaming pass. */
 int rcd_history_configure(rcd_handle h, uint32_t max_history);
 /* Append one sample for each listed slot (slot may be NULL: slots 0..n-1; a slot must not appear
  * twice in one call).  Host arrays. */

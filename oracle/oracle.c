@@ -176,6 +176,24 @@ int32_t orc_pattern(int32_t n, const double *x, const double *y, const double *z
     return cls;
 }
 
+/* orc_pattern for n histories in one call: samples[i][k] = (x, y, z, t) of history i, k < min(count[i], stride),
+ * in insertion order (each history is sorted by orc_pattern itself). */
+void orc_patterns(int64_t n, int32_t stride, const double *samples, const uint32_t *count, uint8_t *out) {
+#pragma omp parallel
+    {
+        double *buf = (double *)malloc(sizeof(double) * 4 * (size_t)(stride > 0 ? stride : 1));
+        double *x = buf, *y = buf + stride, *z = y + stride, *t = z + stride;
+#pragma omp for schedule(static)
+        for (int64_t i = 0; i < n; ++i) {
+            int32_t c = count[i] < (uint32_t)stride ? (int32_t)count[i] : stride;
+            const double *h = samples + (size_t)i * (size_t)stride * 4;
+            for (int32_t k = 0; k < c; ++k) { x[k] = h[4 * k]; y[k] = h[4 * k + 1]; z[k] = h[4 * k + 2]; t[k] = h[4 * k + 3]; }
+            out[i] = (uint8_t)orc_pattern(c, x, y, z, t);
+        }
+        free(buf);
+    }
+}
+
 /* ---- uniform grid accelerator (not part of the reference semantics) --------------------- */
 typedef struct {
     double ox, oy, oz, cell;

@@ -221,6 +221,7 @@ struct Sized {
 
     DevBuf<Sample64> traj;  // trajectory rings, [max_history][cap]
     DevBuf<u32> traj_count;
+    DevBuf<u32> traj_unordered;  // [0] = n, then the n slots whose ring is out of timestamp order (rcd_history_classify)
     u32 traj_len = 0;
     // rcd_retire_stale: per slot, the timestamp of the newest applied record (no_record_time(): none).  Made at the
     // first rcd_apply_records (8 B per object).
@@ -418,6 +419,7 @@ int alloc_queries(rcd_handle h, u64 cap, Sized &s) {
 int alloc_history(rcd_handle h, u64 cap, u32 len, cudaStream_t on, Sized &s) {
     CUDA_TRY(h, s.traj.alloc((size_t)len * cap));
     CUDA_TRY(h, s.traj_count.alloc(cap));
+    CUDA_TRY(h, s.traj_unordered.alloc(cap + 1));
     CUDA_TRY(h, cudaMemsetAsync(s.traj_count, 0, (size_t)cap * sizeof(u32), on));
     s.traj_len = len;
     return RCD_OK;
@@ -1490,7 +1492,7 @@ int rcd_history_configure(rcd_handle h, uint32_t max_history) {
     if (max_history < 2 || max_history > 4096) return fail(h, RCD_EINVAL, "rcd_history_configure: max_history must be in [2, 4096]");
     CUDA_TRY(h, cudaSetDevice(h->device));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    h->traj.reset(); h->traj_count.reset(); h->traj_len = 0;
+    h->traj.reset(); h->traj_count.reset(); h->traj_unordered.reset(); h->traj_len = 0;
     return alloc_history(h, h->cap, max_history, h->stream, *h);
 }
 
@@ -1555,8 +1557,17 @@ int rcd_history_classify(rcd_handle h, uint8_t *pattern_out) {
     RC_TRY(history_ready(h));
     RC_TRY(wait_upload(h));
     if (h->n) {
-        k_history_classify<<<(unsigned)((h->n + 127) / 128), 128, 0, h->stream>>>((u32)h->n, h->traj, h->traj_count,
-                                                                                  (u32)h->cap, h->traj_len, h->in_pattern);
+        CUDA_TRY(h, cudaMemsetAsync(h->traj_unordered, 0, sizeof(u32), h->stream));
+        k_history_classify<<<(unsigned)((h->n + 127) / 128), 128, 0, h->stream>>>(
+            (u32)h->n, h->traj, h->traj_count, (u32)h->cap, h->traj_len, h->in_pattern, h->traj_unordered);
+        KERNEL_CHECK(h);
+        // the rings found out of order, if any: a fixed grid that reads the list's length on the device
+        const size_t smem = (size_t)HISTORY_SORT_BYTES_PER_SAMPLE * h->traj_len;
+        if (smem > 48 * 1024)
+            CUDA_TRY(h, cudaFuncSetAttribute(k_history_classify_sorted, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        const unsigned blocks = (unsigned)std::min<u64>(h->n, (u64)h->sms * 16);
+        k_history_classify_sorted<<<blocks, HISTORY_SORT_THREADS, smem, h->stream>>>(
+            h->traj, h->traj_count, (u32)h->cap, h->traj_len, h->traj_unordered, h->in_pattern);
         KERNEL_CHECK(h);
         if (pattern_out) {
             CUDA_TRY(h, cudaMemcpyAsync(pattern_out, h->in_pattern, (size_t)h->n, cudaMemcpyDeviceToHost, h->stream));

@@ -1828,28 +1828,31 @@ __global__ void __launch_bounds__(128) k_risk_assessment(u32 n, const double *__
 }
 
 // -------------------------------------------------------------------------------------------------
-// Trajectory pattern classifier (collision_detection.py:623-711), one thread per object, fp64,
-// streaming over the (already time-ordered) samples in the reference's summation order.
+// Trajectory pattern classifier (collision_detection.py:623-711), fp64, streaming over samples in
+// timestamp order in the reference's summation order.  get(k) is the k-th sample, k < cnt (cnt >= 2).
+// CHECK_ORDER: stop at the first sample older than the one before it and return PAT_UNORDERED (the
+// reference sorts by timestamp first, :638, so the stream has to be classified in sorted order).
 // -------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128)
-k_classify_patterns(u32 n, u32 stride, const double *__restrict__ samples /* [n][stride][4] */,
-                    const u32 *__restrict__ count, uint8_t *__restrict__ out) {
-    u32 i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    u32 cnt = min(count[i], stride);
-    if (cnt < 2) { out[i] = RCD_PAT_NO_HISTORY; return; }
-    const double *h = samples + (size_t)i * stride * 4;
+struct Sample64 {
+    double x, y, z, t;
+};
+constexpr u32 PAT_UNORDERED = 0xffu;
+
+template <bool CHECK_ORDER, class Get>
+__device__ __forceinline__ u32 classify_samples(u32 cnt, Get get) {
     double svx = 0, svy = 0, svz = 0, sax = 0, say = 0, saz = 0;
     u32 nv = 0, na = 0;
     double pvx = 0, pvy = 0, pvz = 0, pvt = 0;
-    double lx = h[0], ly = h[1], lz = h[2], lt = h[3];
+    Sample64 last = get(0);
     for (u32 k = 1; k < cnt; ++k) {
-        double x = h[4 * k], y = h[4 * k + 1], z = h[4 * k + 2], t = h[4 * k + 3];
-        double dt = dsub(t, lt);
+        const Sample64 cur = get(k);
+        if (CHECK_ORDER && cur.t < last.t) return PAT_UNORDERED;
+        const double dt = dsub(cur.t, last.t);
         if (dt > 0) {
-            double vx = __ddiv_rn(dsub(x, lx), dt), vy = __ddiv_rn(dsub(y, ly), dt), vz = __ddiv_rn(dsub(z, lz), dt);
+            const double vx = __ddiv_rn(dsub(cur.x, last.x), dt), vy = __ddiv_rn(dsub(cur.y, last.y), dt),
+                         vz = __ddiv_rn(dsub(cur.z, last.z), dt);
             if (nv > 0) {
-                double dtv = dsub(t, pvt);
+                const double dtv = dsub(cur.t, pvt);
                 if (dtv > 0) {
                     sax = dadd(sax, __ddiv_rn(dsub(vx, pvx), dtv));
                     say = dadd(say, __ddiv_rn(dsub(vy, pvy), dtv));
@@ -1859,26 +1862,34 @@ k_classify_patterns(u32 n, u32 stride, const double *__restrict__ samples /* [n]
             }
             svx = dadd(svx, vx); svy = dadd(svy, vy); svz = dadd(svz, vz);
             ++nv;
-            pvx = vx; pvy = vy; pvz = vz; pvt = t;
+            pvx = vx; pvy = vy; pvz = vz; pvt = cur.t;
         }
-        lx = x; ly = y; lz = z; lt = t;
+        last = cur;
     }
-    if (nv == 0) { out[i] = RCD_PAT_STATIONARY; return; }
+    if (nv == 0) return RCD_PAT_STATIONARY;
     svx = __ddiv_rn(svx, (double)nv); svy = __ddiv_rn(svy, (double)nv); svz = __ddiv_rn(svz, (double)nv);
     if (na) { sax = __ddiv_rn(sax, (double)na); say = __ddiv_rn(say, (double)na); saz = __ddiv_rn(saz, (double)na); }
-    double speed = mag3_d(svx, svy, svz), accel = mag3_d(sax, say, saz);
-    out[i] = speed < 0.1 ? RCD_PAT_STATIONARY : (accel < 0.1 ? RCD_PAT_CONSTANT_VELOCITY : RCD_PAT_ACCELERATING);
+    const double speed = mag3_d(svx, svy, svz), accel = mag3_d(sax, say, saz);
+    return speed < 0.1 ? RCD_PAT_STATIONARY : (accel < 0.1 ? RCD_PAT_CONSTANT_VELOCITY : RCD_PAT_ACCELERATING);
+}
+
+// Staged histories, one thread per object: the caller passes them already in timestamp order.
+__global__ void __launch_bounds__(128)
+k_classify_patterns(u32 n, u32 stride, const double *__restrict__ samples /* [n][stride][4] */,
+                    const u32 *__restrict__ count, uint8_t *__restrict__ out) {
+    u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    u32 cnt = min(count[i], stride);
+    if (cnt < 2) { out[i] = RCD_PAT_NO_HISTORY; return; }
+    const Sample64 *h = reinterpret_cast<const Sample64 *>(samples) + (size_t)i * stride;
+    out[i] = (uint8_t)classify_samples<false>(cnt, [&](u32 k) { return h[k]; });
 }
 
 // -------------------------------------------------------------------------------------------------
 // Device-resident trajectory rings: hist[k * cap + slot] = k-th ring entry of the object in `slot`
 // (sample-major, so threads of a warp touch consecutive 32-byte samples), count[slot] = samples ever
-// appended.  Same fp64 arithmetic and summation order as k_classify_patterns.
+// appended.  A ring holds the last min(count, H) samples in arrival order, which need not be timestamp order.
 // -------------------------------------------------------------------------------------------------
-struct Sample64 {
-    double x, y, z, t;
-};
-
 __global__ void __launch_bounds__(256)
 k_history_append(u32 n, const u32 *__restrict__ slot, const double *__restrict__ x, const double *__restrict__ y,
                  const double *__restrict__ z, const double *__restrict__ t, Sample64 *__restrict__ hist,
@@ -1904,45 +1915,53 @@ __global__ void __launch_bounds__(128) k_history_move(u32 dst, u32 src, Sample64
     if (threadIdx.x == 0) count[dst] = count[src];
 }
 
+// One thread per slot, one pass over the ring in arrival order.  A ring whose samples arrive in timestamp order
+// (the common case) gets its code here; one with a sample older than the one before it goes on the list
+// unordered[1 + k] (unordered[0] = length, zeroed before the launch) for k_history_classify_sorted.
 __global__ void __launch_bounds__(128)
 k_history_classify(u32 n, const Sample64 *__restrict__ hist, const u32 *__restrict__ count, u32 cap, u32 H,
-                   uint8_t *__restrict__ out) {
+                   uint8_t *__restrict__ out, u32 *__restrict__ unordered) {
     u32 i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const u32 total = count[i];
     const u32 cnt = min(total, H);
     if (cnt < 2) { out[i] = RCD_PAT_NO_HISTORY; return; }
     const u32 first = total - cnt;  // ring position of the oldest kept sample is first % H
-    double svx = 0, svy = 0, svz = 0, sax = 0, say = 0, saz = 0;
-    u32 nv = 0, na = 0;
-    double pvx = 0, pvy = 0, pvz = 0, pvt = 0;
-    Sample64 last = hist[(size_t)(first % H) * cap + i];
-    for (u32 k = 1; k < cnt; ++k) {
-        const Sample64 cur = hist[(size_t)((first + k) % H) * cap + i];
-        const double dt = dsub(cur.t, last.t);
-        if (dt > 0) {
-            const double vx = __ddiv_rn(dsub(cur.x, last.x), dt), vy = __ddiv_rn(dsub(cur.y, last.y), dt),
-                         vz = __ddiv_rn(dsub(cur.z, last.z), dt);
-            if (nv > 0) {
-                const double dtv = dsub(cur.t, pvt);
-                if (dtv > 0) {
-                    sax = dadd(sax, __ddiv_rn(dsub(vx, pvx), dtv));
-                    say = dadd(say, __ddiv_rn(dsub(vy, pvy), dtv));
-                    saz = dadd(saz, __ddiv_rn(dsub(vz, pvz), dtv));
-                    ++na;
-                }
-            }
-            svx = dadd(svx, vx); svy = dadd(svy, vy); svz = dadd(svz, vz);
-            ++nv;
-            pvx = vx; pvy = vy; pvz = vz; pvt = cur.t;
+    const u32 code = classify_samples<true>(cnt, [&](u32 k) { return hist[(size_t)((first + k) % H) * cap + i]; });
+    if (code == PAT_UNORDERED) unordered[1 + atomicAdd(unordered, 1u)] = i;
+    else out[i] = (uint8_t)code;
+}
+
+// The listed rings, one block per ring (grid-stride over the list, whose length is read here: the launch needs no
+// host round trip).  Kept sample a (arrival order) goes to position #{b : t_b < t_a} + #{b < a : t_b == t_a}, the
+// stable sort by timestamp of the reference (:638); thread 0 then runs the same accumulation as the in-order pass.
+// Dynamic shared memory: H timestamps + H sorted samples = HISTORY_SORT_BYTES_PER_SAMPLE * H bytes.
+constexpr int HISTORY_SORT_THREADS = 128;
+constexpr u32 HISTORY_SORT_BYTES_PER_SAMPLE = sizeof(double) + sizeof(Sample64);
+
+__global__ void __launch_bounds__(HISTORY_SORT_THREADS)
+k_history_classify_sorted(const Sample64 *__restrict__ hist, const u32 *__restrict__ count, u32 cap, u32 H,
+                          const u32 *__restrict__ unordered, uint8_t *__restrict__ out) {
+    extern __shared__ double s_hist[];
+    double *s_t = s_hist;
+    Sample64 *s_sorted = reinterpret_cast<Sample64 *>(s_hist + H);
+    const u32 listed = unordered[0];
+    for (u32 b = blockIdx.x; b < listed; b += gridDim.x) {
+        const u32 i = unordered[1 + b];
+        const u32 total = count[i];
+        const u32 cnt = min(total, H), first = total - cnt;
+        for (u32 a = threadIdx.x; a < cnt; a += blockDim.x) s_t[a] = hist[(size_t)((first + a) % H) * cap + i].t;
+        __syncthreads();
+        for (u32 a = threadIdx.x; a < cnt; a += blockDim.x) {
+            const double t = s_t[a];
+            u32 r = 0;
+            for (u32 q = 0; q < cnt; ++q) r += (u32)(s_t[q] < t) | ((u32)(s_t[q] == t) & (u32)(q < a));
+            s_sorted[r] = hist[(size_t)((first + a) % H) * cap + i];
         }
-        last = cur;
+        __syncthreads();
+        if (threadIdx.x == 0) out[i] = (uint8_t)classify_samples<false>(cnt, [&](u32 k) { return s_sorted[k]; });
+        __syncthreads();
     }
-    if (nv == 0) { out[i] = RCD_PAT_STATIONARY; return; }
-    svx = __ddiv_rn(svx, (double)nv); svy = __ddiv_rn(svy, (double)nv); svz = __ddiv_rn(svz, (double)nv);
-    if (na) { sax = __ddiv_rn(sax, (double)na); say = __ddiv_rn(say, (double)na); saz = __ddiv_rn(saz, (double)na); }
-    const double speed = mag3_d(svx, svy, svz), accel = mag3_d(sax, say, saz);
-    out[i] = speed < 0.1 ? RCD_PAT_STATIONARY : (accel < 0.1 ? RCD_PAT_CONSTANT_VELOCITY : RCD_PAT_ACCELERATING);
 }
 
 // -------------------------------------------------------------------------------------------------

@@ -256,9 +256,8 @@ class CollisionDetector:
 class CollisionPredictionModel:
     """Trajectory histories live twice: in ``trajectory_history`` (the reference's public attribute)
     and in ring buffers on the GPU (rcd_history_*), which are fed incrementally, so classifying every
-    vehicle each frame costs one kernel instead of re-staging up to 100 samples per vehicle.  If a
-    vehicle's samples ever arrive out of timestamp order the model switches to staging sorted
-    histories through rcd_classify_patterns (the reference sorts by timestamp, :638)."""
+    vehicle each frame costs one kernel instead of re-staging up to 100 samples per vehicle.  Both keep
+    the last 100 samples in arrival order; the classifier sorts them by timestamp, like the reference (:638)."""
 
     def __init__(self, collision_detector: CollisionDetector):
         self.collision_detector = collision_detector
@@ -271,8 +270,6 @@ class CollisionPredictionModel:
         self._pattern_key = None
         self._patterns: Optional[np.ndarray] = None
         # device rings
-        self._ordered = True
-        self._last_ts: Dict[str, float] = {}
         self._pending: List[Tuple[str, float, float, float, float]] = []
         self._events_seen = 0
         self._ring_generation = -1
@@ -282,11 +279,7 @@ class CollisionPredictionModel:
         h.append((position, timestamp))
         if len(h) > self.max_history_length:
             self.trajectory_history[vehicle_id] = h[-self.max_history_length:]
-        if timestamp < self._last_ts.get(vehicle_id, float("-inf")):
-            self._ordered = False
-        self._last_ts[vehicle_id] = timestamp
-        if self._ordered:
-            self._pending.append((vehicle_id, position.x, position.y, position.z, timestamp))
+        self._pending.append((vehicle_id, position.x, position.y, position.z, timestamp))
         self._hist_version += 1
 
     # -- device rings ------------------------------------------------------------------------------
@@ -353,26 +346,6 @@ class CollisionPredictionModel:
             self._pattern_key = key
             frames.flags_set_on_device(key)
 
-    def _classify_staged(self) -> np.ndarray:
-        table = self.collision_detector.spatial_index._table
-        n = table.n
-        count = np.zeros(n, np.uint32)
-        stride = 1
-        for s in range(n):
-            h = self.trajectory_history.get(table.ids[s])
-            if h:
-                count[s] = len(h)
-                stride = max(stride, len(h))
-        samples = np.zeros((n, stride, 4), np.float64)
-        for s in range(n):
-            h = self.trajectory_history.get(table.ids[s])
-            if h:
-                hs = sorted(h, key=lambda e: e[1])  # stable, like the reference (:638)
-                samples[s, :len(hs)] = [(p.x, p.y, p.z, t) for p, t in hs]
-        frames = self.collision_detector.spatial_index._frames
-        frames.sync_objects()
-        return frames.engine.classify_patterns(samples, count) if n else np.zeros(0, np.uint8)
-
     def trajectory_patterns(self) -> np.ndarray:
         """Pattern code of every indexed vehicle (collision_detection.py:623-711), classified on the
         GPU; 3 = fewer than 2 samples (-> detect path, :590-592)."""
@@ -380,21 +353,13 @@ class CollisionPredictionModel:
         table = self.collision_detector.spatial_index._table
         if table.n == 0:
             return np.zeros(0, np.uint8)
-        if self._ordered:
-            frames.sync_objects()
-            self._classify_on_device(frames)
-            return self._patterns
-        key = (self._hist_version, table.version)
-        if key != self._pattern_key or self._patterns is None:
-            self._patterns = self._classify_staged()
-            self._pattern_key = key
+        frames.sync_objects()
+        self._classify_on_device(frames)
         return self._patterns
 
     def _frame(self, slots: Optional[np.ndarray] = None):
         frames = self.collision_detector.spatial_index._frames
-        if self._ordered:
-            return frames.run(N.MODE_PREDICT, 100.0, 10.0, prepare=self._classify_on_device, slots=slots)
-        return frames.run(N.MODE_PREDICT, 100.0, 10.0, flags=self.trajectory_patterns(), slots=slots)
+        return frames.run(N.MODE_PREDICT, 100.0, 10.0, prepare=self._classify_on_device, slots=slots)
 
     def predict_collisions(self, vehicle_id: str) -> List[CollisionRisk]:
         det = self.collision_detector

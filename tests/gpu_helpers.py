@@ -1,6 +1,8 @@
 """Comparison of GPU frames (through the C-ABI) with the CPU oracle."""
 from __future__ import annotations
 
+import json
+
 import numpy as np
 
 from tests.helpers import assert_close, assert_pairs_equal
@@ -50,3 +52,32 @@ def compare_counts(counts, cand_count, ora, mode, candidates=True):
         assert counts["n_high_risk"] == int(ora["counts"][3]), "high_risk_collisions"
         prio = np.bincount(ora["risks"]["priority"][ora["risks"]["priority"] >= 0], minlength=4)
         assert counts["n_alerts"] == prio.tolist(), "alerts by priority"
+
+
+def vehicle_messages(frame, ids, timestamp, order=None):
+    """The reference producer's JSON (vehicle_simulator.py:721-752) for the objects of a frame; timestamp: one value
+    or one per object."""
+    types = ["car", "truck", "bus", "motorcycle", "drone", "tram", "van", "bike"]
+    ts = np.broadcast_to(np.asarray(timestamp, np.float64), (len(ids),))
+    out = []
+    for i in (range(len(ids)) if order is None else order):
+        f = lambda k: float(frame[k][i])
+        out.append(json.dumps({
+            "id": ids[i], "position": {"x": f("px"), "y": f("py"), "z": f("pz")},
+            "velocity": {"x": f("vx"), "y": f("vy"), "z": f("vz")},
+            "acceleration": {"x": f("ax"), "y": f("ay"), "z": f("az")},
+            "heading": f("heading"), "size": f("size"), "type": types[int(frame["type"][i]) % len(types)],
+            "timestamp": float(ts[i])}))
+    return "\n".join(out)
+
+
+def feed_rounds(stream, frame, ids, rounds, t0, seed):
+    """`rounds` messages per vehicle, 0.5 s apart (trajectory history); returns the frame of the last round."""
+    from rcd_b200.host import workloads as W
+    rng = np.random.default_rng(seed)
+    f = {k: v.copy() for k, v in frame.items()}
+    for r in range(rounds):
+        last = f
+        stream.handle_messages(vehicle_messages(f, ids, t0 + 0.5 * r))
+        f = W.advance(f, 0.5, rng)
+    return last

@@ -2,10 +2,11 @@
 a frame with retired slots must step exactly like an upload of its live vehicles, staleness is strict at the float64
 boundary, recycled slots start from nothing, and the alerts of departed vehicles go with them."""
 import ctypes
-import json
 
 import numpy as np
 import pytest
+
+from tests.gpu_helpers import feed_rounds as _feed, vehicle_messages as _messages
 
 pytestmark = pytest.mark.gpu
 
@@ -24,39 +25,11 @@ def _W():
     return W
 
 
-def _messages(frame, ids, timestamp, order=None):
-    """The reference producer's JSON (vehicle_simulator.py:721-752) for the objects of a frame; timestamp: one value
-    or one per object."""
-    types = ["car", "truck", "bus", "motorcycle", "drone", "tram", "van", "bike"]
-    ts = np.broadcast_to(np.asarray(timestamp, np.float64), (len(ids),))
-    out = []
-    for i in (range(len(ids)) if order is None else order):
-        f = lambda k: float(frame[k][i])
-        out.append(json.dumps({
-            "id": ids[i], "position": {"x": f("px"), "y": f("py"), "z": f("pz")},
-            "velocity": {"x": f("vx"), "y": f("vy"), "z": f("vz")},
-            "acceleration": {"x": f("ax"), "y": f("ay"), "z": f("az")},
-            "heading": f("heading"), "size": f("size"), "type": types[int(frame["type"][i]) % len(types)],
-            "timestamp": float(ts[i])}))
-    return "\n".join(out)
-
-
 def _frame(kind, n, seed):
     W = _W()
     if kind == "uniform":
         return W.uniform_frame(n, seed, map_size=1000.0, drone_fraction=0.3)
     return W.hotspot_frame(n, seed, 1000.0, 4, radius_range=(100.0, 250.0))
-
-
-def _feed(stream, frame, ids, rounds, t0, seed):
-    """`rounds` messages per vehicle, 0.5 s apart (trajectory history); returns the frame of the last round."""
-    rng = np.random.default_rng(seed)
-    f = {k: v.copy() for k, v in frame.items()}
-    for r in range(rounds):
-        last = f
-        stream.handle_messages(_messages(f, ids, t0 + 0.5 * r))
-        f = _W().advance(f, 0.5, rng)
-    return last
 
 
 def _same_step(a, b, run, live, n):

@@ -69,6 +69,12 @@ def test_scalar_functions_match_reference_golden():
     got = [O.pattern([tuple(r) for r in z["hist"][off[k]:off[k + 1]]]) for k in range(len(off) - 1)]
     assert got == z["hist_class"].tolist()
     assert set(got) == {0, 1, 2, 3}
+    # the same histories through the batch entry point, padded with NaN that must never be read
+    lens = np.diff(off)
+    staged = np.full((len(lens), int(lens.max()) + 3, 4), np.nan)
+    for k in range(len(lens)):
+        staged[k, :lens[k]] = z["hist"][off[k]:off[k + 1]]
+    assert O.patterns(staged, lens).tolist() == z["hist_class"].tolist()
     # alert gate + priority
     assert [O.priority(r, t) for r, t in z["prio_in"]] == z["prio_out"].tolist()
     # grid ids, all four levels (cell = base / 2**level)
